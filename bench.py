@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — read bases k-mer-probed per second on the BASELINE.json workload.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one synthetic trio shard: counts reset, the three
@@ -73,7 +73,16 @@ def parse_args(argv=None):
     ap.add_argument("--no-wgs", action="store_true", help="skip the configs[2]-shard measurement")
     ap.add_argument("--separate-launches", action="store_true", help="one launch per sample instead of one per trio")
     ap.add_argument("--tuning", default="", help="seed_len,stride,bloom_hashes[,filter_mode] (default auto)")
-    return ap.parse_args(argv)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (per-entry counters, per-variant hits, "
+                         "distinct, n_kmers, calls; wgs_shard_* for the configs[2] leg; --impl reference: the "
+                         "counters) as DIR/<name>.npy in "
+                         "float64, at most 64 MB in all: an output too large for that keeps a fixed, seeded "
+                         "sample of its entries or variants, in order")
+    a = ap.parse_args(argv)
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 def workload_name(a):
@@ -178,7 +187,7 @@ def run_reference(a):
     sample = (f"{max(1, a.steps)} steps x {'the whole step' if frac >= 1.0 else f'the first {frac:.3f} of every sample of the step'} "
               f"({nb / 1e9:.2f} Gbases per step of {full_bases / 1e9:.2f}) against the full {len(keys)}-entry table; "
               f"oracle/dnk_oracle.c orc_count_stream, OpenMP, {cores} threads; {int(counts.sum())} k-mer hits per step")
-    print(json.dumps({
+    res = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": a.gpus,
         "steps": a.steps, "warmup": a.warmup, "ms_per_step": el / max(1, a.steps) * 1e3,
         "higher_is_better": True, "scaling": a.scaling, "vs_baseline": None, "dtype": "u64",
@@ -188,7 +197,10 @@ def run_reference(a):
                                 "is not mounted and no Rust toolchain exists here"},
         "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": "port", "sample": sample},
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
-    }))
+    }
+    if a.dump_outputs:  # the counters of the last step's sample of the reads
+        res["dumped_outputs"] = dump_outputs(a.dump_outputs, [{"counts": (counts, 1)}])
+    print(json.dumps(res))
 
 
 # ------------------------------------------------------------------------------------
@@ -255,6 +267,40 @@ def profile_traffic(name):
             return json.load(f).get(name)
     except (OSError, ValueError):
         return None
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, groups, budget=DUMP_BYTES):
+    """--dump-outputs: groups = [{name: (array, axis)}] in priority order, `axis` the one that runs
+    over entries or variants.  A group that fits what is left of the budget is written whole;
+    otherwise every array of it keeps the same fraction of its `axis` (a sorted sample drawn with a
+    fixed seed, so that two runs keep the same indices).  -> {name: [shape, stored shape]}"""
+    os.makedirs(out_dir, exist_ok=True)
+    left, done = budget // 8, {}  # in float64 elements; a file's .npy header takes 16 of them
+    for group in groups:
+        total = sum(arr.size for arr, _ in group.values())
+        frac = min(1.0, max(left - 16 * len(group), 0) / max(total, 1))
+        for name, (arr, axis) in group.items():
+            n = arr.shape[axis]
+            keep = min(n, int(n * frac))
+            if keep < n:
+                idx = np.sort(np.random.default_rng(12345).choice(n, keep, replace=False))
+                arr = np.take(arr, idx, axis=axis)
+            out = np.ascontiguousarray(arr, dtype=np.float64)
+            np.save(os.path.join(out_dir, name + ".npy"), out)
+            left -= out.size + 16
+            done[name] = [list(np.shape(group[name][0])), list(out.shape)]
+    return done
+
+
+def job_outputs(prefix, counts, results):
+    """What a caller of the step receives: the [3, n_entries] counters and finalise's per-variant
+    hits [nv, 2, 3], distinct [nv, 2, 3], n_kmers [nv, 2] and calls [nv]."""
+    hits, distinct, n_kmers, calls = results
+    return {prefix + "counts": (counts, 1), prefix + "hits": (hits, 0), prefix + "distinct": (distinct, 0),
+            prefix + "n_kmers": (n_kmers, 0), prefix + "calls": (calls, 0)}
 
 
 class Job:
@@ -406,6 +452,7 @@ def run_ours(a):
     value = total_bases * a.steps / (ms_max * 1e-3)
     hits, distinct, n_kmers, calls = kc.results()
     ref_counts = job.final_counts()
+    dump = [job_outputs("", ref_counts, (hits, distinct, n_kmers, calls))]
     sum_ok = job.check_sum_of_ranks(ref_counts)
     roof = job.roofline(s0, s1, a.steps, "dram_bytes_per_launch")
     comm = kc.comm_info() if world > 1 else None
@@ -642,6 +689,8 @@ def run_ours(a):
         wj = Job(w, rank, world, local, tdist)
         ms_w, w0, w1 = wj.timed(w.steps, max(w.warmup, 3))
         red = wj.final_counts()
+        if a.dump_outputs and rank == 0:
+            dump.append(job_outputs("wgs_shard_", red, wj.kc.results()))
         sum_w = wj.check_sum_of_ranks(red)
         if rank == 0:
             roof_w = wj.roofline(w0, w1, w.steps, "wgs_dram_bytes_per_launch")
@@ -662,6 +711,8 @@ def run_ours(a):
     if rank == 0:
         out["clocks"] = sampler.stop()
         out["clocks"]["samples_by_end_of_timed_region"] = n_clock_timed
+        if a.dump_outputs:
+            out["dumped_outputs"] = dump_outputs(a.dump_outputs, dump)
         print(json.dumps(out))
     if world > 1:
         tdist.destroy_process_group()
