@@ -7,7 +7,8 @@ NVCCFLAGS = -Xcompiler -fPIC -std=c++17 -O3 -lineinfo \
 CSRC = denovo_kmer_b200/csrc
 OBJ = build/make
 LIB = denovo_kmer_b200/libdkb.so
-HDRS = $(CSRC)/dkb_device.cuh $(CSRC)/dkb_scan.cuh $(CSRC)/dkb_build.cuh $(CSRC)/dkb_pack.cuh include/dkb.h
+HDRS = $(CSRC)/dkb_device.cuh $(CSRC)/dkb_scan.cuh $(CSRC)/dkb_build.cuh $(CSRC)/dkb_pack.cuh \
+       $(CSRC)/dkb_regions.cuh include/dkb.h
 STRIDES = 1 2 4 8 16
 OBJS = $(OBJ)/dkb_api.o $(OBJ)/dkb_host.o $(foreach d,$(STRIDES),$(OBJ)/dkb_scan_d$(d).o)
 

@@ -77,6 +77,9 @@ extern "C" {
     pub fn dkb_batch_submit_device_multi(ctx: *mut DkbCtx, n_batches: c_int, d_bases2: *const *const u32,
                                          d_mask1: *const *const u32, n_positions: *const u64,
                                          samples: *const c_int) -> c_int;
+    pub fn dkb_table_set_regions(ctx: *mut DkbCtx, lo: *const u64, hi: *const u64, n_variants: u32) -> c_int;
+    pub fn dkb_batch_set_loci(ctx: *mut DkbCtx, offsets: *const u64, lo: *const u64, hi: *const u64,
+                              n_reads: usize) -> c_int;
     pub fn dkb_sync(ctx: *mut DkbCtx) -> c_int;
     pub fn dkb_counts_reset(ctx: *mut DkbCtx) -> c_int;
     pub fn dkb_entry_counts_fetch(ctx: *mut DkbCtx, out: *mut u32) -> c_int;

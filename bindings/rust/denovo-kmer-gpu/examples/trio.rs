@@ -8,17 +8,35 @@ pub trait ReadSource {
     /// Fills `seq` (ASCII here; `record.seq().encoded` with `four_bit = true` skips the decode),
     /// `qual`, `offsets` (offsets[0] = 0) with the next batch; false at end of file.
     fn next_batch(&mut self, seq: &mut Vec<u8>, qual: &mut Vec<u8>, offsets: &mut Vec<u64>) -> bool;
+    /// The alignment intervals of the last batch's reads in the linear coordinates of
+    /// `cand_pos` (contig offset + `record.pos()` .. `record.cigar().end_pos()`; `lo >= hi` for
+    /// an unmapped read).  Needed in region mode only.
+    fn loci(&self, lo: &mut Vec<u64>, hi: &mut Vec<u64>);
+}
+
+/// Region mode: count a read toward a candidate only if it aligned within `window` bases of it
+/// (what fetching reads per candidate window does).  `cand_pos`: each candidate's position in the
+/// same linear coordinates as `ReadSource::loci`.
+pub struct Regions<'a> {
+    pub cand_pos: &'a [u64],
+    pub window: u64,
 }
 
 pub fn run_trio(device: i32, k: i32, min_baseq: i32, thr: Thresholds, cands: &[Candidate<'_>],
-                samples: &mut [Box<dyn ReadSource>; 3], rank_world: Option<(i32, i32, [u8; 128])>)
-                -> denovo_kmer_gpu::Result<Vec<bool>> {
+                samples: &mut [Box<dyn ReadSource>; 3], rank_world: Option<(i32, i32, [u8; 128])>,
+                regions: Option<Regions<'_>>) -> denovo_kmer_gpu::Result<Vec<bool>> {
     let mut kc = Counter::new(device, k)?;
     kc.bind_thread_near_gpu()?;
     if let Some((rank, world, id)) = rank_world {
         kc.comm_init(&id, rank, world)?; // every rank scans its own slice of the read batches
     }
     kc.build_table(&variant_kmers(cands, k, true)?)?;
+    if let Some(r) = &regions {
+        let w: Vec<(u64, u64)> =
+            r.cand_pos.iter().map(|&p| (p.saturating_sub(r.window), p.saturating_add(r.window + 1))).collect();
+        kc.set_regions(&w)?;
+    }
+    let (mut lo, mut hi) = (Vec::new(), Vec::new());
     let mut packer = kc.batch_packer(1 << 21, 150 << 21, min_baseq)?;
     let (mut seq, mut qual, mut off) = (Vec::new(), Vec::new(), Vec::new());
     for (sample, src) in samples.iter_mut().enumerate() {
@@ -27,6 +45,10 @@ pub fn run_trio(device: i32, k: i32, min_baseq: i32, thr: Thresholds, cands: &[C
             if in_flight == 2 {
                 kc.sync()?; // both pinned buffers are in use: wait before repacking one
                 in_flight = 0;
+            }
+            if regions.is_some() {
+                src.loci(&mut lo, &mut hi);
+                kc.set_loci(&off, &lo, &hi)?;
             }
             let batch = packer.next(&seq, false, Some(qual.as_slice()), &off)?;
             kc.submit(batch, sample as i32)?;

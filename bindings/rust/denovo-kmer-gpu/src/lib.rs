@@ -113,6 +113,8 @@ pub struct Counter {
     ctx: *mut sys::DkbCtx,
     n_entries: usize,
     n_variants: usize,
+    /// region mode: copies of the loci of batches in flight (the library reads them until `sync`)
+    loci_keep: Vec<[Vec<u64>; 3]>,
     _not_sync: PhantomData<*mut ()>,
 }
 unsafe impl Send for Counter {}
@@ -121,7 +123,7 @@ impl Counter {
     pub fn new(device: i32, k: i32) -> Result<Self> {
         let mut ctx = ptr::null_mut();
         check(unsafe { sys::dkb_ctx_create(device, k, &mut ctx) }, ptr::null())?;
-        Ok(Counter { ctx, n_entries: 0, n_variants: 0, _not_sync: PhantomData })
+        Ok(Counter { ctx, n_entries: 0, n_variants: 0, loci_keep: Vec::new(), _not_sync: PhantomData })
     }
 
     fn ck(&self, code: c_int) -> Result<()> { check(code, self.ctx) }
@@ -173,7 +175,41 @@ impl Counter {
         })
     }
 
-    pub fn sync(&mut self) -> Result<()> { self.ck(unsafe { sys::dkb_sync(self.ctx) }) }
+    /// Region mode (`include/dkb.h`): a read counts toward variant `v` only if its alignment
+    /// interval overlaps `windows[v] = (lo, hi)`, half-open, one per variant of the table.  Every
+    /// batch submitted after this needs its loci ([`Counter::set_loci`]).  A new table, or
+    /// [`Counter::clear_regions`], returns to whole-stream counting.
+    pub fn set_regions(&mut self, windows: &[(u64, u64)]) -> Result<()> {
+        let lo: Vec<u64> = windows.iter().map(|w| w.0).collect();
+        let hi: Vec<u64> = windows.iter().map(|w| w.1).collect();
+        self.ck(unsafe { sys::dkb_table_set_regions(self.ctx, lo.as_ptr(), hi.as_ptr(), windows.len() as u32) })
+    }
+
+    pub fn clear_regions(&mut self) -> Result<()> {
+        self.ck(unsafe { sys::dkb_table_set_regions(self.ctx, ptr::null(), ptr::null(), 0) })
+    }
+
+    /// Region mode: the loci of the NEXT submitted batch - the batch's `offsets` (as packed) and
+    /// each read's alignment interval `[lo, hi)` (rust-htslib: `pos()`, `cigar().end_pos()`;
+    /// `lo >= hi` for an unmapped read).  Copied here and kept until [`Counter::sync`].
+    pub fn set_loci(&mut self, offsets: &[u64], lo: &[u64], hi: &[u64]) -> Result<()> {
+        let keep = [offsets.to_vec(), lo.to_vec(), hi.to_vec()];
+        let n_reads = offsets.len().saturating_sub(1);
+        if lo.len() != n_reads || hi.len() != n_reads || offsets.is_empty() {
+            return Err(DkbError { code: sys::DKB_EINVAL, detail: "lo and hi need one entry per read".into() });
+        }
+        self.ck(unsafe {
+            sys::dkb_batch_set_loci(self.ctx, keep[0].as_ptr(), keep[1].as_ptr(), keep[2].as_ptr(), n_reads)
+        })?;
+        self.loci_keep.push(keep);  // (moving the Vecs does not move their heap buffers)
+        Ok(())
+    }
+
+    pub fn sync(&mut self) -> Result<()> {
+        self.ck(unsafe { sys::dkb_sync(self.ctx) })?;
+        self.loci_keep.clear();
+        Ok(())
+    }
     pub fn reset_counts(&mut self) -> Result<()> { self.ck(unsafe { sys::dkb_counts_reset(self.ctx) }) }
 
     /// Per-entry counts, `[3 samples][n_entries]`.

@@ -144,6 +144,25 @@ def variant_kmers(variants, k: int, drop_shared: bool = True) -> KmerEntries:
     return KmerEntries(keys[:m], var[:m], al[:m], wi[:m], wc[:m], n)
 
 
+# ---- region mode (include/dkb.h "region-scoped counting") ------------------------------------
+@dataclass
+class ReadLoci:
+    """Where a batch's reads aligned: offsets as given to the packer (uint64[n_reads + 1]), and
+    each read's half-open alignment interval [lo, hi) in the caller's linear coordinates
+    (lo >= hi: unmapped, counts toward nothing)."""
+    offsets: np.ndarray
+    lo: np.ndarray
+    hi: np.ndarray
+
+    def __post_init__(self):
+        self.offsets = np.ascontiguousarray(self.offsets, dtype=np.uint64)
+        self.lo = np.ascontiguousarray(self.lo, dtype=np.uint64)
+        self.hi = np.ascontiguousarray(self.hi, dtype=np.uint64)
+        n = len(self.offsets) - 1
+        if n < 0 or len(self.lo) != n or len(self.hi) != n:
+            raise ValueError("ReadLoci: lo and hi need one entry per read (len(offsets) - 1)")
+
+
 # ---- the counter -----------------------------------------------------------------------
 class KmerCounter:
     """One GPU context: build the spanning-k-mer table, stream read batches per
@@ -207,36 +226,64 @@ class KmerCounter:
         self.n_entries = len(keys)
         self.n_variants = int(entries.n_variants)
 
-    def submit(self, stream: ReadStream, sample: int):
-        """Host buffers: async H2D copy + scan; buffers are kept alive until sync()."""
+    def set_regions(self, lo, hi):
+        """Region mode: from now on a read's k-mers count toward variant v only if the read's
+        alignment interval overlaps [lo[v], hi[v]) (one entry per variant of the table; lo >= hi:
+        nothing counts toward v).  Every submit then needs loci=ReadLoci(...)."""
+        lo = np.ascontiguousarray(lo, dtype=np.uint64)
+        hi = np.ascontiguousarray(hi, dtype=np.uint64)
+        if len(lo) != len(hi):
+            raise ValueError("set_regions: lo and hi differ in length")
+        self._ck(self._L.dkb_table_set_regions(self._h, _p(lo, u64p), _p(hi, u64p), len(lo)))
+
+    def clear_regions(self):
+        """Back to whole-stream counting."""
+        self._ck(self._L.dkb_table_set_regions(self._h, None, None, 0))
+
+    def _set_loci(self, loci):
+        if loci is None:
+            return
+        self._keep.append(loci)
+        self._ck(self._L.dkb_batch_set_loci(self._h, _p(loci.offsets, u64p), _p(loci.lo, u64p),
+                                            _p(loci.hi, u64p), len(loci.offsets) - 1))
+
+    def submit(self, stream: ReadStream, sample: int, loci: ReadLoci = None):
+        """Host buffers: async H2D copy + scan; buffers are kept alive until sync().
+        loci: the batch's read loci (region mode)."""
+        self._set_loci(loci)
         self._keep.append(stream)
         self._ck(self._L.dkb_batch_submit(self._h, stream.bases2.ctypes.data,
                                           stream.mask1.ctypes.data, stream.n_positions, sample))
 
-    def submit_sparse(self, bases2, zoff, zbytes, n_positions: int, sample: int):
+    def submit_sparse(self, bases2, zoff, zbytes, n_positions: int, sample: int, loci: ReadLoci = None):
         """Host buffers with the flags as a zero list (mask_to_zero_list): less PCIe traffic."""
+        self._set_loci(loci)
         self._keep.append((bases2, zoff, zbytes))
         self._ck(self._L.dkb_batch_submit_sparse(self._h, bases2.ctypes.data, zoff.ctypes.data,
                                                  zbytes.ctypes.data, len(zbytes), n_positions, sample))
 
     def submit_reads(self, seq, qual, offsets, sample: int, min_baseq: int = DEFAULT_MIN_BASEQ,
-                     four_bit: bool = False):
+                     four_bit: bool = False, loci: ReadLoci = None):
         """Decoded reads (ASCII, or BAM 4-bit codes when four_bit) packed on the GPU."""
         seq = np.ascontiguousarray(seq, dtype=np.uint8)
         qual = None if qual is None else np.ascontiguousarray(qual, dtype=np.uint8)
         offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        self._set_loci(loci)
         self._keep.append((seq, qual, offsets))
         self._ck(self._L.dkb_batch_submit_reads(
             self._h, seq.ctypes.data, int(four_bit), None if qual is None else qual.ctypes.data,
             offsets.ctypes.data, len(offsets) - 1, min_baseq, sample))
 
-    def submit_device(self, d_bases2: int, d_mask1: int, n_positions: int, sample: int):
-        """Device pointers (ints) of a resident stream."""
+    def submit_device(self, d_bases2: int, d_mask1: int, n_positions: int, sample: int,
+                      loci: ReadLoci = None):
+        """Device pointers (ints) of a resident stream.  loci stay referenced until sync()."""
+        self._set_loci(loci)
         self._ck(self._L.dkb_batch_submit_device(self._h, d_bases2, d_mask1, n_positions, sample))
 
     def submit_device_multi(self, batches):
         """batches: up to 4 tuples (d_bases2, d_mask1, n_positions, sample) of resident
-        streams, scanned in ONE kernel launch (e.g. the three samples of a trio)."""
+        streams, scanned in ONE kernel launch (e.g. the three samples of a trio).  Not in
+        region mode."""
         n = len(batches)
         b = (C.c_void_p * n)(*[int(x[0]) for x in batches])
         m = (C.c_void_p * n)(*[int(x[1]) for x in batches])

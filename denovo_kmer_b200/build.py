@@ -10,7 +10,8 @@ from concurrent.futures import ThreadPoolExecutor
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
-HEADERS = [os.path.join(CSRC, f) for f in ("dkb_device.cuh", "dkb_scan.cuh", "dkb_build.cuh", "dkb_pack.cuh")] + [
+HEADERS = [os.path.join(CSRC, f) for f in ("dkb_device.cuh", "dkb_scan.cuh", "dkb_build.cuh", "dkb_pack.cuh",
+                                              "dkb_regions.cuh")] + [
     os.path.join(_HERE, "..", "include", "dkb.h")]
 STRIDES = (1, 2, 4, 8, 16)
 OUT = os.path.join(_HERE, "libdkb.so")

@@ -21,6 +21,7 @@
 #include "../../include/dkb.h"
 #include "dkb_build.cuh"
 #include "dkb_pack.cuh"
+#include "dkb_regions.cuh"
 
 using namespace dkb;
 static_assert(DKB_MAX_MULTI == dkb::MAX_SEGMENTS, "ABI and kernel disagree on the batches per launch");
@@ -97,6 +98,27 @@ struct dkb_ctx {
   size_t red_cap = 0;                       // capacity of each, in uint32
   cudaEvent_t ev_snap[2] = {nullptr, nullptr}, ev_red[2] = {nullptr, nullptr};
   int red_next = 0, red_pending = -1, red_last = -1;
+  // region mode (dkb_table_set_regions): each entry's variant window, and the loci the next
+  // single-batch submit takes (dkb_batch_set_loci; host buffers, copied by that submit)
+  bool regions = false;
+  ulonglong2 *d_entry_win = nullptr;
+  struct Loci {
+    const uint64_t *offsets = nullptr, *lo = nullptr, *hi = nullptr;
+    size_t n_reads = 0;
+    uint64_t n_pos = 0;
+    bool set = false;
+  } loci;
+  // the read-locus index of a batch on the device, double-buffered like `stage`
+  struct LociStage {
+    uint64_t *offsets = nullptr, *lo = nullptr, *hi = nullptr;
+    uint32_t *start = nullptr, *tile = nullptr;
+    ulonglong2 *span = nullptr;
+    size_t off_cap = 0, lo_cap = 0, hi_cap = 0, start_cap = 0, tile_cap = 0, span_cap = 0;
+    uint32_t n_tiles = 0;
+    cudaEvent_t copied = nullptr, freed = nullptr;
+    bool in_use = false;
+  } lstage[2];
+  int next_lstage = 0;
 };
 
 namespace {
@@ -144,6 +166,9 @@ void free_table(dkb_ctx *c) {
   dfree(c->d_counts); dfree(c->d_hits);  // (d_distinct, d_nkmers live in d_hits' block)
   c->d_distinct = c->d_nkmers = nullptr;
   dfree(c->d_calls);
+  dfree(c->d_entry_win);
+  c->regions = false;  // a new table counts the whole stream until dkb_table_set_regions
+  c->loci.set = false;
   c->n_entries = c->n_live = 0;
   c->n_variants = 0;
   c->finalised = false;
@@ -332,28 +357,29 @@ typedef void (*scan_fn)(const ScanParams);
 // The scan kernel's instantiations are compiled one stride per translation unit
 // (dkb_scan_inst.cu with -DDKB_INST_D=...), in parallel; each exports its picker.
 namespace dkb {
-scan_fn pick_scan_d1(int NH, int fm, bool prof);
-scan_fn pick_scan_d2(int NH, int fm, bool prof);
-scan_fn pick_scan_d4(int NH, int fm, bool prof);
-scan_fn pick_scan_d8(int NH, int fm, bool prof);
-scan_fn pick_scan_d16(int NH, int fm, bool prof);
+scan_fn pick_scan_d1(int NH, int fm, bool prof, bool rg);
+scan_fn pick_scan_d2(int NH, int fm, bool prof, bool rg);
+scan_fn pick_scan_d4(int NH, int fm, bool prof, bool rg);
+scan_fn pick_scan_d8(int NH, int fm, bool prof, bool rg);
+scan_fn pick_scan_d16(int NH, int fm, bool prof, bool rg);
 }  // namespace dkb
 
 namespace {
-scan_fn pick_scan(int D, int NH, int fm, bool prof) {
+scan_fn pick_scan(int D, int NH, int fm, bool prof, bool rg) {
   switch (D) {
-    case 1: return pick_scan_d1(NH, fm, prof);
-    case 2: return pick_scan_d2(NH, fm, prof);
-    case 4: return pick_scan_d4(NH, fm, prof);
-    case 8: return pick_scan_d8(NH, fm, prof);
-    case 16: return pick_scan_d16(NH, fm, prof);
+    case 1: return pick_scan_d1(NH, fm, prof, rg);
+    case 2: return pick_scan_d2(NH, fm, prof, rg);
+    case 4: return pick_scan_d4(NH, fm, prof, rg);
+    case 8: return pick_scan_d8(NH, fm, prof, rg);
+    case 16: return pick_scan_d16(NH, fm, prof, rg);
   }
   return nullptr;
 }
 
 // One scan launch over n_seg device-resident packed streams (each into its sample's counters).
+// Region mode: exactly one stream, whose read-locus index is ls.
 int launch_scan(dkb_ctx *ctx, int n_seg, const uint32_t *const *d_bases, const uint32_t *const *d_mask,
-                const uint64_t *n_positions, const int *samples) {
+                const uint64_t *n_positions, const int *samples, dkb_ctx::LociStage *ls = nullptr) {
   ScanParams P;
   memset(&P, 0, sizeof(P));
   // work units: tiles, or macro tiles of 4-8 tiles at strides 8/16
@@ -393,7 +419,18 @@ int launch_scan(dkb_ctx *ctx, int n_seg, const uint32_t *const *d_bases, const u
   P.k = ctx->k;
   P.s = ctx->s;
   P.prof = ctx->d_prof;
-  scan_fn fn = pick_scan(ctx->D, ctx->NH, ctx->gf ? (ctx->pre_words ? 2 : 1) + (ctx->gate ? 2 : 0) : 0, ctx->prof);
+  const bool rg = ctx->regions;
+  if (rg) {
+    if (!ls || P.n_seg != 1) return fail(ctx, DKB_ESTATE, "region mode scans one batch with its loci per launch");
+    P.read_start = ls->start;
+    P.tile_read = ls->tile;
+    P.read_span = ls->span;
+    P.entry_win = ctx->d_entry_win;
+    P.n_loci_tiles = ls->n_tiles;
+  }
+  scan_fn fn = pick_scan(ctx->D, ctx->NH, ctx->gf ? (ctx->pre_words ? 2 : 1) + (ctx->gate ? 2 : 0) : 0, ctx->prof, rg);
+  if (!fn && rg && ctx->prof)
+    return fail(ctx, DKB_ESTATE, "region mode has no scan kernel with profiling counters (dkb_profile_counters 0)");
   if (!fn) return fail(ctx, DKB_EINVAL, "no scan kernel for this tuning");
   size_t smem_bytes = !ctx->gf ? SCAN_SMEM_BYTES
                       : ctx->pre_words ? SCAN_SMEM_BYTES_PRE + (size_t)ctx->pre_words * 4 : SCAN_SMEM_BYTES_GF;
@@ -430,6 +467,10 @@ int launch_scan(dkb_ctx *ctx, int n_seg, const uint32_t *const *d_bases, const u
   CU(cudaGetLastError());
   CU(cudaEventRecord(ev.second, ctx->s_scan));
   ctx->ev_pending.push_back(ev);
+  if (rg) {
+    CU(cudaEventRecord(ls->freed, ctx->s_scan));
+    ls->in_use = true;
+  }
   ctx->scan_launches++;
   ctx->positions_scanned += total_pos;
   ctx->finalised = false;
@@ -437,8 +478,8 @@ int launch_scan(dkb_ctx *ctx, int n_seg, const uint32_t *const *d_bases, const u
 }
 
 int launch_scan(dkb_ctx *ctx, const uint32_t *d_bases, const uint32_t *d_mask, uint64_t n_positions,
-                int sample) {
-  return launch_scan(ctx, 1, &d_bases, &d_mask, &n_positions, &sample);
+                int sample, dkb_ctx::LociStage *ls) {
+  return launch_scan(ctx, 1, &d_bases, &d_mask, &n_positions, &sample, ls);
 }
 
 // Grow a staging buffer (elements of T); the caller has made sure no kernel still reads it.
@@ -452,6 +493,59 @@ int grow(dkb_ctx *ctx, T *&p, size_t &cap, size_t need) {
   CU(cudaMalloc(&q, want * sizeof(T)));
   p = q;
   cap = want;
+  return DKB_OK;
+}
+
+// Region mode: the loci dkb_batch_set_loci left for this submit (consumed whatever the outcome;
+// out->set stays false in whole-stream mode).
+int take_loci(dkb_ctx *ctx, uint64_t n_positions, dkb_ctx::Loci *out) {
+  *out = dkb_ctx::Loci{};
+  if (!ctx->regions) return DKB_OK;
+  const dkb_ctx::Loci l = ctx->loci;
+  ctx->loci.set = false;
+  if (!l.set) return fail(ctx, DKB_ESTATE, "region mode: dkb_batch_set_loci must come before every single-batch submit");
+  if (ctx->prof)
+    return fail(ctx, DKB_ESTATE, "region mode has no scan kernel with profiling counters (dkb_profile_counters 0)");
+  if (l.n_pos != n_positions)
+    return fail(ctx, DKB_EINVAL, "the loci's reads cover " + std::to_string(l.n_pos) + " stream positions, the batch " +
+                                     std::to_string(n_positions));
+  *out = l;
+  return DKB_OK;
+}
+
+// Copy a batch's loci (copy stream) and build its read-locus index (scan stream, ahead of the
+// scan).  ls = nullptr in whole-stream mode.
+int stage_loci(dkb_ctx *ctx, const dkb_ctx::Loci &l, dkb_ctx::LociStage *&ls) {
+  ls = nullptr;
+  if (!l.set) return DKB_OK;
+  dkb_ctx::LociStage &st = ctx->lstage[ctx->next_lstage];
+  ctx->next_lstage ^= 1;
+  const size_t nr = l.n_reads;
+  const uint32_t n_tiles = (uint32_t)((l.n_pos + (1u << LOCI_TILE_SHIFT) - 1) >> LOCI_TILE_SHIFT);
+  if (st.in_use) CU(cudaStreamWaitEvent(ctx->s_copy, st.freed, 0));
+  if (st.off_cap < nr + 1 || st.lo_cap < nr || st.hi_cap < nr || st.start_cap < nr || st.span_cap < nr ||
+      st.tile_cap < (size_t)n_tiles + 1) {
+    if (st.in_use) CU(cudaEventSynchronize(st.freed));  // the previous scan may still read the old index
+    int rc;
+    if ((rc = grow(ctx, st.offsets, st.off_cap, nr + 1)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st.lo, st.lo_cap, nr)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st.hi, st.hi_cap, nr)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st.start, st.start_cap, nr)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st.span, st.span_cap, nr)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st.tile, st.tile_cap, (size_t)n_tiles + 1)) != DKB_OK) return rc;
+  }
+  CU(cudaMemcpyAsync(st.offsets, l.offsets, (nr + 1) * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+  CU(cudaMemcpyAsync(st.lo, l.lo, nr * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+  CU(cudaMemcpyAsync(st.hi, l.hi, nr * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+  CU(cudaEventRecord(st.copied, ctx->s_copy));
+  CU(cudaStreamWaitEvent(ctx->s_scan, st.copied, 0));
+  const int TB = 256;
+  k_read_loci<<<(uint32_t)((nr + TB - 1) / TB), TB, 0, ctx->s_scan>>>(st.offsets, st.lo, st.hi, (uint32_t)nr,
+                                                                       st.start, st.span);
+  k_tile_reads<<<(n_tiles + TB) / TB, TB, 0, ctx->s_scan>>>(st.start, (uint32_t)nr, n_tiles, st.tile);
+  CU(cudaGetLastError());
+  st.n_tiles = n_tiles;
+  ls = &st;
   return DKB_OK;
 }
 
@@ -650,6 +744,10 @@ int dkb_ctx_create(int device, int k, dkb_ctx **out) {
       CU(cudaEventCreateWithFlags(&st.copied, cudaEventDisableTiming));
       CU(cudaEventCreateWithFlags(&st.freed, cudaEventDisableTiming));
     }
+    for (auto &st : ctx->lstage) {
+      CU(cudaEventCreateWithFlags(&st.copied, cudaEventDisableTiming));
+      CU(cudaEventCreateWithFlags(&st.freed, cudaEventDisableTiming));
+    }
     CU(cudaMalloc(&ctx->d_prof, 4 * sizeof(unsigned long long)));
     CU(cudaMemset(ctx->d_prof, 0, 4 * sizeof(unsigned long long)));
     return DKB_OK;
@@ -678,6 +776,16 @@ int dkb_ctx_destroy(dkb_ctx *ctx) {
     dfree(st.nib);
     dfree(st.zoff);
     dfree(st.zbytes);
+    if (st.copied) cudaEventDestroy(st.copied);
+    if (st.freed) cudaEventDestroy(st.freed);
+  }
+  for (auto &st : ctx->lstage) {
+    dfree(st.offsets);
+    dfree(st.lo);
+    dfree(st.hi);
+    dfree(st.start);
+    dfree(st.tile);
+    dfree(st.span);
     if (st.copied) cudaEventDestroy(st.copied);
     if (st.freed) cudaEventDestroy(st.freed);
   }
@@ -897,13 +1005,18 @@ int dkb_batch_submit_device(dkb_ctx *ctx, const uint32_t *d_bases2, const uint32
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
   if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
   if (sample < 0 || sample >= DKB_N_SAMPLES) return fail(ctx, DKB_EINVAL, "sample must be 0, 1 or 2");
+  dkb_ctx::Loci loci;
+  int rc = take_loci(ctx, n_positions, &loci);
+  if (rc != DKB_OK) return rc;
   if (n_positions == 0) return DKB_OK;
   if (n_positions > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
   if (!d_bases2 || !d_mask1) return fail(ctx, DKB_EINVAL, "null stream pointer");
   if ((uintptr_t)d_bases2 & 15) return fail(ctx, DKB_EINVAL, "d_bases2 must be 16-byte aligned");
   if ((uintptr_t)d_mask1 & 3) return fail(ctx, DKB_EINVAL, "d_mask1 must be 4-byte aligned");
   CU(cudaSetDevice(ctx->device));
-  return launch_scan(ctx, d_bases2, d_mask1, n_positions, sample);
+  dkb_ctx::LociStage *ls;
+  if ((rc = stage_loci(ctx, loci, ls)) != DKB_OK) return rc;
+  return launch_scan(ctx, d_bases2, d_mask1, n_positions, sample, ls);
 }
 
 int dkb_batch_submit_device_multi(dkb_ctx *ctx, int n_batches, const uint32_t *const *d_bases2,
@@ -911,6 +1024,7 @@ int dkb_batch_submit_device_multi(dkb_ctx *ctx, int n_batches, const uint32_t *c
                                   const int *samples) {
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
   if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
+  if (ctx->regions) return fail(ctx, DKB_ESTATE, "dkb_batch_submit_device_multi does not support region mode");
   if (n_batches < 0 || n_batches > DKB_MAX_MULTI) return fail(ctx, DKB_EINVAL, "n_batches out of range");
   if (n_batches && (!d_bases2 || !d_mask1 || !n_positions || !samples)) return fail(ctx, DKB_EINVAL, "null argument");
   for (int i = 0; i < n_batches; i++) {
@@ -930,6 +1044,9 @@ int dkb_batch_submit(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t *mask1
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
   if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
   if (sample < 0 || sample >= DKB_N_SAMPLES) return fail(ctx, DKB_EINVAL, "sample must be 0, 1 or 2");
+  dkb_ctx::Loci loci;
+  int rc = take_loci(ctx, n_positions, &loci);
+  if (rc != DKB_OK) return rc;
   if (n_positions == 0) return DKB_OK;
   if (n_positions > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
   if (!bases2 || !mask1) return fail(ctx, DKB_EINVAL, "null stream pointer");
@@ -941,7 +1058,6 @@ int dkb_batch_submit(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t *mask1
   if (st.bases_cap < bw || st.mask_cap < mw) {
     // the previous scan may still read the old buffers
     if (st.in_use) CU(cudaEventSynchronize(st.freed));
-    int rc;
     if ((rc = grow(ctx, st.bases, st.bases_cap, bw)) != DKB_OK) return rc;
     if ((rc = grow(ctx, st.mask, st.mask_cap, mw)) != DKB_OK) return rc;
   }
@@ -949,7 +1065,9 @@ int dkb_batch_submit(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t *mask1
   CU(cudaMemcpyAsync(st.mask, mask1, mw * 4, cudaMemcpyHostToDevice, ctx->s_copy));
   CU(cudaEventRecord(st.copied, ctx->s_copy));
   CU(cudaStreamWaitEvent(ctx->s_scan, st.copied, 0));
-  int rc = launch_scan(ctx, st.bases, st.mask, n_positions, sample);
+  dkb_ctx::LociStage *ls;
+  if ((rc = stage_loci(ctx, loci, ls)) != DKB_OK) return rc;
+  rc = launch_scan(ctx, st.bases, st.mask, n_positions, sample, ls);
   if (rc != DKB_OK) return rc;
   CU(cudaEventRecord(st.freed, ctx->s_scan));
   st.in_use = true;
@@ -961,6 +1079,9 @@ int dkb_batch_submit_sparse(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
   if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
   if (sample < 0 || sample >= DKB_N_SAMPLES) return fail(ctx, DKB_EINVAL, "sample must be 0, 1 or 2");
+  dkb_ctx::Loci loci;
+  int rc = take_loci(ctx, n_positions, &loci);
+  if (rc != DKB_OK) return rc;
   if (n_positions == 0) return DKB_OK;
   if (n_positions > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
   if (!bases2 || !zoff || (zbytes_used && !zbytes)) return fail(ctx, DKB_EINVAL, "null stream pointer");
@@ -978,7 +1099,6 @@ int dkb_batch_submit_sparse(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t
   ctx->next_stage ^= 1;
   const size_t zb1 = zbytes_used ? zbytes_used : 1;
   if (st.in_use) CU(cudaStreamWaitEvent(ctx->s_copy, st.freed, 0));
-  int rc;
   if (st.bases_cap < bw || st.mask_cap < mw || st.zoff_cap < nb + 1 || st.zbytes_cap < zb1) {
     if (st.in_use) CU(cudaEventSynchronize(st.freed));  // the previous scan may still read the old buffers
     if ((rc = grow(ctx, st.bases, st.bases_cap, bw)) != DKB_OK) return rc;
@@ -994,7 +1114,9 @@ int dkb_batch_submit_sparse(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t
   k_expand_zero_list<<<(uint32_t)((nb + 7) / 8), 256, 0, ctx->s_scan>>>(st.zoff, st.zbytes, (uint32_t)nb,
                                                                       (uint32_t)mw, st.mask);
   CU(cudaGetLastError());
-  rc = launch_scan(ctx, st.bases, st.mask, n_positions, sample);
+  dkb_ctx::LociStage *ls;
+  if ((rc = stage_loci(ctx, loci, ls)) != DKB_OK) return rc;
+  rc = launch_scan(ctx, st.bases, st.mask, n_positions, sample, ls);
   if (rc != DKB_OK) return rc;
   CU(cudaEventRecord(st.freed, ctx->s_scan));
   st.in_use = true;
@@ -1007,12 +1129,15 @@ int dkb_batch_submit_reads(dkb_ctx *ctx, const uint8_t *seq, int seq_format, con
   if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
   if (sample < 0 || sample >= DKB_N_SAMPLES) return fail(ctx, DKB_EINVAL, "sample must be 0, 1 or 2");
   if (seq_format != 0 && seq_format != 1) return fail(ctx, DKB_EINVAL, "seq_format must be 0 (ASCII) or 1 (BAM 4-bit)");
-  if (n_reads == 0) return DKB_OK;
+  dkb_ctx::Loci loci;
+  if (n_reads == 0) return take_loci(ctx, 0, &loci);
   if (!seq || !offsets) return fail(ctx, DKB_EINVAL, "null read buffer");
   if (n_reads >= 0xFFFFFFFFull) return fail(ctx, DKB_EINVAL, "too many reads in one batch");
   for (size_t r = 0; r < n_reads; r++)
     if (offsets[r + 1] < offsets[r]) return fail(ctx, DKB_EINVAL, "offsets must not decrease");
   const uint64_t n_pos = dkb_stream_positions(offsets, n_reads);
+  int rc = take_loci(ctx, n_pos, &loci);
+  if (rc != DKB_OK) return rc;
   if (n_pos > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
   const uint64_t n_bases = offsets[n_reads] - offsets[0];
   CU(cudaSetDevice(ctx->device));
@@ -1032,7 +1157,6 @@ int dkb_batch_submit_reads(dkb_ctx *ctx, const uint8_t *seq, int seq_format, con
   dkb_ctx::Stage &st = ctx->stage[ctx->next_stage];
   ctx->next_stage ^= 1;
   if (st.in_use) CU(cudaEventSynchronize(st.freed));  // buffers may be regrown below
-  int rc;
   if ((rc = grow(ctx, st.bases, st.bases_cap, bw)) != DKB_OK) return rc;
   if ((rc = grow(ctx, st.mask, st.mask_cap, mw)) != DKB_OK) return rc;
   if ((rc = grow(ctx, st.seq, st.seq_cap, (size_t)seq_bytes)) != DKB_OK) return rc;
@@ -1066,10 +1190,66 @@ int dkb_batch_submit_reads(dkb_ctx *ctx, const uint8_t *seq, int seq_format, con
   const int TB = 256;
   k_pack<<<(uint32_t)((mw + TB - 1) / TB), TB, 0, ctx->s_scan>>>(Q);
   CU(cudaGetLastError());
-  rc = launch_scan(ctx, st.bases, st.mask, n_pos, sample);
+  dkb_ctx::LociStage *ls;
+  if ((rc = stage_loci(ctx, loci, ls)) != DKB_OK) return rc;
+  rc = launch_scan(ctx, st.bases, st.mask, n_pos, sample, ls);
   if (rc != DKB_OK) return rc;
   CU(cudaEventRecord(st.freed, ctx->s_scan));
   st.in_use = true;
+  return DKB_OK;
+}
+
+int dkb_table_set_regions(dkb_ctx *ctx, const uint64_t *lo, const uint64_t *hi, uint32_t n_variants) {
+  if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
+  if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
+  ctx->loci.set = false;
+  if (!lo && !hi) {
+    if (n_variants) return fail(ctx, DKB_EINVAL, "lo == hi == NULL (whole-stream counting) takes n_variants 0");
+    ctx->regions = false;
+    return DKB_OK;
+  }
+  if (!lo || !hi) return fail(ctx, DKB_EINVAL, "lo and hi must be given together");
+  if (n_variants != ctx->n_variants)
+    return fail(ctx, DKB_EINVAL, "n_variants differs from the table's (" + std::to_string(ctx->n_variants) + ")");
+  CU(cudaSetDevice(ctx->device));
+  std::vector<ulonglong2> win(n_variants ? n_variants : 1);
+  for (uint32_t v = 0; v < n_variants; v++) win[v] = make_ulonglong2(lo[v], hi[v]);
+  const size_t n1 = ctx->n_entries ? ctx->n_entries : 1;
+  if (!ctx->d_entry_win) CU(cudaMalloc(&ctx->d_entry_win, n1 * sizeof(ulonglong2)));
+  ulonglong2 *d_win = nullptr;
+  CU(cudaMalloc(&d_win, win.size() * sizeof(ulonglong2)));
+  // on the scan stream: scans queued before this call still read the previous windows
+  int rc = [&]() -> int {
+    CU(cudaMemcpyAsync(d_win, win.data(), win.size() * sizeof(ulonglong2), cudaMemcpyHostToDevice, ctx->s_scan));
+    const int TB = 256;
+    if (ctx->n_entries)
+      k_entry_windows<<<(uint32_t)((ctx->n_entries + TB - 1) / TB), TB, 0, ctx->s_scan>>>(
+          ctx->d_variant, d_win, (uint32_t)ctx->n_entries, ctx->d_entry_win);
+    CU(cudaGetLastError());
+    CU(cudaStreamSynchronize(ctx->s_scan));
+    return DKB_OK;
+  }();
+  dfree(d_win);
+  if (rc != DKB_OK) return rc;
+  ctx->regions = true;
+  return DKB_OK;
+}
+
+int dkb_batch_set_loci(dkb_ctx *ctx, const uint64_t *offsets, const uint64_t *lo, const uint64_t *hi,
+                       size_t n_reads) {
+  if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
+  ctx->loci.set = false;
+  if (!ctx->regions) return fail(ctx, DKB_ESTATE, "dkb_batch_set_loci needs region mode (dkb_table_set_regions)");
+  if ((uint64_t)n_reads >= 0x100000000ull) return fail(ctx, DKB_EINVAL, "too many reads in one batch (max 2^32 - 1)");
+  if (!offsets || (n_reads && (!lo || !hi))) return fail(ctx, DKB_EINVAL, "null loci array");
+  for (size_t r = 0; r < n_reads; r++)
+    if (offsets[r + 1] < offsets[r]) return fail(ctx, DKB_EINVAL, "offsets must not decrease");
+  ctx->loci.offsets = offsets;
+  ctx->loci.lo = lo;
+  ctx->loci.hi = hi;
+  ctx->loci.n_reads = n_reads;
+  ctx->loci.n_pos = dkb_stream_positions(offsets, n_reads);
+  ctx->loci.set = true;
   return DKB_OK;
 }
 

@@ -275,6 +275,24 @@ struct ScanParams {
   uint32_t filter_words;  // = BLOOM_WORDS (shared-memory mode), as a run-time operand of the wide multiply
   int k, s;
   unsigned long long *prof;  // 4 counters or nullptr
+  // ---- region mode only (k_scan<..., RG = true>; one segment).  Kept at the end so that the
+  // whole-stream kernels' parameter offsets stay where they were.
+  const uint32_t *read_start;   // [n_reads] first stream position of read r
+  const uint32_t *tile_read;    // [n_loci_tiles + 1] first read reaching into 2048-position tile t;
+                                // the last entry is n_reads - 1
+  const ulonglong2 *read_span;  // [n_reads] the read's alignment interval {lo, hi}; {*, 0} if empty
+  const ulonglong2 *entry_win;  // [n_entries] the window of the entry's variant; {*, 0} if empty
+  uint32_t n_loci_tiles;
 };
+
+// Region mode: positions per tile of the read-locus index (a position resolves to its read with
+// one hint load and a binary search between two neighbouring hints).
+constexpr int LOCI_TILE_SHIFT = 11;
+
+// Half-open intervals overlap.  Both are normalised so that an empty one has hi = 0, which no
+// unsigned lo is below: an empty read or window never overlaps anything.
+__host__ __device__ __forceinline__ bool spans_overlap(ulonglong2 a, ulonglong2 b) {
+  return a.x < b.y && b.x < a.y;
+}
 
 }  // namespace dkb

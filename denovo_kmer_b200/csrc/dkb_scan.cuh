@@ -27,7 +27,9 @@ namespace dkb {
 
 // FM = filter mode (dkb_device.cuh): 0 seed filter in shared memory, 1 in L2, 2 in L2 behind a
 // one-bit shared-memory pre-filter, 3 / 4 = 1 / 2 with gated lookups.
-template <int D, int NH, int FM, bool PROF>
+// RG = region mode (DESIGN.md §2): a window counts toward an entry only when its read's
+// alignment interval overlaps the entry's variant window; one segment per launch.
+template <int D, int NH, int FM, bool PROF, bool RG>
 struct ScanWarp {
   static constexpr bool GF = FM > 0, PRE = fm_pre(FM), GATE = fm_gate(FM);
   static constexpr int HL_CAP = hl_cap(FM);
@@ -67,10 +69,31 @@ struct ScanWarp {
     return wi < P.seg[cur].n_mwords ? __ldg(P.seg[cur].mask + wi) : 0u;
   }
 
+  // ---- region mode: the read that holds stream position p --------------------------
+  // The last read starting at or before p, searched between the hints of p's tile and the
+  // next one (a tile holds about 14 reads of 150 bases: four steps).
+  __device__ __forceinline__ uint32_t find_read(uint32_t p) const {
+    // (no min() here: naming it in this class changes how the whole-stream kernels compile)
+    uint32_t t = p >> LOCI_TILE_SHIFT;
+    if (t >= P.n_loci_tiles) t = P.n_loci_tiles - 1;
+    uint32_t a = __ldg(P.tile_read + t), b = __ldg(P.tile_read + t + 1);
+    while (a < b) {
+      const uint32_t mid = b - (b - a) / 2;
+      if (__ldg(P.read_start + mid) <= p) a = mid; else b = mid - 1;
+    }
+    return a;
+  }
+  // Region mode: may read rd count toward entry e?  Only key-table matches get here.
+  __device__ __forceinline__ bool in_region(uint32_t rd, uint32_t e) const {
+    if constexpr (RG) return spans_overlap(__ldg(P.read_span + rd), __ldg(P.entry_win + e));
+    else return true;
+  }
+
   // ---- stage C: the candidate windows of up to n verified seeds --------------------
   // Key-table probe of one window: v = its k bases in stream order (first base least
-  // significant), j = the offset at which it would designate the seed that led here.
-  __device__ __forceinline__ void probe_window(uint64_t v, int j) {
+  // significant), j = the offset at which it would designate the seed that led here,
+  // rd = the read it lies in (region mode only).
+  __device__ __forceinline__ void probe_window(uint64_t v, int j, uint32_t rd) {
     const int k = P.k;
     const uint64_t km = kmer_mask(k);
     if (PROF) n_probe++;
@@ -85,11 +108,11 @@ struct ScanWarp {
       const uint4 s0 = ldg_v4_hint(bp, keep), s1 = ldg_v4_hint(bp + 1, keep);
       const uint64_t k0 = slot_key(s0), k1 = slot_key(s1);
       if (k0 == key && s0.z != ENTRY_DEAD && slot_offset(s0.w, ori, j % D, D) == (uint32_t)j) {
-        atomicAdd(counts + s0.z, 1u);
+        if (in_region(rd, s0.z)) atomicAdd(counts + s0.z, 1u);
         if (PROF) n_hit++;
       }
       if (k1 == key && s1.z != ENTRY_DEAD && slot_offset(s1.w, ori, j % D, D) == (uint32_t)j) {
-        atomicAdd(counts + s1.z, 1u);
+        if (in_region(rd, s1.z)) atomicAdd(counts + s1.z, 1u);
         if (PROF) n_hit++;
       }
       if (k0 == KEY_EMPTY || k1 == KEY_EMPTY) break;  // bucket not full: nothing spilled
@@ -107,10 +130,13 @@ struct ScanWarp {
   // Phase 2, one lane per surviving window: the owners list (lane, offset) pairs in the ring
   // slots just consumed, and the warp probes them 32 at a time - a seed's ~16 windows no
   // longer cost one dependent L2 round trip each inside a single lane.
+  // Region mode resolves the seed's read once here: a counted window contains the seed and
+  // no separator, so it lies in the seed's read; phase 2 takes it from the owner lane.
   __device__ __forceinline__ void stage_c(uint32_t n) {
     const int k = P.k, s = P.s, E = k - s;
     const uint64_t km = kmer_mask(k);
     uint32_t info = 0, p = 0, rn0 = 0, rn1 = 0, rn2 = 0;
+    uint32_t rd = 0;  // region mode: the seed's read
     const uint32_t n_pos = P.seg[cur].n_pos;
     if ((uint32_t)lane < n) {
       const uint64_t e = cq[(ch + lane) & (CQ_CAP - 1)];
@@ -156,10 +182,14 @@ struct ScanWarp {
         const int jlo = E + k - R > 0 ? E + k - R : 0, jhi = E - Lm - 1;
         info = jhi >= jlo ? info & ((2u << jhi) - 1u) & ~((1u << jlo) - 1u) : 0u;
         if ((inv >> E) & ((1ull << s) - 1)) info = 0;  // an invalid base inside the seed itself
+        if constexpr (RG) {
+          if (info) rd = find_read(p);  // (a chance seed match needs no read)
+        }
       } else {
         // no usable neighbourhood (stream start, or 2k - s > NB_BASES): every designated
         // offset is checked here, one after the other
         const uint32_t vm = (1u << k) - 1;  // k <= 31
+        if constexpr (RG) rd = find_read(p);
         while (info) {
           const int j = __ffs(info) - 1;
           info &= info - 1;
@@ -175,7 +205,7 @@ struct ScanWarp {
           if (bo >= 16) { x0 = b[1]; x1 = b[2]; x2 = b[3]; }
           if (bo >= 32) { x0 = b[2]; x1 = b[3]; x2 = b[4]; }
           const uint32_t sh = 2 * (bo & 15);
-          probe_window(((uint64_t)__funnelshift_r(x1, x2, sh) << 32 | __funnelshift_r(x0, x1, sh)) & km, j);
+          probe_window(((uint64_t)__funnelshift_r(x1, x2, sh) << 32 | __funnelshift_r(x0, x1, sh)) & km, j, rd);
         }
       }
     }
@@ -207,11 +237,13 @@ struct ScanWarp {
         const int src = task >> 5, j = task & 31;
         const uint32_t q0 = __shfl_sync(FULL_MASK, rn0, src), q1 = __shfl_sync(FULL_MASK, rn1, src),
                        q2 = __shfl_sync(FULL_MASK, rn2, src);
+        uint32_t qr = 0;
+        if constexpr (RG) qr = __shfl_sync(FULL_MASK, rd, src);
         if (act) {
           const int o = E - j;  // first base of the window in the neighbourhood, 0 .. E
           const uint32_t x0 = o < 16 ? q0 : q1, x1 = o < 16 ? q1 : q2, x2 = o < 16 ? q2 : 0u;
           const uint32_t sh = 2 * (o & 15);
-          probe_window(((uint64_t)__funnelshift_r(x1, x2, sh) << 32 | __funnelshift_r(x0, x1, sh)) & km, j);
+          probe_window(((uint64_t)__funnelshift_r(x1, x2, sh) << 32 | __funnelshift_r(x0, x1, sh)) & km, j, qr);
         }
       }
       __syncwarp();
@@ -822,7 +854,7 @@ struct UnitCursor {
   }
 };
 
-template <int D, int NH, int FM, bool PROF>
+template <int D, int NH, int FM, bool PROF, bool RG>
 __global__ void __launch_bounds__(SCAN_THREADS, 1) k_scan(const ScanParams P) {
   constexpr bool GF = FM > 0;
   extern __shared__ __align__(16) uint32_t smem[];
@@ -839,17 +871,17 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) k_scan(const ScanParams P) {
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   constexpr int HL_CAP = hl_cap(FM);
-  ScanWarp<D, NH, FM, PROF> W(P, filt, hl_all + warp * HL_CAP, cq_all + warp * CQ_CAP, lane);
+  ScanWarp<D, NH, FM, PROF, RG> W(P, filt, hl_all + warp * HL_CAP, cq_all + warp * CQ_CAP, lane);
 
   const uint32_t n_warps = gridDim.x * SCAN_WARPS;
   UnitCursor c{warp * gridDim.x + blockIdx.x, 0};  // consecutive units on different SMs
   c.settle_seg(P);
   W.cur = c.live(P) ? c.seg : 0;
-  if constexpr (ScanWarp<D, NH, FM, PROF>::MACRO) {
+  if constexpr (ScanWarp<D, NH, FM, PROF, RG>::MACRO) {
     // Strides 8 / 16: a macro tile = SUB sub-tiles of 2048 positions (32 lookups per lane),
     // read in groups of GS sub-tiles (GS LDG.128 per lane in flight, 1-2 KB per warp), with
     // the next group prefetched while the current one is filtered.
-    constexpr int SUB = ScanWarp<D, NH, FM, PROF>::SUB, LPT = ScanWarp<D, NH, FM, PROF>::LPT;
+    constexpr int SUB = ScanWarp<D, NH, FM, PROF, RG>::SUB, LPT = ScanWarp<D, NH, FM, PROF, RG>::LPT;
     constexpr int GS = MACRO_GS, GPM = SUB / GS;  // sub-tiles per group, groups per macro tile
     constexpr bool HALO = D < 16;          // at stride 16 every seed lies inside one word
     // a group that ends beyond the stream (the last one of a segment) is read word by word
@@ -1040,7 +1072,7 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) k_scan(const ScanParams P) {
   } else {
   uint32_t nxt[5];
   if (c.live(P)) load_tile(P.seg[c.seg], c.local(P), lane, nxt);
-  if constexpr (ScanWarp<D, NH, FM, PROF>::LOCAL) {
+  if constexpr (ScanWarp<D, NH, FM, PROF, RG>::LOCAL) {
     // Rotated loop: the table loads of tile t (its rounds) are issued at the top of
     // iteration t + 1, right after the prefetched words of tile t + 1 have been settled and
     // before tile t + 2 is requested; they are looked at after stage A of tile t + 1.  The

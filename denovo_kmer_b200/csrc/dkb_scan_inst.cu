@@ -2,7 +2,8 @@
 // 4, 8 or 16), compiled as its own translation unit so that the strides build in parallel.
 // Shared-memory filter: 1..4 filter bits; L2 filter with and without the pre-filter (strides
 // 2..16): 1..2 bits; each with and
-// without the profiling counters.  DKB_AB_BUILD (scripts/ab_build.sh): 2 filter bits only.
+// without the profiling counters, and in region mode (RG, DESIGN.md §2) without them.
+// DKB_AB_BUILD (scripts/ab_build.sh): 2 filter bits only.
 #include "dkb_scan.cuh"
 
 #ifndef DKB_INST_D
@@ -15,12 +16,14 @@ namespace dkb {
 typedef void (*scan_fn)(const ScanParams);
 
 // fm: 0 = filter in shared memory, 1 = in L2, 2 = in L2 behind the shared-memory pre-filter,
-// 3 / 4 = 1 / 2 with gated lookups (macro path: strides 8 and 16)
-scan_fn DKB_CAT(pick_scan_d, DKB_INST_D)(int NH, int fm, bool prof) {
+// 3 / 4 = 1 / 2 with gated lookups (macro path: strides 8 and 16).  Region mode with the
+// profiling counters is not built: nullptr.
+scan_fn DKB_CAT(pick_scan_d, DKB_INST_D)(int NH, int fm, bool prof, bool rg) {
   constexpr int D = DKB_INST_D;
 #define PICK(h, m)                                                                      \
   if (NH == h && fm == m)                                                               \
-    return prof ? (scan_fn)k_scan<D, h, m, true> : (scan_fn)k_scan<D, h, m, false>;
+    return rg ? (prof ? nullptr : (scan_fn)k_scan<D, h, m, false, true>)                \
+              : prof ? (scan_fn)k_scan<D, h, m, true, false> : (scan_fn)k_scan<D, h, m, false, false>;
   PICK(2, 0)
 #if DKB_INST_D >= 2
   PICK(2, 1) PICK(2, 2)

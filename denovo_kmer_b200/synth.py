@@ -33,6 +33,9 @@ class Trio:
     genome: np.ndarray  # uint8 ASCII
     variants: list
     reads: dict = field(default_factory=dict)  # sample -> (seq uint8, qual uint8, offsets uint64)
+    # sample -> (lo, hi) uint64: each read's true alignment interval [lo, hi) in genome coordinates
+    loci: dict = field(default_factory=dict)
+    paralogs: list = field(default_factory=list)  # indices of the variants given a paralog copy
 
     def variant_tuples(self):
         """(left flank, ref, alt, right flank) per variant, flanks k-1 long (shorter at ends)."""
@@ -92,11 +95,43 @@ def apply_variants(genome: np.ndarray, variants) -> np.ndarray:
     return np.concatenate(parts)
 
 
+def hap_ref_positions(genome: np.ndarray, variants) -> np.ndarray:
+    """For every base of apply_variants(genome, variants): the genome position it aligns to.
+    ALT base i of a variant at pos maps to pos + min(i, len(REF) - 1): substituted bases to
+    themselves, inserted bases to their anchor, and a deletion's anchor to itself."""
+    parts, cur = [], 0
+    for v in sorted(variants, key=lambda x: x.pos):
+        parts.append(np.arange(cur, v.pos, dtype=np.int64))
+        parts.append(v.pos + np.minimum(np.arange(len(v.alt)), len(v.ref) - 1))
+        cur = v.pos + len(v.ref)
+    parts.append(np.arange(cur, len(genome), dtype=np.int64))
+    return np.concatenate(parts)
+
+
+def read_loci(refpos, hap_of, starts, lens):
+    """Alignment intervals [lo, hi) in genome coordinates of reads drawn from haplotypes whose
+    bases align to refpos[h] (hap_ref_positions; None = the genome itself): the aligned
+    positions of the read's first and last base.  An empty read gets [lo, lo)."""
+    hap_of = np.asarray(hap_of, dtype=np.int64)
+    starts = np.asarray(starts, dtype=np.int64)
+    lens = np.asarray(lens, dtype=np.int64)
+    lo = np.zeros(len(starts), dtype=np.int64)
+    hi = np.zeros(len(starts), dtype=np.int64)
+    last = starts + np.maximum(lens, 1) - 1
+    for h, rp in enumerate(refpos):
+        sel = hap_of == h
+        lo[sel] = starts[sel] if rp is None else rp[starts[sel]]
+        hi[sel] = (last[sel] if rp is None else rp[last[sel]]) + 1
+    hi = np.where(lens > 0, hi, lo)
+    return lo.astype(np.uint64), hi.astype(np.uint64)
+
+
 def sample_reads(haps, n_reads: int, read_len: int, seed: int, err_rate: float = 0.002,
                  n_rate: float = 0.0005, lowq_frac: float = 0.03, rc_frac: float = 0.5,
-                 ragged: bool = False):
+                 ragged: bool = False, return_meta: bool = False):
     """Reads drawn uniformly from the given haplotypes (equal weight).  Returns
-    (seq ASCII uint8, qual uint8, offsets uint64[n_reads+1])."""
+    (seq ASCII uint8, qual uint8, offsets uint64[n_reads+1]); with return_meta also
+    (haplotype of each read, its start on that haplotype)."""
     rng = np.random.default_rng(seed)
     hap_of = rng.integers(0, len(haps), size=n_reads)
     lens = np.full(n_reads, read_len, dtype=np.int64)
@@ -106,11 +141,13 @@ def sample_reads(haps, n_reads: int, read_len: int, seed: int, err_rate: float =
     offsets[1:] = np.cumsum(lens)
     total = int(offsets[-1])
     seq = np.empty(total, dtype=np.uint8)
+    all_starts = np.zeros(n_reads, dtype=np.int64)
     for h, hap in enumerate(haps):
         idx = np.nonzero(hap_of == h)[0]
         if len(idx) == 0:
             continue
         starts = rng.integers(0, len(hap) - read_len + 1, size=len(idx))
+        all_starts[idx] = starts
         if not ragged:  # fixed length: one gather
             seq.reshape(n_reads, read_len)[idx] = hap[starts[:, None] + np.arange(read_len)[None, :]]
             continue
@@ -134,23 +171,57 @@ def sample_reads(haps, n_reads: int, read_len: int, seed: int, err_rate: float =
     qual = rng.integers(25, 41, size=total).astype(np.uint8)
     low = rng.random(total) < lowq_frac
     qual[low] = rng.integers(2, 20, size=int(low.sum())).astype(np.uint8)
+    if return_meta:
+        return seq, qual, offsets, (hap_of, all_starts)
     return seq, qual, offsets
+
+
+def plant_paralogs(genome: np.ndarray, variants, k: int, which, seed: int, spacer: int = 20_000):
+    """Append to the genome, `spacer` random bases past its end (so far from every candidate
+    window), one copy of the 2k - 1 bases around each variant in `which` carrying its ALT
+    allele, the copies `spacer` apart.  Every sample then holds that variant's alt k-mers at a
+    second locus, as with a paralog or a segmental duplication."""
+    rng = np.random.default_rng(seed)
+    parts = [genome]
+    for i in which:
+        v = variants[i]
+        end = v.pos + len(v.ref)
+        parts.append(make_genome(spacer, int(rng.integers(1 << 30))))
+        parts.append(genome[max(0, v.pos - (k - 1)):v.pos])
+        parts.append(np.frombuffer(v.alt.encode(), dtype=np.uint8))
+        parts.append(genome[end:end + k - 1])
+    parts.append(make_genome(spacer, int(rng.integers(1 << 30))))
+    return np.concatenate(parts)
 
 
 def make_trio_host(genome_len: int, depth: float, n_variants: int, k: int, seed: int = 1,
                    read_len: int = 150, indel_frac: float = 0.0, ragged: bool = False,
-                   **read_kw) -> Trio:
+                   paralog_frac: float = 0.0, **read_kw) -> Trio:
     """Child is heterozygous for every variant; the mother also carries the
-    `inherited` ones; the father carries none."""
+    `inherited` ones; the father carries none.  trio.loci holds every read's true alignment
+    interval.  paralog_frac: that fraction of the de novo (not inherited) variants gets an
+    ALT-carrying copy far away (plant_paralogs; trio.paralogs lists them)."""
     genome = make_genome(genome_len, seed)
     variants = plant_variants(genome, n_variants, k, seed + 1, indel_frac=indel_frac)
+    paralogs = []
+    if paralog_frac > 0:
+        rng = np.random.default_rng(seed + 3)
+        denovo = [i for i, v in enumerate(variants) if not v.inherited]
+        paralogs = sorted(rng.choice(denovo, size=max(1, int(round(paralog_frac * len(denovo)))),
+                                     replace=False).tolist())
+        genome = plant_paralogs(genome, variants, k, paralogs, seed + 4)
     child_alt = apply_variants(genome, variants)
-    mother_alt = apply_variants(genome, [v for v in variants if v.inherited])
-    n_reads = int(genome_len * depth / read_len)
-    trio = Trio(k, genome, variants)
-    trio.reads[0] = sample_reads([genome, child_alt], n_reads, read_len, seed + 10, ragged=ragged, **read_kw)
-    trio.reads[1] = sample_reads([genome, mother_alt], n_reads, read_len, seed + 11, ragged=ragged, **read_kw)
-    trio.reads[2] = sample_reads([genome, genome], n_reads, read_len, seed + 12, ragged=ragged, **read_kw)
+    mother_var = [v for v in variants if v.inherited]
+    mother_alt = apply_variants(genome, mother_var)
+    n_reads = int(len(genome) * depth / read_len)
+    trio = Trio(k, genome, variants, paralogs=paralogs)
+    refpos = {0: [None, hap_ref_positions(genome, variants)],
+              1: [None, hap_ref_positions(genome, mother_var)], 2: [None, None]}
+    for smp, haps in enumerate([[genome, child_alt], [genome, mother_alt], [genome, genome]]):
+        seq, qual, off, (hap_of, starts) = sample_reads(haps, n_reads, read_len, seed + 10 + smp, ragged=ragged,
+                                                        return_meta=True, **read_kw)
+        trio.reads[smp] = (seq, qual, off)
+        trio.loci[smp] = read_loci(refpos[smp], hap_of, starts, np.diff(off).astype(np.int64))
     return trio
 
 
@@ -224,3 +295,14 @@ def make_sample_device(haps_codes, n_reads: int, read_len: int, seed: int, devic
     if return_meta:
         return bases2, mask1, n_pos, n_reads * read_len, (torch.cat(meta_h), torch.cat(meta_s))
     return bases2, mask1, n_pos, n_reads * read_len
+
+
+def device_read_loci(meta, refpos, read_len: int):
+    """The loci of make_sample_device's reads from its return_meta output: (offsets, lo, hi)
+    uint64 host arrays for dkb_batch_set_loci.  refpos[h]: hap_ref_positions of haplotype h
+    (None = the genome itself)."""
+    hap_of, starts = (t.cpu().numpy() for t in meta)
+    n = len(starts)
+    offsets = np.arange(n + 1, dtype=np.uint64) * np.uint64(read_len)
+    lo, hi = read_loci(refpos, hap_of, starts, np.full(n, read_len, dtype=np.int64))
+    return offsets, lo, hi

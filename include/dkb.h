@@ -195,9 +195,35 @@ int dkb_batch_submit_device(dkb_ctx *ctx, const uint32_t *d_bases2, const uint32
  * launch; batch i goes into the counters of samples[i].  Same alignment rules; a batch of 0
  * positions is skipped.  Worth it for short batches, where a launch costs as much as the scan. */
 #define DKB_MAX_MULTI 4
+/* Not supported in region mode (below): returns DKB_ESTATE there. */
 int dkb_batch_submit_device_multi(dkb_ctx *ctx, int n_batches, const uint32_t *const *d_bases2,
                                   const uint32_t *const *d_mask1, const uint64_t *n_positions,
                                   const int *samples);
+
+/* ---- region-scoped counting (opt-in; DESIGN.md §2) ---------------------------- */
+/* In region mode an occurrence of entry e's key in read r counts iff the read's alignment
+ * interval [rlo, rhi) overlaps the window [lo, hi) of e's variant (both half-open, in one
+ * linear coordinate system the caller chooses, e.g. contig offset + 0-based position).  An
+ * empty interval (rlo >= rhi: an unmapped read) or an empty window (lo >= hi) overlaps nothing.
+ * Counters, finalise and the multi-GPU sum are unchanged.
+ * After dkb_table_build: variant v's window is [lo[v], hi[v]), n_variants as built.
+ * lo == hi == NULL (n_variants 0) returns to whole-stream counting.  A new
+ * dkb_table_build also returns to it.  DKB_ESTATE before dkb_table_build; DKB_EINVAL if
+ * n_variants differs from the table's.  Scans queued earlier keep the windows they were
+ * submitted with. */
+int dkb_table_set_regions(dkb_ctx *ctx, const uint64_t *lo, const uint64_t *hi, uint32_t n_variants);
+/* The read loci of the NEXT single-batch submit (dkb_batch_submit, _sparse, _reads, _device).
+ * offsets: n_reads + 1 entries as given to the packer (read r's first base is at stream
+ * position offsets[r] - offsets[0] + r).  lo/hi: the reads' alignment intervals.  Copied by
+ * that submit with the batch; the buffers follow the submit's validity rule (dkb_batch_submit:
+ * valid until dkb_sync; for _device too).  In region mode a single-batch submit without loci
+ * returns DKB_ESTATE, and one whose loci cover a different number of stream positions
+ * (dkb_stream_positions(offsets, n_reads) != n_positions) DKB_EINVAL; either way the loci are
+ * used up.  DKB_ESTATE in whole-stream mode; DKB_EINVAL for descending offsets or
+ * n_reads >= 2^32.  Region mode has no profiling counters: with dkb_profile_counters on, a
+ * submit returns DKB_ESTATE. */
+int dkb_batch_set_loci(dkb_ctx *ctx, const uint64_t *offsets, const uint64_t *lo,
+                       const uint64_t *hi, size_t n_reads);
 int dkb_sync(dkb_ctx *ctx);
 int dkb_counts_reset(dkb_ctx *ctx);
 

@@ -145,6 +145,21 @@ class Counter {
   void counts_allreduce() { check(dkb_counts_allreduce(ctx_), ctx_); }
   void reduce_push(const dkb_thresholds &t) { check(dkb_reduce_push(ctx_, &t), ctx_); }
   void reduce_flush(const dkb_thresholds &t) { check(dkb_reduce_flush(ctx_, &t), ctx_); }
+  // Region mode (dkb.h): a read counts toward variant v only if its alignment interval
+  // overlaps [lo[v], hi[v]); every later submit needs set_loci() first.
+  void set_regions(const std::vector<uint64_t> &lo, const std::vector<uint64_t> &hi) {
+    if (lo.size() != hi.size()) throw Error(DKB_EINVAL, "set_regions: lo and hi differ in length");
+    check(dkb_table_set_regions(ctx_, lo.data(), hi.data(), (uint32_t)lo.size()), ctx_);
+  }
+  void clear_regions() { check(dkb_table_set_regions(ctx_, nullptr, nullptr, 0), ctx_); }
+  // The loci of the next submit: the batch's offsets and its reads' [lo, hi).  The vectors
+  // must stay alive and unchanged until sync().
+  void set_loci(const std::vector<uint64_t> &offsets, const std::vector<uint64_t> &lo,
+                const std::vector<uint64_t> &hi) {
+    if (offsets.empty() || lo.size() + 1 != offsets.size() || hi.size() != lo.size())
+      throw Error(DKB_EINVAL, "set_loci: lo and hi need one entry per read");
+    check(dkb_batch_set_loci(ctx_, offsets.data(), lo.data(), hi.data(), lo.size()), ctx_);
+  }
   void sync() { check(dkb_sync(ctx_), ctx_); }
   void reset_counts() { check(dkb_counts_reset(ctx_), ctx_); }
   std::vector<uint32_t> entry_counts() {  // [3 samples][n_entries]
