@@ -33,6 +33,11 @@ pub const DKB_ENODEV: c_int = 5;
 pub const DKB_ENCCL: c_int = 6;
 pub const DKB_COMM_ID_BYTES: usize = 128;
 pub const DKB_MAX_MULTI: usize = 4;
+pub const DKB_N_SAMPLES: usize = 3;
+/// A family context holds at most 2 + DKB_MAX_CHILDREN samples.
+pub const DKB_MAX_CHILDREN: usize = 6;
+/// Sample index of child `c` in a family (DKB_CHILD_SAMPLE): 0 for c == 0, else 2 + c.
+pub const fn dkb_child_sample(c: usize) -> usize { if c == 0 { 0 } else { c + 2 } }
 pub const DKB_CALL_DENOVO: u8 = 0x01;
 
 extern "C" {
@@ -40,6 +45,8 @@ extern "C" {
     pub fn dkb_strerror(code: c_int) -> *const c_char;
     pub fn dkb_last_error(ctx: *const DkbCtx) -> *const c_char;
     pub fn dkb_ctx_create(device: c_int, k: c_int, out: *mut *mut DkbCtx) -> c_int;
+    pub fn dkb_ctx_create_family(device: c_int, k: c_int, n_children: c_int, out: *mut *mut DkbCtx) -> c_int;
+    pub fn dkb_ctx_get_children(ctx: *const DkbCtx, n_children_out: *mut c_int) -> c_int;
     pub fn dkb_ctx_destroy(ctx: *mut DkbCtx) -> c_int;
     pub fn dkb_ctx_set_tuning(ctx: *mut DkbCtx, t: *const DkbTuning) -> c_int;
     pub fn dkb_ctx_get_tuning(ctx: *const DkbCtx, out: *mut DkbTuning) -> c_int;

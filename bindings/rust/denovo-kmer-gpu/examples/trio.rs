@@ -1,7 +1,7 @@
 //! The loop INTEGRATION.md §3 describes, as code: what the reference's `main.rs` does around
 //! `kmer.rs` / `counter.rs`, with the GPU counter in their place.  The BAM / VCF / FASTA side is
 //! the reference's own (rust-htslib) and is represented here by the `ReadSource` trait.
-use denovo_kmer_gpu::{comm_unique_id, variant_kmers, Candidate, Counter, Thresholds, CALL_DENOVO};
+use denovo_kmer_gpu::{child_sample, comm_unique_id, variant_kmers, Candidate, Counter, Thresholds, CALL_DENOVO};
 
 /// What the reference's BAM layer yields: decoded reads of one sample, in batches.
 pub trait ReadSource {
@@ -22,10 +22,15 @@ pub struct Regions<'a> {
     pub window: u64,
 }
 
+/// `samples`: child, mother, father.  `second_child`: a quad - one family context counts both
+/// children against one table, and each parent's BAM is read once (the second child is
+/// sample `child_sample(1)` = 3).  Returns the de novo calls per child, then per candidate.
 pub fn run_trio(device: i32, k: i32, min_baseq: i32, thr: Thresholds, cands: &[Candidate<'_>],
-                samples: &mut [Box<dyn ReadSource>; 3], rank_world: Option<(i32, i32, [u8; 128])>,
-                regions: Option<Regions<'_>>) -> denovo_kmer_gpu::Result<Vec<bool>> {
-    let mut kc = Counter::new(device, k)?;
+                samples: &mut [Box<dyn ReadSource>; 3], second_child: Option<Box<dyn ReadSource>>,
+                rank_world: Option<(i32, i32, [u8; 128])>,
+                regions: Option<Regions<'_>>) -> denovo_kmer_gpu::Result<Vec<Vec<bool>>> {
+    let n_children = if second_child.is_some() { 2 } else { 1 };
+    let mut kc = Counter::new_family(device, k, n_children)?;
     kc.bind_thread_near_gpu()?;
     if let Some((rank, world, id)) = rank_world {
         kc.comm_init(&id, rank, world)?; // every rank scans its own slice of the read batches
@@ -39,7 +44,9 @@ pub fn run_trio(device: i32, k: i32, min_baseq: i32, thr: Thresholds, cands: &[C
     let (mut lo, mut hi) = (Vec::new(), Vec::new());
     let mut packer = kc.batch_packer(1 << 21, 150 << 21, min_baseq)?;
     let (mut seq, mut qual, mut off) = (Vec::new(), Vec::new(), Vec::new());
-    for (sample, src) in samples.iter_mut().enumerate() {
+    let mut second = second_child.into_iter().map(|src| (child_sample(1), src)).collect::<Vec<_>>();
+    let sources = samples.iter_mut().enumerate().chain(second.iter_mut().map(|(s, src)| (*s, src)));
+    for (sample, src) in sources {
         let mut in_flight = 0;
         while src.next_batch(&mut seq, &mut qual, &mut off) {
             if in_flight == 2 {
@@ -58,11 +65,14 @@ pub fn run_trio(device: i32, k: i32, min_baseq: i32, thr: Thresholds, cands: &[C
     }
     kc.counts_allreduce()?; // no-op without a communicator
     let res = kc.finalise(&thr)?;
-    Ok(res.calls.iter().map(|c| c & CALL_DENOVO != 0).collect())
+    // calls[v * n_children + c]: child c's byte for candidate v
+    Ok((0..n_children)
+        .map(|c| res.calls.iter().skip(c).step_by(n_children).map(|b| b & CALL_DENOVO != 0).collect())
+        .collect())
 }
 
 fn main() {
     // rank 0 of a multi-GPU job would make the id and send it round:
     let _ = comm_unique_id();
-    eprintln!("see run_trio(); the reference's CLI supplies the candidates and the three BAM readers");
+    eprintln!("see run_trio(); the reference's CLI supplies the candidates and the three (or four) BAM readers");
 }

@@ -25,6 +25,7 @@ pub const CHILD: i32 = 0;
 pub const MOTHER: i32 = 1;
 pub const FATHER: i32 = 2;
 pub const CALL_DENOVO: u8 = 0x01;
+pub use sys::{dkb_child_sample as child_sample, DKB_MAX_CHILDREN as MAX_CHILDREN};
 
 /// Error code of the C ABI plus the library's detail string.
 #[derive(Debug, Clone)]
@@ -97,20 +98,21 @@ pub fn variant_kmers(cands: &[Candidate<'_>], k: i32, drop_shared: bool) -> Resu
     Ok(e)
 }
 
-/// Per-variant results of kernel 3.
+/// Per-variant results of kernel 3 (`n_samples` = 3 for a trio, 2 + `n_children` for a family).
 pub struct Results {
-    /// `[n_variants][allele 0..2][sample 0..3]`
+    /// `[n_variants][allele 0..2][sample 0..n_samples]`
     pub hits: Vec<u32>,
     pub distinct: Vec<u32>,
     /// `[n_variants][allele 0..2]`
     pub n_kmers: Vec<u32>,
-    /// `DKB_CALL_*` bits per variant
+    /// `DKB_CALL_*` bits, `[n_variants][child 0..n_children]` (one per variant for a trio)
     pub calls: Vec<u8>,
 }
 
 /// One GPU context: table, streams, counters.  One per GPU, used from one thread at a time.
 pub struct Counter {
     ctx: *mut sys::DkbCtx,
+    n_children: usize,
     n_entries: usize,
     n_variants: usize,
     /// region mode: copies of the loci of batches in flight (the library reads them until `sync`)
@@ -120,11 +122,26 @@ pub struct Counter {
 unsafe impl Send for Counter {}
 
 impl Counter {
+    /// A trio context: child (sample 0), mother (1), father (2).
     pub fn new(device: i32, k: i32) -> Result<Self> {
         let mut ctx = ptr::null_mut();
         check(unsafe { sys::dkb_ctx_create(device, k, &mut ctx) }, ptr::null())?;
-        Ok(Counter { ctx, n_entries: 0, n_variants: 0, loci_keep: Vec::new(), _not_sync: PhantomData })
+        Ok(Counter { ctx, n_children: 1, n_entries: 0, n_variants: 0, loci_keep: Vec::new(), _not_sync: PhantomData })
     }
+
+    /// A family context: mother (sample 1), father (2) and `n_children` children (1..=6), child
+    /// `c` being sample [`child_sample`]`(c)`, all counted against one table; the de novo rule
+    /// is applied once per child.
+    pub fn new_family(device: i32, k: i32, n_children: usize) -> Result<Self> {
+        let mut ctx = ptr::null_mut();
+        let n = c_int::try_from(n_children).unwrap_or(c_int::MAX);
+        check(unsafe { sys::dkb_ctx_create_family(device, k, n, &mut ctx) }, ptr::null())?;
+        Ok(Counter { ctx, n_children, n_entries: 0, n_variants: 0, loci_keep: Vec::new(), _not_sync: PhantomData })
+    }
+
+    pub fn n_children(&self) -> usize { self.n_children }
+    /// 2 + n_children: the rows of the counters and the last axis of `hits` / `distinct`.
+    pub fn n_samples(&self) -> usize { 2 + self.n_children }
 
     fn ck(&self, code: c_int) -> Result<()> { check(code, self.ctx) }
 
@@ -212,9 +229,9 @@ impl Counter {
     }
     pub fn reset_counts(&mut self) -> Result<()> { self.ck(unsafe { sys::dkb_counts_reset(self.ctx) }) }
 
-    /// Per-entry counts, `[3 samples][n_entries]`.
+    /// Per-entry counts, `[n_samples][n_entries]`.
     pub fn entry_counts(&mut self) -> Result<Vec<u32>> {
-        let mut out = vec![0u32; 3 * self.n_entries];
+        let mut out = vec![0u32; self.n_samples() * self.n_entries];
         self.ck(unsafe { sys::dkb_entry_counts_fetch(self.ctx, out.as_mut_ptr()) })?;
         Ok(out)
     }
@@ -226,9 +243,9 @@ impl Counter {
     }
 
     pub fn results(&mut self) -> Result<Results> {
-        let nv = self.n_variants;
-        let mut r = Results { hits: vec![0; nv * 6], distinct: vec![0; nv * 6], n_kmers: vec![0; nv * 2],
-                              calls: vec![0; nv] };
+        let (nv, ns) = (self.n_variants, self.n_samples());
+        let mut r = Results { hits: vec![0; nv * 2 * ns], distinct: vec![0; nv * 2 * ns], n_kmers: vec![0; nv * 2],
+                              calls: vec![0; nv * self.n_children] };
         self.ck(unsafe {
             sys::dkb_results_fetch(self.ctx, r.hits.as_mut_ptr(), r.distinct.as_mut_ptr(),
                                    r.n_kmers.as_mut_ptr(), r.calls.as_mut_ptr())
@@ -254,7 +271,7 @@ impl Counter {
     pub fn reduce_push(&mut self, thr: &Thresholds) -> Result<()> { self.ck(unsafe { sys::dkb_reduce_push(self.ctx, thr) }) }
     pub fn reduce_flush(&mut self, thr: &Thresholds) -> Result<()> { self.ck(unsafe { sys::dkb_reduce_flush(self.ctx, thr) }) }
     pub fn reduced_counts(&mut self) -> Result<Vec<u32>> {
-        let mut out = vec![0u32; 3 * self.n_entries];
+        let mut out = vec![0u32; self.n_samples() * self.n_entries];
         self.ck(unsafe { sys::dkb_reduced_counts_fetch(self.ctx, out.as_mut_ptr()) })?;
         Ok(out)
     }

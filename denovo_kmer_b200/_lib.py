@@ -10,6 +10,7 @@ SO_PATH = os.environ.get("DKB_LIBRARY") or os.path.join(_HERE, "libdkb.so")  # o
 OK, EINVAL, ECUDA, ENOMEM, ESTATE, ENODEV, ENCCL = range(7)
 COMM_ID_BYTES = 128
 MAX_MULTI = 4
+MAX_CHILDREN = 6
 
 u8p = C.POINTER(C.c_uint8)
 u16p = C.POINTER(C.c_uint16)
@@ -42,6 +43,8 @@ SYMBOLS = {
     "dkb_strerror": (C.c_char_p, [C.c_int]),
     "dkb_last_error": (C.c_char_p, [C.c_void_p]),
     "dkb_ctx_create": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    "dkb_ctx_create_family": (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    "dkb_ctx_get_children": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),
     "dkb_ctx_destroy": (C.c_int, [C.c_void_p]),
     "dkb_ctx_set_tuning": (C.c_int, [C.c_void_p, C.POINTER(Tuning)]),
     "dkb_ctx_get_tuning": (C.c_int, [C.c_void_p, C.POINTER(Tuning)]),

@@ -19,6 +19,7 @@ CALL_DENOVO, CALL_CHILD_LOW, CALL_MOTHER_ALT, CALL_FATHER_ALT, CALL_PARENT_UNCOV
     0x01, 0x02, 0x04, 0x08, 0x10)
 DEFAULT_THRESHOLDS = (3, 2, 0, 1)
 DEFAULT_MIN_BASEQ = 20
+MAX_CHILDREN = _lib.MAX_CHILDREN
 
 
 def _p(a, t):
@@ -164,22 +165,36 @@ class ReadLoci:
 
 
 # ---- the counter -----------------------------------------------------------------------
+def child_sample(c: int) -> int:
+    """Sample index of child c of a family (DKB_CHILD_SAMPLE): 0 for c == 0, else 2 + c; the
+    mother stays 1 and the father 2."""
+    return 0 if c == 0 else c + 2
+
+
 class KmerCounter:
     """One GPU context: build the spanning-k-mer table, stream read batches per
-    sample, fetch per-entry / per-variant counts and de novo calls."""
+    sample, fetch per-entry / per-variant counts and de novo calls.
 
-    def __init__(self, k: int, device: int = 0, tuning=None):
+    n_children > 1 makes a family context: the mother (sample 1), the father (sample 2) and
+    n_children children (sample child_sample(c)) counted against one table, n_samples =
+    2 + n_children, and the de novo rule applied once per child."""
+
+    def __init__(self, k: int, device: int = 0, tuning=None, n_children: int = 1):
         self._L = _lib.lib()
         self._h = C.c_void_p()
         self.k = k
         self.device = device
-        check(self._L.dkb_ctx_create(device, k, C.byref(self._h)))
+        self.n_children = int(n_children)
+        self.n_samples = 2 + self.n_children
+        check(self._L.dkb_ctx_create_family(device, k, self.n_children, C.byref(self._h)))
         if tuning is not None:
             self.set_tuning(*tuning)
         self.n_entries = 0
         self.n_variants = 0
         self._keep = []  # host buffers of in-flight submits
         self._pinned = []  # dkb_host_alloc blocks
+
+    child_sample = staticmethod(child_sample)
 
     def close(self):
         if getattr(self, "_h", None):
@@ -282,7 +297,8 @@ class KmerCounter:
 
     def submit_device_multi(self, batches):
         """batches: up to 4 tuples (d_bases2, d_mask1, n_positions, sample) of resident
-        streams, scanned in ONE kernel launch (e.g. the three samples of a trio).  Not in
+        streams, scanned in ONE kernel launch (e.g. the three samples of a trio, or the four of
+        a quad).  Not in
         region mode."""
         n = len(batches)
         b = (C.c_void_p * n)(*[int(x[0]) for x in batches])
@@ -299,13 +315,14 @@ class KmerCounter:
         self._ck(self._L.dkb_counts_reset(self._h))
 
     def entry_counts(self) -> np.ndarray:
-        out = np.zeros((3, max(self.n_entries, 1)), dtype=np.uint32)
+        """[n_samples, n_entries] per-entry counters."""
+        out = np.zeros((self.n_samples, max(self.n_entries, 1)), dtype=np.uint32)
         self._ck(self._L.dkb_entry_counts_fetch(self._h, _p(out, u32p)))
         self._keep.clear()
         return out[:, : self.n_entries]
 
     def entry_counts_device(self):
-        """(device pointer, number of uint32) of the [3][n_entries] counters."""
+        """(device pointer, number of uint32) of the [n_samples][n_entries] counters."""
         p = C.c_void_p()
         n = C.c_size_t(0)
         self._ck(self._L.dkb_entry_counts_device(self._h, C.byref(p), C.byref(n)))
@@ -313,7 +330,7 @@ class KmerCounter:
 
     def finalise_launch(self, thresholds=DEFAULT_THRESHOLDS, counts_ptr=None):
         """Queue kernel 3 on the scan stream without waiting for it.  counts_ptr: device
-        pointer of a caller-owned copy of the [3][n_entries] counters (dkb_finalise_from)."""
+        pointer of a caller-owned copy of the [n_samples][n_entries] counters (dkb_finalise_from)."""
         t = Thresholds(*[int(x) for x in thresholds])
         if counts_ptr is None:
             self._ck(self._L.dkb_finalise(self._h, C.byref(t)))
@@ -321,16 +338,18 @@ class KmerCounter:
             self._ck(self._L.dkb_finalise_from(self._h, C.byref(t), C.c_void_p(int(counts_ptr))))
 
     def finalise(self, thresholds=DEFAULT_THRESHOLDS):
-        """Kernel 3 + fetch: (hits[nv,2,3], distinct[nv,2,3], n_kmers[nv,2], calls[nv])."""
+        """Kernel 3 + fetch: (hits[nv,2,n_samples], distinct[nv,2,n_samples], n_kmers[nv,2],
+        calls[nv] for a trio or calls[nv,n_children] for a family)."""
         self.finalise_launch(thresholds)
         return self.results()
 
     def results(self):
+        """(hits, distinct, n_kmers, calls) of the last finalise; shapes as in finalise()."""
         nv = max(self.n_variants, 1)
-        hits = np.zeros((nv, 2, 3), dtype=np.uint32)
-        dist = np.zeros((nv, 2, 3), dtype=np.uint32)
+        hits = np.zeros((nv, 2, self.n_samples), dtype=np.uint32)
+        dist = np.zeros((nv, 2, self.n_samples), dtype=np.uint32)
         nk = np.zeros((nv, 2), dtype=np.uint32)
-        calls = np.zeros(nv, dtype=np.uint8)
+        calls = np.zeros((nv, self.n_children) if self.n_children > 1 else nv, dtype=np.uint8)
         self._ck(self._L.dkb_results_fetch(self._h, _p(hits, u32p), _p(dist, u32p), _p(nk, u32p),
                                            _p(calls, u8p)))
         self._keep.clear()  # the fetch waited for the scan stream: every submit has been consumed
@@ -382,8 +401,8 @@ class KmerCounter:
         self._ck(self._L.dkb_reduce_flush(self._h, C.byref(t)))
 
     def reduced_counts(self) -> np.ndarray:
-        """Summed counters of the most recently finalised snapshot, [3, n_entries]."""
-        out = np.zeros((3, max(self.n_entries, 1)), dtype=np.uint32)
+        """Summed counters of the most recently finalised snapshot, [n_samples, n_entries]."""
+        out = np.zeros((self.n_samples, max(self.n_entries, 1)), dtype=np.uint32)
         self._ck(self._L.dkb_reduced_counts_fetch(self._h, _p(out, u32p)))
         return out[:, : self.n_entries]
 

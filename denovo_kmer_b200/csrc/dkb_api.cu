@@ -29,6 +29,7 @@ static_assert(DKB_MAX_MULTI == dkb::MAX_SEGMENTS, "ABI and kernel disagree on th
 struct dkb_ctx {
   int device = 0;
   int k = 0;
+  int n_children = 1, n_samples = DKB_N_SAMPLES;  // a family: 2 + n_children samples
   int n_sms = 0;
   std::string err;
 
@@ -60,7 +61,7 @@ struct dkb_ctx {
   bool want_pre = false;   // the tuner's choice
   uint64_t bloom_bits_set = 0;
   // counters and results
-  uint32_t *d_counts = nullptr;  // [3][n_entries]
+  uint32_t *d_counts = nullptr;  // [n_samples][n_entries]
   uint32_t *d_hits = nullptr, *d_distinct = nullptr, *d_nkmers = nullptr;
   uint8_t *d_calls = nullptr;
   bool finalised = false;
@@ -662,7 +663,7 @@ Nccl *nccl() {
 
 // Side stream, events and the two snapshot buffers of the overlapped reduction.
 int reduce_setup(dkb_ctx *ctx) {
-  const size_t need = (ctx->n_entries ? ctx->n_entries : 1) * 3;
+  const size_t need = (ctx->n_entries ? ctx->n_entries : 1) * ctx->n_samples;
   if (!ctx->s_side) {
     CU(cudaStreamCreateWithFlags(&ctx->s_side, cudaStreamNonBlocking));
     for (int i = 0; i < 2; i++) {
@@ -683,6 +684,14 @@ int reduce_setup(dkb_ctx *ctx) {
 }
 
 int finalise_counts(dkb_ctx *ctx, const dkb_thresholds *thr, const uint32_t *d_counts);
+
+// Samples a submit may name: [0, n_samples).
+int check_sample(dkb_ctx *ctx, int sample) {
+  if (sample >= 0 && sample < ctx->n_samples) return DKB_OK;
+  return fail(ctx, DKB_EINVAL, ctx->n_samples == DKB_N_SAMPLES
+                                   ? std::string("sample must be 0, 1 or 2")
+                                   : "sample must be in [0, " + std::to_string(ctx->n_samples) + ")");
+}
 
 // Kernel 3 on snapshot b, on the scan stream, once its sum over ranks is complete.
 int finalise_snapshot(dkb_ctx *ctx, const dkb_thresholds *thr, int b) {
@@ -713,11 +722,15 @@ const char *dkb_strerror(int code) {
 
 const char *dkb_last_error(const dkb_ctx *ctx) { return ctx ? ctx->err.c_str() : g_err.c_str(); }
 
-int dkb_ctx_create(int device, int k, dkb_ctx **out) {
+int dkb_ctx_create(int device, int k, dkb_ctx **out) { return dkb_ctx_create_family(device, k, 1, out); }
+
+int dkb_ctx_create_family(int device, int k, int n_children, dkb_ctx **out) {
   dkb_ctx *ctx = nullptr;
   if (!out) return fail(nullptr, DKB_EINVAL, "out is null");
   *out = nullptr;
   if (k < DKB_MIN_K || k > DKB_MAX_K) return fail(nullptr, DKB_EINVAL, "k out of range [8, 31]");
+  if (n_children < 1 || n_children > DKB_MAX_CHILDREN)
+    return fail(nullptr, DKB_EINVAL, "n_children out of range [1, " + std::to_string(DKB_MAX_CHILDREN) + "]");
   int n_dev = 0;
   if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev == 0) {
     cudaGetLastError();
@@ -735,6 +748,8 @@ int dkb_ctx_create(int device, int k, dkb_ctx **out) {
   if (!ctx) return fail(nullptr, DKB_ENOMEM, "host allocation failed");
   ctx->device = device;
   ctx->k = k;
+  ctx->n_children = n_children;
+  ctx->n_samples = 2 + n_children;
   ctx->n_sms = prop.multiProcessorCount;
   int rc = [&]() -> int {
     CU(cudaSetDevice(device));
@@ -807,6 +822,12 @@ int dkb_ctx_destroy(dkb_ctx *ctx) {
   return DKB_OK;
 }
 
+int dkb_ctx_get_children(const dkb_ctx *ctx, int *n_children_out) {
+  if (!ctx || !n_children_out) return fail(nullptr, DKB_EINVAL, "null argument");
+  *n_children_out = ctx->n_children;
+  return DKB_OK;
+}
+
 int dkb_ctx_set_tuning(dkb_ctx *ctx, const dkb_tuning *tuning) {
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
   ctx->user_tuning = tuning ? *tuning : dkb_tuning{0, 0, 0, 0};
@@ -847,7 +868,7 @@ int dkb_table_build(dkb_ctx *ctx, const uint64_t *keys, const uint32_t *variant_
 
   ctx->n_entries = n;
   ctx->n_variants = n_variants;
-  const size_t n1 = n ? n : 1, nv1 = n_variants ? n_variants : 1;
+  const size_t n1 = n ? n : 1, nv1 = n_variants ? n_variants : 1, ns = ctx->n_samples;
   int slots_per_entry = 8;
   if (const char *e = getenv("DKB_KEY_SLOTS_PER_ENTRY")) slots_per_entry = atoi(e) > 0 ? atoi(e) : 8;
   ctx->table_slots = pow2_at_least((uint64_t)slots_per_entry * n + 2);  // <= 0.25 entries per 2-slot bucket
@@ -867,14 +888,15 @@ int dkb_table_build(dkb_ctx *ctx, const uint64_t *keys, const uint32_t *variant_
     CU(cudaMalloc(&ctx->d_dead, n1));
     CU(cudaMalloc(&d_slot_of, n1 * 4));
     CU(cudaMalloc(&ctx->d_tslots, (size_t)ctx->table_slots * 16));
-    CU(cudaMalloc(&ctx->d_counts, n1 * 3 * 4));
-    CU(cudaMalloc(&ctx->d_hits, nv1 * 14 * 4));  // hits, distinct, n_kmers: one block, one memset per finalise
-    ctx->d_distinct = ctx->d_hits + nv1 * 6;
-    ctx->d_nkmers = ctx->d_hits + nv1 * 12;
-    CU(cudaMalloc(&ctx->d_calls, nv1));
+    CU(cudaMalloc(&ctx->d_counts, n1 * ns * 4));
+    // hits, distinct, n_kmers: one block of nv1 * (4 * ns + 2) words, one memset per finalise
+    CU(cudaMalloc(&ctx->d_hits, nv1 * (4 * ns + 2) * 4));
+    ctx->d_distinct = ctx->d_hits + nv1 * 2 * ns;
+    ctx->d_nkmers = ctx->d_hits + nv1 * 4 * ns;
+    CU(cudaMalloc(&ctx->d_calls, nv1 * ctx->n_children));
     CU(cudaMalloc(&d_nseeds, 4));
     CU(cudaMemsetAsync(ctx->d_tslots, 0xFF, (size_t)ctx->table_slots * 16, st));
-    CU(cudaMemsetAsync(ctx->d_counts, 0, n1 * 3 * 4, st));
+    CU(cudaMemsetAsync(ctx->d_counts, 0, n1 * ns * 4, st));
     CU(cudaMemsetAsync(ctx->d_dead, 0, n1, st));
     CU(cudaMemsetAsync(d_nseeds, 0, 4, st));
     if (n) {
@@ -1004,7 +1026,7 @@ int dkb_batch_submit_device(dkb_ctx *ctx, const uint32_t *d_bases2, const uint32
                             uint64_t n_positions, int sample) {
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
   if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
-  if (sample < 0 || sample >= DKB_N_SAMPLES) return fail(ctx, DKB_EINVAL, "sample must be 0, 1 or 2");
+  if (check_sample(ctx, sample) != DKB_OK) return DKB_EINVAL;
   dkb_ctx::Loci loci;
   int rc = take_loci(ctx, n_positions, &loci);
   if (rc != DKB_OK) return rc;
@@ -1028,7 +1050,7 @@ int dkb_batch_submit_device_multi(dkb_ctx *ctx, int n_batches, const uint32_t *c
   if (n_batches < 0 || n_batches > DKB_MAX_MULTI) return fail(ctx, DKB_EINVAL, "n_batches out of range");
   if (n_batches && (!d_bases2 || !d_mask1 || !n_positions || !samples)) return fail(ctx, DKB_EINVAL, "null argument");
   for (int i = 0; i < n_batches; i++) {
-    if (samples[i] < 0 || samples[i] >= DKB_N_SAMPLES) return fail(ctx, DKB_EINVAL, "sample must be 0, 1 or 2");
+    if (check_sample(ctx, samples[i]) != DKB_OK) return DKB_EINVAL;
     if (n_positions[i] == 0) continue;
     if (n_positions[i] > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
     if (!d_bases2[i] || !d_mask1[i]) return fail(ctx, DKB_EINVAL, "null stream pointer");
@@ -1043,7 +1065,7 @@ int dkb_batch_submit(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t *mask1
                      uint64_t n_positions, int sample) {
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
   if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
-  if (sample < 0 || sample >= DKB_N_SAMPLES) return fail(ctx, DKB_EINVAL, "sample must be 0, 1 or 2");
+  if (check_sample(ctx, sample) != DKB_OK) return DKB_EINVAL;
   dkb_ctx::Loci loci;
   int rc = take_loci(ctx, n_positions, &loci);
   if (rc != DKB_OK) return rc;
@@ -1078,7 +1100,7 @@ int dkb_batch_submit_sparse(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t
                             const uint8_t *zbytes, size_t zbytes_used, uint64_t n_positions, int sample) {
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
   if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
-  if (sample < 0 || sample >= DKB_N_SAMPLES) return fail(ctx, DKB_EINVAL, "sample must be 0, 1 or 2");
+  if (check_sample(ctx, sample) != DKB_OK) return DKB_EINVAL;
   dkb_ctx::Loci loci;
   int rc = take_loci(ctx, n_positions, &loci);
   if (rc != DKB_OK) return rc;
@@ -1127,7 +1149,7 @@ int dkb_batch_submit_reads(dkb_ctx *ctx, const uint8_t *seq, int seq_format, con
                            const uint64_t *offsets, size_t n_reads, int min_baseq, int sample) {
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
   if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
-  if (sample < 0 || sample >= DKB_N_SAMPLES) return fail(ctx, DKB_EINVAL, "sample must be 0, 1 or 2");
+  if (check_sample(ctx, sample) != DKB_OK) return DKB_EINVAL;
   if (seq_format != 0 && seq_format != 1) return fail(ctx, DKB_EINVAL, "seq_format must be 0 (ASCII) or 1 (BAM 4-bit)");
   dkb_ctx::Loci loci;
   if (n_reads == 0) return take_loci(ctx, 0, &loci);
@@ -1265,7 +1287,7 @@ int dkb_counts_reset(dkb_ctx *ctx) {
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
   if (!ctx->d_counts) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
   CU(cudaSetDevice(ctx->device));
-  CU(cudaMemsetAsync(ctx->d_counts, 0, (ctx->n_entries ? ctx->n_entries : 1) * 3 * 4, ctx->s_scan));
+  CU(cudaMemsetAsync(ctx->d_counts, 0, (ctx->n_entries ? ctx->n_entries : 1) * ctx->n_samples * 4, ctx->s_scan));
   if (ctx->prof) CU(cudaMemsetAsync(ctx->d_prof, 0, 4 * sizeof(unsigned long long), ctx->s_scan));
   ctx->finalised = false;
   return DKB_OK;
@@ -1276,7 +1298,7 @@ int dkb_entry_counts_fetch(dkb_ctx *ctx, uint32_t *out) {
   if (!ctx->d_counts) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
   CU(cudaSetDevice(ctx->device));
   CU(cudaStreamSynchronize(ctx->s_copy));
-  CU(cudaMemcpyAsync(out, ctx->d_counts, ctx->n_entries * 3 * 4, cudaMemcpyDeviceToHost, ctx->s_scan));
+  CU(cudaMemcpyAsync(out, ctx->d_counts, ctx->n_entries * ctx->n_samples * 4, cudaMemcpyDeviceToHost, ctx->s_scan));
   CU(cudaStreamSynchronize(ctx->s_scan));
   return DKB_OK;
 }
@@ -1285,7 +1307,7 @@ int dkb_entry_counts_device(dkb_ctx *ctx, void **d_ptr, size_t *n_u32) {
   if (!ctx || !d_ptr || !n_u32) return fail(ctx, DKB_EINVAL, "null argument");
   if (!ctx->d_counts) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
   *d_ptr = ctx->d_counts;
-  *n_u32 = ctx->n_entries * 3;
+  *n_u32 = ctx->n_entries * ctx->n_samples;
   return DKB_OK;
 }
 
@@ -1305,20 +1327,35 @@ int dkb_finalise_from(dkb_ctx *ctx, const dkb_thresholds *thr, const uint32_t *d
 }  // extern "C"
 
 namespace {
-int finalise_counts(dkb_ctx *ctx, const dkb_thresholds *thr, const uint32_t *d_counts) {
+// Kernel 3 for NS samples.
+template <int NS>
+void launch_finalise(dkb_ctx *ctx, const Thresholds &T, const uint32_t *d_counts) {
   cudaStream_t st = ctx->s_scan;
-  const size_t nv1 = ctx->n_variants ? ctx->n_variants : 1;
-  CU(cudaMemsetAsync(ctx->d_hits, 0, nv1 * 14 * 4, st));
   const int TB = 256;
   if (ctx->n_entries)
-    k_variant_reduce<<<(uint32_t)((ctx->n_entries + TB - 1) / TB), TB, 0, st>>>(
+    k_variant_reduce<NS><<<(uint32_t)((ctx->n_entries + TB - 1) / TB), TB, 0, st>>>(
         d_counts, ctx->d_variant, ctx->d_allele, ctx->d_dead, (uint32_t)ctx->n_entries,
         ctx->d_hits, ctx->d_distinct, ctx->d_nkmers);
+  const uint32_t n_items = ctx->n_variants * (uint32_t)(NS - 2);  // (variant, child) pairs
+  if (n_items)
+    k_calls<NS><<<(n_items + TB - 1) / TB, TB, 0, st>>>(ctx->d_hits, ctx->d_distinct, n_items, T, ctx->d_calls);
+}
+
+int finalise_counts(dkb_ctx *ctx, const dkb_thresholds *thr, const uint32_t *d_counts) {
+  const size_t nv1 = ctx->n_variants ? ctx->n_variants : 1;
+  CU(cudaMemsetAsync(ctx->d_hits, 0, nv1 * (4 * (size_t)ctx->n_samples + 2) * 4, ctx->s_scan));
   Thresholds T{thr->min_child_alt_hits, thr->min_child_alt_distinct, thr->max_parent_alt_hits,
                thr->min_parent_ref_hits};
-  if (ctx->n_variants)
-    k_calls<<<(ctx->n_variants + TB - 1) / TB, TB, 0, st>>>(ctx->d_hits, ctx->d_distinct,
-                                                            ctx->n_variants, T, ctx->d_calls);
+  static_assert(DKB_MAX_CHILDREN == 6, "one kernel-3 instantiation per family size");
+  switch (ctx->n_samples) {
+    case 3: launch_finalise<3>(ctx, T, d_counts); break;
+    case 4: launch_finalise<4>(ctx, T, d_counts); break;
+    case 5: launch_finalise<5>(ctx, T, d_counts); break;
+    case 6: launch_finalise<6>(ctx, T, d_counts); break;
+    case 7: launch_finalise<7>(ctx, T, d_counts); break;
+    case 8: launch_finalise<8>(ctx, T, d_counts); break;
+    default: return fail(ctx, DKB_EINVAL, "no kernel 3 for this family size");
+  }
   CU(cudaGetLastError());
   ctx->finalised = true;
   return DKB_OK;
@@ -1386,7 +1423,7 @@ int dkb_counts_allreduce(dkb_ctx *ctx) {
   if (!ctx->comm || ctx->world == 1) return DKB_OK;
   CU(cudaSetDevice(ctx->device));
   if (ctx->n_entries)
-    NC(nccl()->AllReduce(ctx->d_counts, ctx->d_counts, ctx->n_entries * 3, NCCL_UINT32, NCCL_SUM,
+    NC(nccl()->AllReduce(ctx->d_counts, ctx->d_counts, ctx->n_entries * ctx->n_samples, NCCL_UINT32, NCCL_SUM,
                          ctx->comm, ctx->s_scan));
   ctx->finalised = false;
   return DKB_OK;
@@ -1400,7 +1437,7 @@ int dkb_reduce_push(dkb_ctx *ctx, const dkb_thresholds *thr) {
   if (rc != DKB_OK) return rc;
   const int b = ctx->red_next;
   ctx->red_next ^= 1;
-  const size_t n = ctx->n_entries * 3;
+  const size_t n = ctx->n_entries * ctx->n_samples;
   // snapshot on the scan stream (behind this batch's scans) ...
   if (n) CU(cudaMemcpyAsync(ctx->d_red[b], ctx->d_counts, n * 4, cudaMemcpyDeviceToDevice, ctx->s_scan));
   CU(cudaEventRecord(ctx->ev_snap[b], ctx->s_scan));
@@ -1428,7 +1465,7 @@ int dkb_reduced_counts_fetch(dkb_ctx *ctx, uint32_t *out) {
   if (!ctx || !out) return fail(ctx, DKB_EINVAL, "null argument");
   if (ctx->red_last < 0) return fail(ctx, DKB_ESTATE, "no reduced batch has been finalised yet");
   CU(cudaSetDevice(ctx->device));
-  CU(cudaMemcpyAsync(out, ctx->d_red[ctx->red_last], ctx->n_entries * 3 * 4, cudaMemcpyDeviceToHost,
+  CU(cudaMemcpyAsync(out, ctx->d_red[ctx->red_last], ctx->n_entries * ctx->n_samples * 4, cudaMemcpyDeviceToHost,
                      ctx->s_scan));
   CU(cudaStreamSynchronize(ctx->s_scan));
   return DKB_OK;
@@ -1440,11 +1477,11 @@ int dkb_results_fetch(dkb_ctx *ctx, uint32_t *hits, uint32_t *distinct, uint32_t
   if (!ctx->finalised) return fail(ctx, DKB_ESTATE, "dkb_finalise must come first");
   CU(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->s_scan;
-  const size_t nv = ctx->n_variants;
-  if (hits) CU(cudaMemcpyAsync(hits, ctx->d_hits, nv * 6 * 4, cudaMemcpyDeviceToHost, st));
-  if (distinct) CU(cudaMemcpyAsync(distinct, ctx->d_distinct, nv * 6 * 4, cudaMemcpyDeviceToHost, st));
+  const size_t nv = ctx->n_variants, ns = ctx->n_samples;
+  if (hits) CU(cudaMemcpyAsync(hits, ctx->d_hits, nv * 2 * ns * 4, cudaMemcpyDeviceToHost, st));
+  if (distinct) CU(cudaMemcpyAsync(distinct, ctx->d_distinct, nv * 2 * ns * 4, cudaMemcpyDeviceToHost, st));
   if (n_kmers) CU(cudaMemcpyAsync(n_kmers, ctx->d_nkmers, nv * 2 * 4, cudaMemcpyDeviceToHost, st));
-  if (calls) CU(cudaMemcpyAsync(calls, ctx->d_calls, nv, cudaMemcpyDeviceToHost, st));
+  if (calls) CU(cudaMemcpyAsync(calls, ctx->d_calls, nv * ctx->n_children, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
   return DKB_OK;
 }

@@ -284,7 +284,9 @@ __global__ void k_assign_seeds(const BuildParams B, int pass, uint32_t *set, uin
 }
 
 // ---- kernel 3: finalise -----------------------------------------------------
-// counts: [3][n]; hits/distinct: [n_variants][2][3]; n_kmers: [n_variants][2]
+// NS samples (3: a trio; 2 + n_children in a family).
+// counts: [NS][n]; hits/distinct: [n_variants][2][NS]; n_kmers: [n_variants][2]
+template <int NS>
 __global__ void k_variant_reduce(const uint32_t *counts, const uint32_t *variant,
                                  const uint8_t *allele, const uint8_t *dead, uint32_t n,
                                  uint32_t *hits, uint32_t *distinct, uint32_t *n_kmers) {
@@ -294,27 +296,27 @@ __global__ void k_variant_reduce(const uint32_t *counts, const uint32_t *variant
   // them so): the lanes of a warp that share an owner add up among themselves (REDUX) and one
   // of them issues the atomics - ~10x fewer than one set per entry.  Any order stays correct.
   const uint32_t va = live ? variant[i] * 2u + allele[i] : 0xFFFFFFFFu;
-  uint32_t c[3] = {0, 0, 0};
+  uint32_t c[NS] = {};
   if (live) {
 #pragma unroll
-    for (int smp = 0; smp < 3; smp++) c[smp] = counts[(size_t)smp * n + i];
+    for (int smp = 0; smp < NS; smp++) c[smp] = counts[(size_t)smp * n + i];
   }
   const unsigned peers = __match_any_sync(FULL_MASK, va);
   const bool leader = live && (__ffs(peers) - 1) == (int)(threadIdx.x & 31);
   const uint32_t nk = __reduce_add_sync(peers, live ? 1u : 0u);
-  uint32_t h[3], d[3];
+  uint32_t h[NS], d[NS];
 #pragma unroll
-  for (int smp = 0; smp < 3; smp++) {
+  for (int smp = 0; smp < NS; smp++) {
     h[smp] = __reduce_add_sync(peers, c[smp]);
     d[smp] = __reduce_add_sync(peers, c[smp] ? 1u : 0u);
   }
   if (!leader) return;
   atomicAdd(n_kmers + va, nk);
 #pragma unroll
-  for (int smp = 0; smp < 3; smp++) {
+  for (int smp = 0; smp < NS; smp++) {
     if (h[smp]) {
-      atomicAdd(hits + (size_t)va * 3 + smp, h[smp]);
-      atomicAdd(distinct + (size_t)va * 3 + smp, d[smp]);
+      atomicAdd(hits + (size_t)va * NS + smp, h[smp]);
+      atomicAdd(distinct + (size_t)va * NS + smp, d[smp]);
     }
   }
 }
@@ -323,17 +325,23 @@ struct Thresholds {
   uint32_t min_child_alt_hits, min_child_alt_distinct, max_parent_alt_hits, min_parent_ref_hits;
 };
 
-__global__ void k_calls(const uint32_t *hits, const uint32_t *distinct, uint32_t n_variants,
+// One thread per (variant, child): the trio rule on child ch's alt support and the parents'
+// hits; calls: [n_variants][NS - 2].  n_items = n_variants * (NS - 2).
+template <int NS>
+__global__ void k_calls(const uint32_t *hits, const uint32_t *distinct, uint32_t n_items,
                         const Thresholds T, uint8_t *calls) {
-  const uint32_t v = blockIdx.x * blockDim.x + threadIdx.x;
-  if (v >= n_variants) return;
-  const uint32_t *h = hits + (size_t)v * 6, *d = distinct + (size_t)v * 6;  // [allele*3+sample]
+  constexpr uint32_t NC = NS - 2;
+  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_items) return;
+  const uint32_t v = t / NC, ch = t % NC;
+  const uint32_t cs = ch == 0 ? 0 : ch + 2;  // DKB_CHILD_SAMPLE
+  const uint32_t *h = hits + (size_t)v * 2 * NS, *d = distinct + (size_t)v * 2 * NS;  // [allele*NS+sample]
   uint8_t c = 0;
-  if (h[3] < T.min_child_alt_hits || d[3] < T.min_child_alt_distinct) c |= 0x02;
-  if (h[4] > T.max_parent_alt_hits) c |= 0x04;
-  if (h[5] > T.max_parent_alt_hits) c |= 0x08;
+  if (h[NS + cs] < T.min_child_alt_hits || d[NS + cs] < T.min_child_alt_distinct) c |= 0x02;
+  if (h[NS + 1] > T.max_parent_alt_hits) c |= 0x04;
+  if (h[NS + 2] > T.max_parent_alt_hits) c |= 0x08;
   if (h[1] < T.min_parent_ref_hits || h[2] < T.min_parent_ref_hits) c |= 0x10;
-  calls[v] = c ? c : 0x01;
+  calls[t] = c ? c : 0x01;
 }
 
 }  // namespace dkb

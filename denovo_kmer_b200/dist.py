@@ -30,7 +30,7 @@ class _DevArray:
 
 
 def counts_tensor(kc):
-    """torch int32 view (no copy) of the context's [3][n_entries] device counters (tests and
+    """torch int32 view (no copy) of the context's [n_samples][n_entries] device counters (tests and
     checks; the product's own sum over ranks never leaves the library)."""
     import torch
     ptr, n = kc.entry_counts_device()

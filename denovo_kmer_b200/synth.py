@@ -5,7 +5,8 @@ here counts k-mers.
 
 Two generators with the same model:
   * `make_trio_host`   — NumPy, decoded reads (ASCII + qualities), for parity tests and
-                         the CPU baseline sample;
+                         the CPU baseline sample (`make_family_host`: the same for a family
+                         of one mother, one father and several children);
   * `make_sample_device` — PyTorch on the GPU, emits the packed stream (2-bit bases +
                          1-bit flags + separators) directly in HBM for the bench.
 """
@@ -25,6 +26,10 @@ class Variant:
     ref: str
     alt: str
     inherited: bool = False  # also carried by the mother (should NOT be called de novo)
+    # family generator: the child that owns the variant, and the children that carry it (the
+    # trio generators: child 0 carries every variant)
+    owner: int = 0
+    carriers: frozenset = frozenset({0})
 
 
 @dataclass
@@ -36,6 +41,7 @@ class Trio:
     # sample -> (lo, hi) uint64: each read's true alignment interval [lo, hi) in genome coordinates
     loci: dict = field(default_factory=dict)
     paralogs: list = field(default_factory=list)  # indices of the variants given a paralog copy
+    n_children: int = 1  # reads / loci of child c are under sample child_sample(c)
 
     def variant_tuples(self):
         """(left flank, ref, alt, right flank) per variant, flanks k-1 long (shorter at ends)."""
@@ -223,6 +229,60 @@ def make_trio_host(genome_len: int, depth: float, n_variants: int, k: int, seed:
         trio.reads[smp] = (seq, qual, off)
         trio.loci[smp] = read_loci(refpos[smp], hap_of, starts, np.diff(off).astype(np.int64))
     return trio
+
+
+def child_sample(c: int) -> int:
+    """Sample index of child c of a family (DKB_CHILD_SAMPLE in include/dkb.h): 0 for c == 0,
+    else 2 + c.  (Kept here, not imported from the api: generating data loads no library.)"""
+    return 0 if c == 0 else c + 2
+
+
+def make_family_host(genome_len: int, depth: float, n_variants: int, k: int, n_children: int, seed: int = 1,
+                     shared_frac: float = 0.2, inherited_frac: float = 0.2, indel_frac: float = 0.0,
+                     paralog_frac: float = 0.0, read_len: int = 150, ragged: bool = False, **read_kw) -> Trio:
+    """A family: mother (sample 1), father (sample 2) and n_children children (sample
+    child_sample(c)), reads and loci keyed by sample index.  Variant i is owned by child
+    i % n_children; each is, drawn independently:
+      * inherited (inherited_frac): the mother carries it, each child with probability 1/2;
+      * shared de novo (shared_frac, two children or more): the owner and one other child carry
+        it, neither parent does (gonadal mosaicism in a parent);
+      * de novo otherwise: only the owner carries it.
+    Every child carrying a variant is heterozygous for it.  paralog_frac: that fraction of the
+    variants not inherited gets an ALT-carrying copy far away (plant_paralogs)."""
+    genome = make_genome(genome_len, seed)
+    variants = plant_variants(genome, n_variants, k, seed + 1, indel_frac=indel_frac, inherited_frac=0.0)
+    rng = np.random.default_rng(seed + 2)
+    for i, v in enumerate(variants):
+        v.owner = i % n_children
+        r = rng.random()
+        if r < inherited_frac:
+            v.inherited = True
+            v.carriers = frozenset(int(c) for c in np.nonzero(rng.random(n_children) < 0.5)[0])
+        elif r < inherited_frac + shared_frac and n_children > 1:
+            other = (v.owner + 1 + int(rng.integers(0, n_children - 1))) % n_children
+            v.carriers = frozenset({v.owner, other})
+        else:
+            v.carriers = frozenset({v.owner})
+    paralogs = []
+    if paralog_frac > 0:
+        prng = np.random.default_rng(seed + 3)
+        denovo = [i for i, v in enumerate(variants) if not v.inherited]
+        paralogs = sorted(prng.choice(denovo, size=max(1, int(round(paralog_frac * len(denovo)))),
+                                      replace=False).tolist())
+        genome = plant_paralogs(genome, variants, k, paralogs, seed + 4)
+    carried = {1: [v for v in variants if v.inherited], 2: []}
+    for c in range(n_children):
+        carried[child_sample(c)] = [v for v in variants if c in v.carriers]
+    n_reads = int(len(genome) * depth / read_len)
+    fam = Trio(k, genome, variants, paralogs=paralogs, n_children=n_children)
+    for smp in sorted(carried):
+        alt = apply_variants(genome, carried[smp])
+        refpos = [None, hap_ref_positions(genome, carried[smp])]
+        seq, qual, off, (hap_of, starts) = sample_reads([genome, alt], n_reads, read_len, seed + 10 + smp,
+                                                        ragged=ragged, return_meta=True, **read_kw)
+        fam.reads[smp] = (seq, qual, off)
+        fam.loci[smp] = read_loci(refpos, hap_of, starts, np.diff(off).astype(np.int64))
+    return fam
 
 
 # ---------------------------------------------------------------------------------------

@@ -45,6 +45,13 @@ extern "C" {
 #define DKB_MIN_K 8
 #define DKB_MAX_K 31
 #define DKB_N_SAMPLES 3 /* 0 child, 1 mother, 2 father */
+/* Family contexts (dkb_ctx_create_family): one mother, one father and n_children children counted
+ * against one table, NS = 2 + n_children samples.  Mother stays sample 1 and father sample 2, so
+ * a one-child family IS a trio.  Every array laid out with DKB_N_SAMPLES below holds NS samples
+ * in a family context. */
+#define DKB_MAX_CHILDREN 6 /* a family has at most 2 + 6 = 8 samples */
+/* sample index of child c (0 <= c < n_children): 0 for c == 0, else 2 + c */
+#define DKB_CHILD_SAMPLE(c) ((c) == 0 ? 0 : (c) + 2)
 #define DKB_N_ALLELES 2 /* 0 ref, 1 alt (multi-allelic sites are split by the host) */
 
 enum {
@@ -59,8 +66,9 @@ enum {
 
 typedef struct dkb_ctx dkb_ctx;
 
-/* De novo support rule (integer only).  A variant is called (bit 0 of the
- * call byte) iff
+/* De novo support rule (integer only), applied once per child of a family: the clauses
+ * name that child's alt hits and distinct k-mers, and both parents' hits.  A variant is
+ * called (bit 0 of the call byte) iff
  *   child  alt hits     >= min_child_alt_hits      and
  *   child  alt distinct >= min_child_alt_distinct  and
  *   mother alt hits     <= max_parent_alt_hits     and
@@ -98,7 +106,13 @@ const char *dkb_strerror(int code);
 const char *dkb_last_error(const dkb_ctx *ctx);
 
 /* ---- context ---------------------------------------------------------- */
+/* A trio: dkb_ctx_create_family(device, k, 1, out). */
 int dkb_ctx_create(int device, int k, dkb_ctx **out);
+/* A family of n_children children (1..DKB_MAX_CHILDREN; DKB_EINVAL otherwise, checked before
+ * the device) and both parents.  Submits take sample in [0, NS): DKB_CHILD_SAMPLE(c) for child
+ * c, 1 for the mother, 2 for the father. */
+int dkb_ctx_create_family(int device, int k, int n_children, dkb_ctx **out);
+int dkb_ctx_get_children(const dkb_ctx *ctx, int *n_children_out);
 int dkb_ctx_destroy(dkb_ctx *ctx);
 int dkb_ctx_set_tuning(dkb_ctx *ctx, const dkb_tuning *tuning);
 int dkb_ctx_get_tuning(const dkb_ctx *ctx, dkb_tuning *out);
@@ -172,7 +186,8 @@ int dkb_table_build(dkb_ctx *ctx, const uint64_t *keys, const uint32_t *variant_
 /* ---- kernel 2: streaming extract-and-probe ------------------------------- */
 /* Host buffers (pinned for full speed); H2D copy + scan are queued on the
  * context's streams and overlap with the next submit.  The buffers must stay
- * valid until dkb_sync. */
+ * valid until dkb_sync.  sample: 0..2 in a trio, [0, NS) in a family (DKB_EINVAL otherwise),
+ * in every submit form below. */
 int dkb_batch_submit(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t *mask1,
                      uint64_t n_positions, int sample);
 /* Same as dkb_batch_submit with the flags as a zero list (above): bases2 + zoff + zbytes cross
@@ -191,7 +206,7 @@ int dkb_batch_submit_reads(dkb_ctx *ctx, const uint8_t *seq, int seq_format, con
  * dkb_stream_*_words long.  Flags at positions >= n_positions are ignored. */
 int dkb_batch_submit_device(dkb_ctx *ctx, const uint32_t *d_bases2, const uint32_t *d_mask1,
                             uint64_t n_positions, int sample);
-/* Up to DKB_MAX_MULTI device-resident streams (e.g. the three samples of a trio) in ONE kernel
+/* Up to DKB_MAX_MULTI device-resident streams (e.g. the three samples of a trio, or a quad's four) in ONE kernel
  * launch; batch i goes into the counters of samples[i].  Same alignment rules; a batch of 0
  * positions is skipped.  Worth it for short batches, where a launch costs as much as the scan. */
 #define DKB_MAX_MULTI 4
@@ -227,20 +242,22 @@ int dkb_batch_set_loci(dkb_ctx *ctx, const uint64_t *offsets, const uint64_t *lo
 int dkb_sync(dkb_ctx *ctx);
 int dkb_counts_reset(dkb_ctx *ctx);
 
-/* per-entry counts, layout [DKB_N_SAMPLES][n_entries] */
+/* per-entry counts, layout [DKB_N_SAMPLES][n_entries]; [NS][n_entries] in a family */
 int dkb_entry_counts_fetch(dkb_ctx *ctx, uint32_t *out);
-/* device pointer of the same array, for the multi-GPU sum (NCCL allreduce) */
+/* device pointer of the same array, for the multi-GPU sum (NCCL allreduce); *n_u32 =
+ * NS * n_entries */
 int dkb_entry_counts_device(dkb_ctx *ctx, void **d_ptr, size_t *n_u32);
 
 /* ---- kernel 3: finalise ---------------------------------------------------- */
 int dkb_finalise(dkb_ctx *ctx, const dkb_thresholds *thr);
-/* Same, from a caller-owned DEVICE copy of the counters ([DKB_N_SAMPLES][n_entries], the
-   layout of dkb_entry_counts_device) - e.g. a copy that is being summed over ranks while
+/* Same, from a caller-owned DEVICE copy of the counters ([DKB_N_SAMPLES][n_entries], or
+   [NS][n_entries] in a family: the layout of dkb_entry_counts_device) - e.g. a copy that is being summed over ranks while
    the context's own counters already take the next batch.  Runs on the scan stream: order
    it after the copy is complete (dkb_scan_stream). */
 int dkb_finalise_from(dkb_ctx *ctx, const dkb_thresholds *thr, const uint32_t *d_counts);
-/* hits / distinct: [n_variants][DKB_N_ALLELES][DKB_N_SAMPLES]; n_kmers:
- * [n_variants][DKB_N_ALLELES]; calls: [n_variants].  Any pointer may be NULL. */
+/* hits / distinct: [n_variants][DKB_N_ALLELES][DKB_N_SAMPLES] ([n_variants][2][NS] in a
+ * family); n_kmers: [n_variants][DKB_N_ALLELES]; calls: [n_variants][n_children], child c's
+ * byte at calls[v * n_children + c] (a trio: [n_variants]).  Any pointer may be NULL. */
 int dkb_results_fetch(dkb_ctx *ctx, uint32_t *hits, uint32_t *distinct, uint32_t *n_kmers,
                       uint8_t *calls);
 
@@ -278,6 +295,7 @@ int dkb_comm_info(const dkb_ctx *ctx, int *rank, int *world, int *nccl_version);
 int dkb_counts_allreduce(dkb_ctx *ctx);
 int dkb_reduce_push(dkb_ctx *ctx, const dkb_thresholds *thr);
 int dkb_reduce_flush(dkb_ctx *ctx, const dkb_thresholds *thr);
+/* [DKB_N_SAMPLES][n_entries], [NS][n_entries] in a family */
 int dkb_reduced_counts_fetch(dkb_ctx *ctx, uint32_t *out);
 
 /* ---- introspection (bench / tests) --------------------------------------- */

@@ -79,16 +79,19 @@ inline Stream pack_reads(const std::vector<uint8_t> &seq, const std::vector<uint
 }
 
 struct Results {
-  std::vector<uint32_t> hits, distinct;  // [n_variants][2 alleles][3 samples]
+  std::vector<uint32_t> hits, distinct;  // [n_variants][2 alleles][n_samples]
   std::vector<uint32_t> n_kmers;         // [n_variants][2]
-  std::vector<uint8_t> calls;            // [n_variants], DKB_CALL_* bits
+  std::vector<uint8_t> calls;            // [n_variants][n_children], DKB_CALL_* bits
 };
 
 // One GPU context.  Throws Error{DKB_ENODEV} when no sm_100 device exists: there is no
-// CPU fallback.
+// CPU fallback.  n_children > 1: a family (dkb_ctx_create_family) - mother 1, father 2, child
+// c at DKB_CHILD_SAMPLE(c), n_samples() = 2 + n_children.
 class Counter {
  public:
-  Counter(int k, int device = 0) { check(dkb_ctx_create(device, k, &ctx_)); }
+  Counter(int k, int device = 0, int n_children = 1) : n_children_(n_children) {
+    check(dkb_ctx_create_family(device, k, n_children, &ctx_));
+  }
   ~Counter() { dkb_ctx_destroy(ctx_); }
   Counter(const Counter &) = delete;
   Counter &operator=(const Counter &) = delete;
@@ -162,32 +165,36 @@ class Counter {
   }
   void sync() { check(dkb_sync(ctx_), ctx_); }
   void reset_counts() { check(dkb_counts_reset(ctx_), ctx_); }
-  std::vector<uint32_t> entry_counts() {  // [3 samples][n_entries]
-    std::vector<uint32_t> out(3 * n_entries_ + 1);
+  int n_children() const { return n_children_; }
+  size_t n_samples() const { return 2 + (size_t)n_children_; }
+  std::vector<uint32_t> entry_counts() {  // [n_samples][n_entries]
+    std::vector<uint32_t> out(n_samples() * n_entries_ + 1);
     check(dkb_entry_counts_fetch(ctx_, out.data()), ctx_);
-    out.resize(3 * n_entries_);
+    out.resize(n_samples() * n_entries_);
     return out;
   }
   // d_counts: optional caller-owned DEVICE copy of the counters (dkb_finalise_from)
   Results finalise(const dkb_thresholds &t, const uint32_t *d_counts = nullptr) {
     check(d_counts ? dkb_finalise_from(ctx_, &t, d_counts) : dkb_finalise(ctx_, &t), ctx_);
     Results r;
-    r.hits.resize(6 * (size_t)n_variants_ + 1);
-    r.distinct.resize(6 * (size_t)n_variants_ + 1);
+    const size_t nh = 2 * n_samples() * n_variants_, nc = (size_t)n_children_ * n_variants_;
+    r.hits.resize(nh + 1);
+    r.distinct.resize(nh + 1);
     r.n_kmers.resize(2 * (size_t)n_variants_ + 1);
-    r.calls.resize((size_t)n_variants_ + 1);
+    r.calls.resize(nc + 1);
     check(dkb_results_fetch(ctx_, r.hits.data(), r.distinct.data(), r.n_kmers.data(), r.calls.data()),
           ctx_);
-    r.hits.resize(6 * (size_t)n_variants_);
-    r.distinct.resize(6 * (size_t)n_variants_);
+    r.hits.resize(nh);
+    r.distinct.resize(nh);
     r.n_kmers.resize(2 * (size_t)n_variants_);
-    r.calls.resize(n_variants_);
+    r.calls.resize(nc);
     return r;
   }
   dkb_ctx *raw() { return ctx_; }
 
  private:
   dkb_ctx *ctx_ = nullptr;
+  int n_children_ = 1;
   size_t n_entries_ = 0;
   uint32_t n_variants_ = 0;
 };
