@@ -286,6 +286,14 @@ __global__ void k_assign_seeds(const BuildParams B, int pass, uint32_t *set, uin
 // ---- kernel 3: finalise -----------------------------------------------------
 // NS samples (3: a trio; 2 + n_children in a family).
 // counts: [NS][n]; hits/distinct: [n_variants][2][NS]; n_kmers: [n_variants][2]
+// A (variant, allele, sample) hit total saturates at UINT32_MAX instead of wrapping: the sum of
+// up to 32 u32 counters is formed from their 16-bit halves in 64 bits, and a leader whose
+// atomicAdd wrapped the cell sets it to UINT32_MAX.  Until the first wrap the cell holds the exact
+// partial sum; after it, every add wraps again (the cell is UINT32_MAX or wrapped), so the last
+// operation on the cell is an exchange: the cell ends at UINT32_MAX exactly when the total passes
+// it.  The NS adds are issued back to back and checked after (one round trip per leader).  The
+// calls of k_calls then equal the rule on the exact sums for every max_parent_alt_hits below
+// UINT32_MAX.
 template <int NS>
 __global__ void k_variant_reduce(const uint32_t *counts, const uint32_t *variant,
                                  const uint8_t *allele, const uint8_t *dead, uint32_t n,
@@ -307,7 +315,9 @@ __global__ void k_variant_reduce(const uint32_t *counts, const uint32_t *variant
   uint32_t h[NS], d[NS];
 #pragma unroll
   for (int smp = 0; smp < NS; smp++) {
-    h[smp] = __reduce_add_sync(peers, c[smp]);
+    const uint64_t sum = ((uint64_t)__reduce_add_sync(peers, c[smp] >> 16) << 16) +
+                         __reduce_add_sync(peers, c[smp] & 0xFFFFu);
+    h[smp] = sum > 0xFFFFFFFFull ? 0xFFFFFFFFu : (uint32_t)sum;
     d[smp] = __reduce_add_sync(peers, c[smp] ? 1u : 0u);
   }
   if (!leader) return;
@@ -315,10 +325,13 @@ __global__ void k_variant_reduce(const uint32_t *counts, const uint32_t *variant
 #pragma unroll
   for (int smp = 0; smp < NS; smp++) {
     if (h[smp]) {
-      atomicAdd(hits + (size_t)va * NS + smp, h[smp]);
+      c[smp] = atomicAdd(hits + (size_t)va * NS + smp, h[smp]);  // c: the cell before the add
       atomicAdd(distinct + (size_t)va * NS + smp, d[smp]);
     }
   }
+#pragma unroll
+  for (int smp = 0; smp < NS; smp++)
+    if (h[smp] && c[smp] + h[smp] < c[smp]) atomicExch(hits + (size_t)va * NS + smp, 0xFFFFFFFFu);
 }
 
 struct Thresholds {

@@ -249,6 +249,10 @@ int dkb_entry_counts_fetch(dkb_ctx *ctx, uint32_t *out);
 int dkb_entry_counts_device(dkb_ctx *ctx, void **d_ptr, size_t *n_u32);
 
 /* ---- kernel 3: finalise ---------------------------------------------------- */
+/* Per (variant, allele, sample) hits saturate at UINT32_MAX: a sum past 2^32 - 1 reads as
+ * UINT32_MAX, never as its wrapped remainder.  The calls therefore equal the de novo rule on the
+ * exact sums for every max_parent_alt_hits below UINT32_MAX and every min_child_alt_hits and
+ * min_parent_ref_hits. */
 int dkb_finalise(dkb_ctx *ctx, const dkb_thresholds *thr);
 /* Same, from a caller-owned DEVICE copy of the counters ([DKB_N_SAMPLES][n_entries], or
    [NS][n_entries] in a family: the layout of dkb_entry_counts_device) - e.g. a copy that is being summed over ranks while
