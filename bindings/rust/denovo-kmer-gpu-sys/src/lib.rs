@@ -87,6 +87,10 @@ extern "C" {
     pub fn dkb_table_set_regions(ctx: *mut DkbCtx, lo: *const u64, hi: *const u64, n_variants: u32) -> c_int;
     pub fn dkb_batch_set_loci(ctx: *mut DkbCtx, offsets: *const u64, lo: *const u64, hi: *const u64,
                               n_reads: usize) -> c_int;
+    pub fn dkb_batch_submit_multi(ctx: *mut DkbCtx, n_batches: c_int, bases2: *const *const u32,
+                                  mask1: *const *const u32, n_positions: *const u64, samples: *const c_int) -> c_int;
+    pub fn dkb_batch_set_loci_multi(ctx: *mut DkbCtx, n_batches: c_int, offsets: *const *const u64,
+                                    lo: *const *const u64, hi: *const *const u64, n_reads: *const usize) -> c_int;
     pub fn dkb_sync(ctx: *mut DkbCtx) -> c_int;
     pub fn dkb_counts_reset(ctx: *mut DkbCtx) -> c_int;
     pub fn dkb_entry_counts_fetch(ctx: *mut DkbCtx, out: *mut u32) -> c_int;

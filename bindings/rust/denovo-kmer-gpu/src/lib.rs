@@ -182,6 +182,19 @@ impl Counter {
         self.ck(unsafe { sys::dkb_batch_submit(self.ctx, b.bases2, b.mask1, b.n_positions, sample) })
     }
 
+    /// Kernel 2 on up to [`sys::DKB_MAX_MULTI`] packed batches, `(batch, sample)`, in ONE scan
+    /// launch: a trio step is one call.  Each batch must not be repacked before
+    /// [`Counter::sync`], as for [`Counter::submit`] (one [`BatchPacker`] per sample keeps that
+    /// rule when `sync` is called every second step).  Region mode: [`Counter::set_loci_multi`] first.
+    pub fn submit_multi(&mut self, batches: &[(&PinnedBatch, i32)]) -> Result<()> {
+        let b: Vec<*const u32> = batches.iter().map(|(x, _)| x.bases2 as *const u32).collect();
+        let m: Vec<*const u32> = batches.iter().map(|(x, _)| x.mask1 as *const u32).collect();
+        let n: Vec<u64> = batches.iter().map(|(x, _)| x.n_positions).collect();
+        let s: Vec<c_int> = batches.iter().map(|(_, smp)| *smp).collect();
+        let nb = c_int::try_from(batches.len()).unwrap_or(c_int::MAX);
+        self.ck(unsafe { sys::dkb_batch_submit_multi(self.ctx, nb, b.as_ptr(), m.as_ptr(), n.as_ptr(), s.as_ptr()) })
+    }
+
     /// Kernel 0 + 2: decoded reads as the BAM layer holds them (ASCII or 4-bit), packed on the GPU.
     pub fn submit_reads(&mut self, seq: &[u8], four_bit: bool, qual: Option<&[u8]>, offsets: &[u64],
                         min_baseq: i32, sample: i32) -> Result<()> {
@@ -219,6 +232,27 @@ impl Counter {
             sys::dkb_batch_set_loci(self.ctx, keep[0].as_ptr(), keep[1].as_ptr(), keep[2].as_ptr(), n_reads)
         })?;
         self.loci_keep.push(keep);  // (moving the Vecs does not move their heap buffers)
+        Ok(())
+    }
+
+    /// Region mode: the loci of the NEXT multi-batch submit ([`Counter::submit_multi`]), one
+    /// `(offsets, lo, hi)` per batch with the meaning of [`Counter::set_loci`].  Copied here and
+    /// kept until [`Counter::sync`].
+    pub fn set_loci_multi(&mut self, loci: &[(&[u64], &[u64], &[u64])]) -> Result<()> {
+        let mut keep = Vec::with_capacity(loci.len());
+        for (offsets, lo, hi) in loci {
+            let n_reads = offsets.len().saturating_sub(1);
+            if lo.len() != n_reads || hi.len() != n_reads || offsets.is_empty() {
+                return Err(DkbError { code: sys::DKB_EINVAL, detail: "lo and hi need one entry per read".into() });
+            }
+            keep.push([offsets.to_vec(), lo.to_vec(), hi.to_vec()]);
+        }
+        let ptrs = |i: usize| keep.iter().map(|k| k[i].as_ptr()).collect::<Vec<*const u64>>();
+        let (o, l, h) = (ptrs(0), ptrs(1), ptrs(2));
+        let n: Vec<usize> = keep.iter().map(|k| k[1].len()).collect();
+        let nb = c_int::try_from(loci.len()).unwrap_or(c_int::MAX);
+        self.ck(unsafe { sys::dkb_batch_set_loci_multi(self.ctx, nb, o.as_ptr(), l.as_ptr(), h.as_ptr(), n.as_ptr()) })?;
+        self.loci_keep.extend(keep);  // (moving the Vecs does not move their heap buffers)
         Ok(())
     }
 

@@ -73,6 +73,10 @@ SYMBOLS = {
                                                 C.POINTER(C.c_void_p), u64p, C.POINTER(C.c_int)]),
     "dkb_table_set_regions": (C.c_int, [C.c_void_p, u64p, u64p, C.c_uint32]),
     "dkb_batch_set_loci": (C.c_int, [C.c_void_p, u64p, u64p, u64p, C.c_size_t]),
+    "dkb_batch_submit_multi": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), u64p,
+                                         C.POINTER(C.c_int)]),
+    "dkb_batch_set_loci_multi": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(u64p), C.POINTER(u64p), C.POINTER(u64p),
+                                           C.POINTER(C.c_size_t)]),
     "dkb_sync": (C.c_int, [C.c_void_p]),
     "dkb_counts_reset": (C.c_int, [C.c_void_p]),
     "dkb_entry_counts_fetch": (C.c_int, [C.c_void_p, u32p]),

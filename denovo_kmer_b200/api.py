@@ -295,12 +295,37 @@ class KmerCounter:
         self._set_loci(loci)
         self._ck(self._L.dkb_batch_submit_device(self._h, d_bases2, d_mask1, n_positions, sample))
 
-    def submit_device_multi(self, batches):
+    def _set_loci_multi(self, loci, n):
+        if loci is None:
+            return
+        if len(loci) != n:
+            raise ValueError("loci: one ReadLoci per batch")
+        self._keep.append(loci)
+        arr = lambda f: (u64p * n)(*[_p(getattr(x, f), u64p) for x in loci])  # noqa: E731
+        nr = (C.c_size_t * n)(*[len(x.offsets) - 1 for x in loci])
+        self._ck(self._L.dkb_batch_set_loci_multi(self._h, n, arr("offsets"), arr("lo"), arr("hi"), nr))
+
+    def submit_multi(self, streams, samples, loci=None):
+        """Up to 4 host streams (ReadStream) scanned in ONE kernel launch, streams[i] into the
+        counters of samples[i] (e.g. the three samples of a trio step).  loci: region mode, one
+        ReadLoci per stream.  Buffers are kept alive until sync()."""
+        n = len(streams)
+        if len(samples) != n:
+            raise ValueError("submit_multi: one sample per stream")
+        self._set_loci_multi(loci, n)
+        self._keep.append(streams)
+        b = (C.c_void_p * n)(*[s.bases2.ctypes.data for s in streams])
+        m = (C.c_void_p * n)(*[s.mask1.ctypes.data for s in streams])
+        npos = (C.c_uint64 * n)(*[int(s.n_positions) for s in streams])
+        smp = (C.c_int * n)(*[int(x) for x in samples])
+        self._ck(self._L.dkb_batch_submit_multi(self._h, n, b, m, npos, smp))
+
+    def submit_device_multi(self, batches, loci=None):
         """batches: up to 4 tuples (d_bases2, d_mask1, n_positions, sample) of resident
         streams, scanned in ONE kernel launch (e.g. the three samples of a trio, or the four of
-        a quad).  Not in
-        region mode."""
+        a quad).  loci: region mode, one ReadLoci per batch, referenced until sync()."""
         n = len(batches)
+        self._set_loci_multi(loci, n)
         b = (C.c_void_p * n)(*[int(x[0]) for x in batches])
         m = (C.c_void_p * n)(*[int(x[1]) for x in batches])
         npos = (C.c_uint64 * n)(*[int(x[2]) for x in batches])

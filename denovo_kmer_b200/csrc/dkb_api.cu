@@ -100,7 +100,8 @@ struct dkb_ctx {
   cudaEvent_t ev_snap[2] = {nullptr, nullptr}, ev_red[2] = {nullptr, nullptr};
   int red_next = 0, red_pending = -1, red_last = -1;
   // region mode (dkb_table_set_regions): each entry's variant window, and the loci the next
-  // single-batch submit takes (dkb_batch_set_loci; host buffers, copied by that submit)
+  // submit takes (host buffers, copied by that submit): one batch's (dkb_batch_set_loci) or
+  // one set per batch of a multi-batch submit (dkb_batch_set_loci_multi)
   bool regions = false;
   ulonglong2 *d_entry_win = nullptr;
   struct Loci {
@@ -108,14 +109,17 @@ struct dkb_ctx {
     size_t n_reads = 0;
     uint64_t n_pos = 0;
     bool set = false;
-  } loci;
-  // the read-locus index of a batch on the device, double-buffered like `stage`
+  } loci, mloci[DKB_MAX_MULTI];
+  int mloci_n = 0;
+  bool mloci_set = false;
+  // the read-locus index of one launch's batches on the device (concatenated, one segment per
+  // batch with reads), double-buffered like `stage`
   struct LociStage {
     uint64_t *offsets = nullptr, *lo = nullptr, *hi = nullptr;
     uint32_t *start = nullptr, *tile = nullptr;
     ulonglong2 *span = nullptr;
     size_t off_cap = 0, lo_cap = 0, hi_cap = 0, start_cap = 0, tile_cap = 0, span_cap = 0;
-    uint32_t n_tiles = 0;
+    uint32_t tile_base[DKB_MAX_MULTI] = {}, n_tiles[DKB_MAX_MULTI] = {};  // per batch of the submit
     cudaEvent_t copied = nullptr, freed = nullptr;
     bool in_use = false;
   } lstage[2];
@@ -159,6 +163,12 @@ void dfree(T *&p) {
   p = nullptr;
 }
 
+// Forget whatever loci are pending, single-batch or multi-batch.
+void drop_loci(dkb_ctx *c) {
+  c->loci.set = false;
+  c->mloci_set = false;
+}
+
 void free_table(dkb_ctx *c) {
   dfree(c->d_keys); dfree(c->d_variant); dfree(c->d_allele); dfree(c->d_dead);
   dfree(c->d_tslots);
@@ -169,7 +179,7 @@ void free_table(dkb_ctx *c) {
   dfree(c->d_calls);
   dfree(c->d_entry_win);
   c->regions = false;  // a new table counts the whole stream until dkb_table_set_regions
-  c->loci.set = false;
+  drop_loci(c);
   c->n_entries = c->n_live = 0;
   c->n_variants = 0;
   c->finalised = false;
@@ -378,9 +388,9 @@ scan_fn pick_scan(int D, int NH, int fm, bool prof, bool rg) {
 }
 
 // One scan launch over n_seg device-resident packed streams (each into its sample's counters).
-// Region mode: exactly one stream, whose read-locus index is ls.
+// Region mode: ls is the read-locus index of all of them (stage_loci).
 int launch_scan(dkb_ctx *ctx, int n_seg, const uint32_t *const *d_bases, const uint32_t *const *d_mask,
-                const uint64_t *n_positions, const int *samples, dkb_ctx::LociStage *ls = nullptr) {
+                const uint64_t *n_positions, const int *samples, dkb_ctx::LociStage *ls) {
   ScanParams P;
   memset(&P, 0, sizeof(P));
   // work units: tiles, or macro tiles of 4-8 tiles at strides 8/16
@@ -400,6 +410,10 @@ int launch_scan(dkb_ctx *ctx, int n_seg, const uint32_t *const *d_bases, const u
     S.unit_begin = (uint32_t)units;
     units += (S.n_tiles + per_unit - 1) / per_unit;
     S.unit_end = (uint32_t)units;
+    if (ls) {
+      P.rseg[P.n_seg - 1].tile_base = ls->tile_base[i];
+      P.rseg[P.n_seg - 1].n_tiles = ls->n_tiles[i];
+    }
     total_pos += n_positions[i];
   }
   if (P.n_seg == 0) return DKB_OK;
@@ -422,12 +436,11 @@ int launch_scan(dkb_ctx *ctx, int n_seg, const uint32_t *const *d_bases, const u
   P.prof = ctx->d_prof;
   const bool rg = ctx->regions;
   if (rg) {
-    if (!ls || P.n_seg != 1) return fail(ctx, DKB_ESTATE, "region mode scans one batch with its loci per launch");
+    if (!ls) return fail(ctx, DKB_ESTATE, "region mode scans batches with their loci");
     P.read_start = ls->start;
     P.tile_read = ls->tile;
     P.read_span = ls->span;
     P.entry_win = ctx->d_entry_win;
-    P.n_loci_tiles = ls->n_tiles;
   }
   scan_fn fn = pick_scan(ctx->D, ctx->NH, ctx->gf ? (ctx->pre_words ? 2 : 1) + (ctx->gate ? 2 : 0) : 0, ctx->prof, rg);
   if (!fn && rg && ctx->prof)
@@ -497,16 +510,57 @@ int grow(dkb_ctx *ctx, T *&p, size_t &cap, size_t need) {
   return DKB_OK;
 }
 
+// Copy n host-resident batches into one staging buffer, each at a 16-byte-aligned offset, on
+// the copy stream; the scan stream waits for the copies.  d_bases / d_mask get the batches'
+// device addresses.  After launching the scan the caller records st->freed and sets in_use.
+int stage_batches(dkb_ctx *ctx, int n, const uint32_t *const *bases2, const uint32_t *const *mask1,
+                  const uint64_t *n_positions, const uint32_t **d_bases, const uint32_t **d_mask,
+                  dkb_ctx::Stage *&out) {
+  size_t bo[DKB_MAX_MULTI], mo[DKB_MAX_MULTI], bw = 0, mw = 0;
+  for (int i = 0; i < n; i++) {
+    bo[i] = bw;
+    mo[i] = mw;
+    bw += (dkb_stream_bases_words(n_positions[i]) + 3) / 4 * 4;
+    mw += (dkb_stream_mask_words(n_positions[i]) + 3) / 4 * 4;
+  }
+  dkb_ctx::Stage &st = ctx->stage[ctx->next_stage];
+  ctx->next_stage ^= 1;
+  if (st.in_use) CU(cudaStreamWaitEvent(ctx->s_copy, st.freed, 0));
+  if (st.bases_cap < bw || st.mask_cap < mw) {
+    // the previous scan may still read the old buffers
+    if (st.in_use) CU(cudaEventSynchronize(st.freed));
+    int rc;
+    if ((rc = grow(ctx, st.bases, st.bases_cap, bw)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st.mask, st.mask_cap, mw)) != DKB_OK) return rc;
+  }
+  for (int i = 0; i < n; i++) {
+    d_bases[i] = st.bases + bo[i];
+    d_mask[i] = st.mask + mo[i];
+    if (n_positions[i] == 0) continue;
+    CU(cudaMemcpyAsync(st.bases + bo[i], bases2[i], dkb_stream_bases_words(n_positions[i]) * 4,
+                       cudaMemcpyHostToDevice, ctx->s_copy));
+    CU(cudaMemcpyAsync(st.mask + mo[i], mask1[i], dkb_stream_mask_words(n_positions[i]) * 4, cudaMemcpyHostToDevice,
+                       ctx->s_copy));
+  }
+  CU(cudaEventRecord(st.copied, ctx->s_copy));
+  CU(cudaStreamWaitEvent(ctx->s_scan, st.copied, 0));
+  out = &st;
+  return DKB_OK;
+}
+
+const char *const NO_PROF_REGIONS = "region mode has no scan kernel with profiling counters (dkb_profile_counters 0)";
+
 // Region mode: the loci dkb_batch_set_loci left for this submit (consumed whatever the outcome;
 // out->set stays false in whole-stream mode).
 int take_loci(dkb_ctx *ctx, uint64_t n_positions, dkb_ctx::Loci *out) {
   *out = dkb_ctx::Loci{};
   if (!ctx->regions) return DKB_OK;
   const dkb_ctx::Loci l = ctx->loci;
-  ctx->loci.set = false;
+  const bool multi = ctx->mloci_set;
+  drop_loci(ctx);
+  if (multi) return fail(ctx, DKB_ESTATE, "region mode: multi-batch loci are pending, but this is a single-batch submit");
   if (!l.set) return fail(ctx, DKB_ESTATE, "region mode: dkb_batch_set_loci must come before every single-batch submit");
-  if (ctx->prof)
-    return fail(ctx, DKB_ESTATE, "region mode has no scan kernel with profiling counters (dkb_profile_counters 0)");
+  if (ctx->prof) return fail(ctx, DKB_ESTATE, NO_PROF_REGIONS);
   if (l.n_pos != n_positions)
     return fail(ctx, DKB_EINVAL, "the loci's reads cover " + std::to_string(l.n_pos) + " stream positions, the batch " +
                                      std::to_string(n_positions));
@@ -514,38 +568,87 @@ int take_loci(dkb_ctx *ctx, uint64_t n_positions, dkb_ctx::Loci *out) {
   return DKB_OK;
 }
 
-// Copy a batch's loci (copy stream) and build its read-locus index (scan stream, ahead of the
-// scan).  ls = nullptr in whole-stream mode.
-int stage_loci(dkb_ctx *ctx, const dkb_ctx::Loci &l, dkb_ctx::LociStage *&ls) {
+// The same for a multi-batch submit: the loci dkb_batch_set_loci_multi left, one set per batch.
+int take_loci_multi(dkb_ctx *ctx, int n_batches, const uint64_t *n_positions, dkb_ctx::Loci *out) {
+  for (int i = 0; i < DKB_MAX_MULTI; i++) out[i] = dkb_ctx::Loci{};
+  if (!ctx->regions) return DKB_OK;
+  const bool single = ctx->loci.set, multi = ctx->mloci_set;
+  const int n = ctx->mloci_n;
+  drop_loci(ctx);
+  if (single) return fail(ctx, DKB_ESTATE, "region mode: single-batch loci are pending, but this is a multi-batch submit");
+  if (!multi)
+    return fail(ctx, DKB_ESTATE, "region mode: dkb_batch_set_loci_multi must come before every multi-batch submit");
+  if (ctx->prof) return fail(ctx, DKB_ESTATE, NO_PROF_REGIONS);
+  if (n != n_batches)
+    return fail(ctx, DKB_EINVAL, "the loci are for " + std::to_string(n) + " batches, the submit has " +
+                                     std::to_string(n_batches));
+  if (n && !n_positions) return fail(ctx, DKB_EINVAL, "null argument");
+  for (int i = 0; i < n; i++)
+    if (ctx->mloci[i].n_pos != n_positions[i])
+      return fail(ctx, DKB_EINVAL, "batch " + std::to_string(i) + ": the loci's reads cover " +
+                                       std::to_string(ctx->mloci[i].n_pos) + " stream positions, the batch " +
+                                       std::to_string(n_positions[i]));
+  for (int i = 0; i < n; i++) out[i] = ctx->mloci[i];
+  return DKB_OK;
+}
+
+// Copy the loci of a launch's n batches (copy stream) into one LociStage, concatenated, and
+// build their read-locus index with one launch of each index kernel (scan stream, ahead of the
+// scan).  ls = nullptr in whole-stream mode, and when no batch has reads (nothing to scan).
+int stage_loci(dkb_ctx *ctx, int n, const dkb_ctx::Loci *l, dkb_ctx::LociStage *&ls) {
   ls = nullptr;
-  if (!l.set) return DKB_OK;
+  if (n == 0 || !l[0].set) return DKB_OK;
+  LociSegments S;
+  memset(&S, 0, sizeof(S));
+  uint32_t tile_base[DKB_MAX_MULTI], n_tiles[DKB_MAX_MULTI];
+  int batch_of[DKB_MAX_MULTI];
+  size_t nr = 0, nt = 0;
+  for (int i = 0; i < n; i++) {
+    tile_base[i] = (uint32_t)nt;
+    n_tiles[i] = 0;
+    if (l[i].n_reads == 0) continue;  // (no positions: launch_scan skips the batch too)
+    n_tiles[i] = (uint32_t)((l[i].n_pos + (1u << LOCI_TILE_SHIFT) - 1) >> LOCI_TILE_SHIFT);
+    S.read_base[S.n_seg] = (uint32_t)nr;
+    S.tile_base[S.n_seg] = (uint32_t)nt;
+    batch_of[S.n_seg++] = i;
+    nr += l[i].n_reads;
+    nt += n_tiles[i] + 1;
+  }
+  if (S.n_seg == 0) return DKB_OK;
+  S.read_base[S.n_seg] = (uint32_t)nr;
+  S.tile_base[S.n_seg] = (uint32_t)nt;
+  const size_t no = nr + S.n_seg;  // offsets: n_reads + 1 per segment
   dkb_ctx::LociStage &st = ctx->lstage[ctx->next_lstage];
   ctx->next_lstage ^= 1;
-  const size_t nr = l.n_reads;
-  const uint32_t n_tiles = (uint32_t)((l.n_pos + (1u << LOCI_TILE_SHIFT) - 1) >> LOCI_TILE_SHIFT);
   if (st.in_use) CU(cudaStreamWaitEvent(ctx->s_copy, st.freed, 0));
-  if (st.off_cap < nr + 1 || st.lo_cap < nr || st.hi_cap < nr || st.start_cap < nr || st.span_cap < nr ||
-      st.tile_cap < (size_t)n_tiles + 1) {
+  if (st.off_cap < no || st.lo_cap < nr || st.hi_cap < nr || st.start_cap < nr || st.span_cap < nr ||
+      st.tile_cap < nt) {
     if (st.in_use) CU(cudaEventSynchronize(st.freed));  // the previous scan may still read the old index
     int rc;
-    if ((rc = grow(ctx, st.offsets, st.off_cap, nr + 1)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st.offsets, st.off_cap, no)) != DKB_OK) return rc;
     if ((rc = grow(ctx, st.lo, st.lo_cap, nr)) != DKB_OK) return rc;
     if ((rc = grow(ctx, st.hi, st.hi_cap, nr)) != DKB_OK) return rc;
     if ((rc = grow(ctx, st.start, st.start_cap, nr)) != DKB_OK) return rc;
     if ((rc = grow(ctx, st.span, st.span_cap, nr)) != DKB_OK) return rc;
-    if ((rc = grow(ctx, st.tile, st.tile_cap, (size_t)n_tiles + 1)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st.tile, st.tile_cap, nt)) != DKB_OK) return rc;
   }
-  CU(cudaMemcpyAsync(st.offsets, l.offsets, (nr + 1) * 8, cudaMemcpyHostToDevice, ctx->s_copy));
-  CU(cudaMemcpyAsync(st.lo, l.lo, nr * 8, cudaMemcpyHostToDevice, ctx->s_copy));
-  CU(cudaMemcpyAsync(st.hi, l.hi, nr * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+  for (uint32_t j = 0; j < S.n_seg; j++) {
+    const dkb_ctx::Loci &b = l[batch_of[j]];
+    const size_t r0 = S.read_base[j];
+    CU(cudaMemcpyAsync(st.offsets + r0 + j, b.offsets, (b.n_reads + 1) * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+    CU(cudaMemcpyAsync(st.lo + r0, b.lo, b.n_reads * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+    CU(cudaMemcpyAsync(st.hi + r0, b.hi, b.n_reads * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+  }
   CU(cudaEventRecord(st.copied, ctx->s_copy));
   CU(cudaStreamWaitEvent(ctx->s_scan, st.copied, 0));
   const int TB = 256;
-  k_read_loci<<<(uint32_t)((nr + TB - 1) / TB), TB, 0, ctx->s_scan>>>(st.offsets, st.lo, st.hi, (uint32_t)nr,
-                                                                       st.start, st.span);
-  k_tile_reads<<<(n_tiles + TB) / TB, TB, 0, ctx->s_scan>>>(st.start, (uint32_t)nr, n_tiles, st.tile);
+  k_read_loci<<<(uint32_t)((nr + TB - 1) / TB), TB, 0, ctx->s_scan>>>(S, st.offsets, st.lo, st.hi, st.start, st.span);
+  k_tile_reads<<<(uint32_t)((nt + TB - 1) / TB), TB, 0, ctx->s_scan>>>(S, st.start, st.tile);
   CU(cudaGetLastError());
-  st.n_tiles = n_tiles;
+  for (int i = 0; i < n; i++) {
+    st.tile_base[i] = tile_base[i];
+    st.n_tiles[i] = n_tiles[i];
+  }
   ls = &st;
   return DKB_OK;
 }
@@ -691,6 +794,33 @@ int check_sample(dkb_ctx *ctx, int sample) {
   return fail(ctx, DKB_EINVAL, ctx->n_samples == DKB_N_SAMPLES
                                    ? std::string("sample must be 0, 1 or 2")
                                    : "sample must be in [0, " + std::to_string(ctx->n_samples) + ")");
+}
+
+// Checks shared by the multi-batch submits, after their loci have been taken.
+int check_multi(dkb_ctx *ctx, int n_batches, const void *bases2, const void *mask1, const uint64_t *n_positions,
+                const int *samples) {
+  if (n_batches < 0 || n_batches > DKB_MAX_MULTI) return fail(ctx, DKB_EINVAL, "n_batches out of range");
+  if (n_batches && (!bases2 || !mask1 || !n_positions || !samples)) return fail(ctx, DKB_EINVAL, "null argument");
+  for (int i = 0; i < n_batches; i++) {
+    if (check_sample(ctx, samples[i]) != DKB_OK) return DKB_EINVAL;
+    if (n_positions[i] > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
+  }
+  return DKB_OK;
+}
+
+// One batch's loci, as dkb_batch_set_loci takes them, checked and kept in *out (out->set untouched).
+int check_loci(dkb_ctx *ctx, const uint64_t *offsets, const uint64_t *lo, const uint64_t *hi, size_t n_reads,
+               dkb_ctx::Loci *out) {
+  if ((uint64_t)n_reads >= 0x100000000ull) return fail(ctx, DKB_EINVAL, "too many reads in one batch (max 2^32 - 1)");
+  if (!offsets || (n_reads && (!lo || !hi))) return fail(ctx, DKB_EINVAL, "null loci array");
+  for (size_t r = 0; r < n_reads; r++)
+    if (offsets[r + 1] < offsets[r]) return fail(ctx, DKB_EINVAL, "offsets must not decrease");
+  out->offsets = offsets;
+  out->lo = lo;
+  out->hi = hi;
+  out->n_reads = n_reads;
+  out->n_pos = dkb_stream_positions(offsets, n_reads);
+  return DKB_OK;
 }
 
 // Kernel 3 on snapshot b, on the scan stream, once its sum over ranks is complete.
@@ -1037,7 +1167,7 @@ int dkb_batch_submit_device(dkb_ctx *ctx, const uint32_t *d_bases2, const uint32
   if ((uintptr_t)d_mask1 & 3) return fail(ctx, DKB_EINVAL, "d_mask1 must be 4-byte aligned");
   CU(cudaSetDevice(ctx->device));
   dkb_ctx::LociStage *ls;
-  if ((rc = stage_loci(ctx, loci, ls)) != DKB_OK) return rc;
+  if ((rc = stage_loci(ctx, 1, &loci, ls)) != DKB_OK) return rc;
   return launch_scan(ctx, d_bases2, d_mask1, n_positions, sample, ls);
 }
 
@@ -1046,19 +1176,48 @@ int dkb_batch_submit_device_multi(dkb_ctx *ctx, int n_batches, const uint32_t *c
                                   const int *samples) {
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
   if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
-  if (ctx->regions) return fail(ctx, DKB_ESTATE, "dkb_batch_submit_device_multi does not support region mode");
-  if (n_batches < 0 || n_batches > DKB_MAX_MULTI) return fail(ctx, DKB_EINVAL, "n_batches out of range");
-  if (n_batches && (!d_bases2 || !d_mask1 || !n_positions || !samples)) return fail(ctx, DKB_EINVAL, "null argument");
+  dkb_ctx::Loci loci[DKB_MAX_MULTI];
+  int rc = take_loci_multi(ctx, n_batches, n_positions, loci);
+  if (rc != DKB_OK) return rc;
+  if ((rc = check_multi(ctx, n_batches, d_bases2, d_mask1, n_positions, samples)) != DKB_OK) return rc;
   for (int i = 0; i < n_batches; i++) {
-    if (check_sample(ctx, samples[i]) != DKB_OK) return DKB_EINVAL;
     if (n_positions[i] == 0) continue;
-    if (n_positions[i] > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
     if (!d_bases2[i] || !d_mask1[i]) return fail(ctx, DKB_EINVAL, "null stream pointer");
     if ((uintptr_t)d_bases2[i] & 15) return fail(ctx, DKB_EINVAL, "d_bases2 must be 16-byte aligned");
     if ((uintptr_t)d_mask1[i] & 3) return fail(ctx, DKB_EINVAL, "d_mask1 must be 4-byte aligned");
   }
   CU(cudaSetDevice(ctx->device));
-  return launch_scan(ctx, n_batches, d_bases2, d_mask1, n_positions, samples);
+  dkb_ctx::LociStage *ls;
+  if ((rc = stage_loci(ctx, n_batches, loci, ls)) != DKB_OK) return rc;
+  return launch_scan(ctx, n_batches, d_bases2, d_mask1, n_positions, samples, ls);
+}
+
+int dkb_batch_submit_multi(dkb_ctx *ctx, int n_batches, const uint32_t *const *bases2,
+                           const uint32_t *const *mask1, const uint64_t *n_positions, const int *samples) {
+  if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
+  if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
+  dkb_ctx::Loci loci[DKB_MAX_MULTI];
+  int rc = take_loci_multi(ctx, n_batches, n_positions, loci);
+  if (rc != DKB_OK) return rc;
+  if ((rc = check_multi(ctx, n_batches, bases2, mask1, n_positions, samples)) != DKB_OK) return rc;
+  bool any = false;
+  for (int i = 0; i < n_batches; i++) {
+    if (n_positions[i] == 0) continue;
+    if (!bases2[i] || !mask1[i]) return fail(ctx, DKB_EINVAL, "null stream pointer");
+    any = true;
+  }
+  if (!any) return DKB_OK;
+  CU(cudaSetDevice(ctx->device));
+  const uint32_t *d_bases[DKB_MAX_MULTI], *d_mask[DKB_MAX_MULTI];
+  dkb_ctx::Stage *st;
+  if ((rc = stage_batches(ctx, n_batches, bases2, mask1, n_positions, d_bases, d_mask, st)) != DKB_OK) return rc;
+  dkb_ctx::LociStage *ls;
+  if ((rc = stage_loci(ctx, n_batches, loci, ls)) != DKB_OK) return rc;
+  rc = launch_scan(ctx, n_batches, d_bases, d_mask, n_positions, samples, ls);
+  if (rc != DKB_OK) return rc;
+  CU(cudaEventRecord(st->freed, ctx->s_scan));
+  st->in_use = true;
+  return DKB_OK;
 }
 
 int dkb_batch_submit(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t *mask1,
@@ -1073,26 +1232,15 @@ int dkb_batch_submit(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t *mask1
   if (n_positions > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
   if (!bases2 || !mask1) return fail(ctx, DKB_EINVAL, "null stream pointer");
   CU(cudaSetDevice(ctx->device));
-  const size_t bw = dkb_stream_bases_words(n_positions), mw = dkb_stream_mask_words(n_positions);
-  dkb_ctx::Stage &st = ctx->stage[ctx->next_stage];
-  ctx->next_stage ^= 1;
-  if (st.in_use) CU(cudaStreamWaitEvent(ctx->s_copy, st.freed, 0));
-  if (st.bases_cap < bw || st.mask_cap < mw) {
-    // the previous scan may still read the old buffers
-    if (st.in_use) CU(cudaEventSynchronize(st.freed));
-    if ((rc = grow(ctx, st.bases, st.bases_cap, bw)) != DKB_OK) return rc;
-    if ((rc = grow(ctx, st.mask, st.mask_cap, mw)) != DKB_OK) return rc;
-  }
-  CU(cudaMemcpyAsync(st.bases, bases2, bw * 4, cudaMemcpyHostToDevice, ctx->s_copy));
-  CU(cudaMemcpyAsync(st.mask, mask1, mw * 4, cudaMemcpyHostToDevice, ctx->s_copy));
-  CU(cudaEventRecord(st.copied, ctx->s_copy));
-  CU(cudaStreamWaitEvent(ctx->s_scan, st.copied, 0));
+  const uint32_t *d_bases, *d_mask;
+  dkb_ctx::Stage *st;
+  if ((rc = stage_batches(ctx, 1, &bases2, &mask1, &n_positions, &d_bases, &d_mask, st)) != DKB_OK) return rc;
   dkb_ctx::LociStage *ls;
-  if ((rc = stage_loci(ctx, loci, ls)) != DKB_OK) return rc;
-  rc = launch_scan(ctx, st.bases, st.mask, n_positions, sample, ls);
+  if ((rc = stage_loci(ctx, 1, &loci, ls)) != DKB_OK) return rc;
+  rc = launch_scan(ctx, d_bases, d_mask, n_positions, sample, ls);
   if (rc != DKB_OK) return rc;
-  CU(cudaEventRecord(st.freed, ctx->s_scan));
-  st.in_use = true;
+  CU(cudaEventRecord(st->freed, ctx->s_scan));
+  st->in_use = true;
   return DKB_OK;
 }
 
@@ -1137,7 +1285,7 @@ int dkb_batch_submit_sparse(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t
                                                                       (uint32_t)mw, st.mask);
   CU(cudaGetLastError());
   dkb_ctx::LociStage *ls;
-  if ((rc = stage_loci(ctx, loci, ls)) != DKB_OK) return rc;
+  if ((rc = stage_loci(ctx, 1, &loci, ls)) != DKB_OK) return rc;
   rc = launch_scan(ctx, st.bases, st.mask, n_positions, sample, ls);
   if (rc != DKB_OK) return rc;
   CU(cudaEventRecord(st.freed, ctx->s_scan));
@@ -1213,7 +1361,7 @@ int dkb_batch_submit_reads(dkb_ctx *ctx, const uint8_t *seq, int seq_format, con
   k_pack<<<(uint32_t)((mw + TB - 1) / TB), TB, 0, ctx->s_scan>>>(Q);
   CU(cudaGetLastError());
   dkb_ctx::LociStage *ls;
-  if ((rc = stage_loci(ctx, loci, ls)) != DKB_OK) return rc;
+  if ((rc = stage_loci(ctx, 1, &loci, ls)) != DKB_OK) return rc;
   rc = launch_scan(ctx, st.bases, st.mask, n_pos, sample, ls);
   if (rc != DKB_OK) return rc;
   CU(cudaEventRecord(st.freed, ctx->s_scan));
@@ -1224,7 +1372,7 @@ int dkb_batch_submit_reads(dkb_ctx *ctx, const uint8_t *seq, int seq_format, con
 int dkb_table_set_regions(dkb_ctx *ctx, const uint64_t *lo, const uint64_t *hi, uint32_t n_variants) {
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
   if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
-  ctx->loci.set = false;
+  drop_loci(ctx);
   if (!lo && !hi) {
     if (n_variants) return fail(ctx, DKB_EINVAL, "lo == hi == NULL (whole-stream counting) takes n_variants 0");
     ctx->regions = false;
@@ -1260,18 +1408,31 @@ int dkb_table_set_regions(dkb_ctx *ctx, const uint64_t *lo, const uint64_t *hi, 
 int dkb_batch_set_loci(dkb_ctx *ctx, const uint64_t *offsets, const uint64_t *lo, const uint64_t *hi,
                        size_t n_reads) {
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
-  ctx->loci.set = false;
+  drop_loci(ctx);
   if (!ctx->regions) return fail(ctx, DKB_ESTATE, "dkb_batch_set_loci needs region mode (dkb_table_set_regions)");
-  if ((uint64_t)n_reads >= 0x100000000ull) return fail(ctx, DKB_EINVAL, "too many reads in one batch (max 2^32 - 1)");
-  if (!offsets || (n_reads && (!lo || !hi))) return fail(ctx, DKB_EINVAL, "null loci array");
-  for (size_t r = 0; r < n_reads; r++)
-    if (offsets[r + 1] < offsets[r]) return fail(ctx, DKB_EINVAL, "offsets must not decrease");
-  ctx->loci.offsets = offsets;
-  ctx->loci.lo = lo;
-  ctx->loci.hi = hi;
-  ctx->loci.n_reads = n_reads;
-  ctx->loci.n_pos = dkb_stream_positions(offsets, n_reads);
+  int rc = check_loci(ctx, offsets, lo, hi, n_reads, &ctx->loci);
+  if (rc != DKB_OK) return rc;
   ctx->loci.set = true;
+  return DKB_OK;
+}
+
+int dkb_batch_set_loci_multi(dkb_ctx *ctx, int n_batches, const uint64_t *const *offsets,
+                             const uint64_t *const *lo, const uint64_t *const *hi, const size_t *n_reads) {
+  if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
+  drop_loci(ctx);
+  if (!ctx->regions) return fail(ctx, DKB_ESTATE, "dkb_batch_set_loci_multi needs region mode (dkb_table_set_regions)");
+  if (n_batches < 0 || n_batches > DKB_MAX_MULTI) return fail(ctx, DKB_EINVAL, "n_batches out of range");
+  if (n_batches && (!offsets || !lo || !hi || !n_reads)) return fail(ctx, DKB_EINVAL, "null argument");
+  uint64_t total = 0;  // reads are numbered across the launch's batches in 32 bits
+  for (int i = 0; i < n_batches; i++) {
+    int rc = check_loci(ctx, offsets[i], lo[i], hi[i], n_reads[i], &ctx->mloci[i]);
+    if (rc != DKB_OK) return rc;
+    total += n_reads[i];
+  }
+  if (total >= 0x100000000ull) return fail(ctx, DKB_EINVAL, "too many reads in one launch (max 2^32 - 1)");
+  for (int i = 0; i < n_batches; i++) ctx->mloci[i].set = true;
+  ctx->mloci_n = n_batches;
+  ctx->mloci_set = true;
   return DKB_OK;
 }
 

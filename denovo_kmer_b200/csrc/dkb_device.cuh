@@ -275,14 +275,19 @@ struct ScanParams {
   uint32_t filter_words;  // = BLOOM_WORDS (shared-memory mode), as a run-time operand of the wide multiply
   int k, s;
   unsigned long long *prof;  // 4 counters or nullptr
-  // ---- region mode only (k_scan<..., RG = true>; one segment).  Kept at the end so that the
-  // whole-stream kernels' parameter offsets stay where they were.
-  const uint32_t *read_start;   // [n_reads] first stream position of read r
-  const uint32_t *tile_read;    // [n_loci_tiles + 1] first read reaching into 2048-position tile t;
-                                // the last entry is n_reads - 1
+  // ---- region mode only (k_scan<..., RG = true>).  Kept at the end so that the whole-stream
+  // kernels' parameter offsets stay where they were.  The read-locus index of every segment of
+  // the launch is one set of concatenated arrays: reads are numbered across the segments.
+  const uint32_t *read_start;   // [n_reads] first stream position of read r, inside its segment
+  const uint32_t *tile_read;    // per segment, at rseg[i].tile_base: [n_tiles + 1] the first read
+                                // reaching into 2048-position tile t; the last entry is the
+                                // segment's last read
   const ulonglong2 *read_span;  // [n_reads] the read's alignment interval {lo, hi}; {*, 0} if empty
   const ulonglong2 *entry_win;  // [n_entries] the window of the entry's variant; {*, 0} if empty
-  uint32_t n_loci_tiles;
+  struct {
+    uint32_t tile_base;  // first entry of the segment's hints in tile_read
+    uint32_t n_tiles;    // its 2048-position tiles
+  } rseg[MAX_SEGMENTS];
 };
 
 // Region mode: positions per tile of the read-locus index (a position resolves to its read with

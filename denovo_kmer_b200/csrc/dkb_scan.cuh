@@ -28,7 +28,7 @@ namespace dkb {
 // FM = filter mode (dkb_device.cuh): 0 seed filter in shared memory, 1 in L2, 2 in L2 behind a
 // one-bit shared-memory pre-filter, 3 / 4 = 1 / 2 with gated lookups.
 // RG = region mode (DESIGN.md §2): a window counts toward an entry only when its read's
-// alignment interval overlaps the entry's variant window; one segment per launch.
+// alignment interval overlaps the entry's variant window.
 template <int D, int NH, int FM, bool PROF, bool RG>
 struct ScanWarp {
   static constexpr bool GF = FM > 0, PRE = fm_pre(FM), GATE = fm_gate(FM);
@@ -71,12 +71,16 @@ struct ScanWarp {
 
   // ---- region mode: the read that holds stream position p --------------------------
   // The last read starting at or before p, searched between the hints of p's tile and the
-  // next one (a tile holds about 14 reads of 150 bases: four steps).
+  // next one (a tile holds about 14 reads of 150 bases: four steps).  p is a position of
+  // segment `cur`, whose hints are read here: stage C only sees seeds of `cur`, because a warp
+  // drains every pending probe and verified seed (drain()) before it moves to another segment.
   __device__ __forceinline__ uint32_t find_read(uint32_t p) const {
     // (no min() here: naming it in this class changes how the whole-stream kernels compile)
+    const uint32_t nt = P.rseg[cur].n_tiles;
     uint32_t t = p >> LOCI_TILE_SHIFT;
-    if (t >= P.n_loci_tiles) t = P.n_loci_tiles - 1;
-    uint32_t a = __ldg(P.tile_read + t), b = __ldg(P.tile_read + t + 1);
+    if (t >= nt) t = nt - 1;
+    const uint32_t *const hint = P.tile_read + P.rseg[cur].tile_base + t;
+    uint32_t a = __ldg(hint), b = __ldg(hint + 1);
     while (a < b) {
       const uint32_t mid = b - (b - a) / 2;
       if (__ldg(P.read_start + mid) <= p) a = mid; else b = mid - 1;

@@ -210,10 +210,18 @@ int dkb_batch_submit_device(dkb_ctx *ctx, const uint32_t *d_bases2, const uint32
  * launch; batch i goes into the counters of samples[i].  Same alignment rules; a batch of 0
  * positions is skipped.  Worth it for short batches, where a launch costs as much as the scan. */
 #define DKB_MAX_MULTI 4
-/* Not supported in region mode (below): returns DKB_ESTATE there. */
+/* In region mode (below) it needs the loci of dkb_batch_set_loci_multi first. */
 int dkb_batch_submit_device_multi(dkb_ctx *ctx, int n_batches, const uint32_t *const *d_bases2,
                                   const uint32_t *const *d_mask1, const uint64_t *n_positions,
                                   const int *samples);
+/* Up to DKB_MAX_MULTI host-resident batches scanned in ONE kernel launch; batch i goes into the
+ * counters of samples[i].  Same buffer rules as dkb_batch_submit: valid until dkb_sync.  A batch
+ * of 0 positions is skipped; n_batches 0 is a no-op.  The batches are copied into one staging
+ * buffer, each with its own copy, and double-buffered like dkb_batch_submit: a trio step is one
+ * submit and one scan launch.  In region mode it needs the loci of dkb_batch_set_loci_multi
+ * first. */
+int dkb_batch_submit_multi(dkb_ctx *ctx, int n_batches, const uint32_t *const *bases2,
+                           const uint32_t *const *mask1, const uint64_t *n_positions, const int *samples);
 
 /* ---- region-scoped counting (opt-in; DESIGN.md §2) ---------------------------- */
 /* In region mode an occurrence of entry e's key in read r counts iff the read's alignment
@@ -239,6 +247,17 @@ int dkb_table_set_regions(dkb_ctx *ctx, const uint64_t *lo, const uint64_t *hi, 
  * submit returns DKB_ESTATE. */
 int dkb_batch_set_loci(dkb_ctx *ctx, const uint64_t *offsets, const uint64_t *lo,
                        const uint64_t *hi, size_t n_reads);
+/* Region mode: the read loci of the NEXT multi-batch submit (dkb_batch_submit_multi or
+ * dkb_batch_submit_device_multi), one set per batch, with the same meaning and validity rules
+ * as dkb_batch_set_loci.  DKB_ESTATE in whole-stream mode; DKB_EINVAL for n_batches outside
+ * [0, DKB_MAX_MULTI], descending offsets in any batch, n_reads[i] >= 2^32, or 2^32 or more
+ * reads in all.  The submit returns DKB_EINVAL unless its n_batches equals these loci's and
+ * dkb_stream_positions(offsets[i], n_reads[i]) == n_positions[i] for every batch.  Loci of the
+ * wrong kind are refused with DKB_ESTATE: a single-batch submit with multi-batch loci pending,
+ * a multi-batch submit with single-batch loci pending.  Setting either kind replaces whatever
+ * was pending, and every submit uses up the pending loci whatever its outcome. */
+int dkb_batch_set_loci_multi(dkb_ctx *ctx, int n_batches, const uint64_t *const *offsets,
+                             const uint64_t *const *lo, const uint64_t *const *hi, const size_t *n_reads);
 int dkb_sync(dkb_ctx *ctx);
 int dkb_counts_reset(dkb_ctx *ctx);
 

@@ -6,6 +6,7 @@
 #include <cstdint>
 #include <stdexcept>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "dkb.h"
@@ -162,6 +163,37 @@ class Counter {
     if (offsets.empty() || lo.size() + 1 != offsets.size() || hi.size() != lo.size())
       throw Error(DKB_EINVAL, "set_loci: lo and hi need one entry per read");
     check(dkb_batch_set_loci(ctx_, offsets.data(), lo.data(), hi.data(), lo.size()), ctx_);
+  }
+  // Loci of the next multi-batch submit, one set per batch (each as in set_loci); same lifetime rule.
+  struct LociRef {
+    const std::vector<uint64_t> *offsets, *lo, *hi;
+  };
+  void set_loci_multi(const std::vector<LociRef> &loci) {
+    std::vector<const uint64_t *> o, l, h;
+    std::vector<size_t> n;
+    for (const LociRef &x : loci) {
+      if (x.offsets->empty() || x.lo->size() + 1 != x.offsets->size() || x.hi->size() != x.lo->size())
+        throw Error(DKB_EINVAL, "set_loci_multi: lo and hi need one entry per read");
+      o.push_back(x.offsets->data());
+      l.push_back(x.lo->data());
+      h.push_back(x.hi->data());
+      n.push_back(x.lo->size());
+    }
+    check(dkb_batch_set_loci_multi(ctx_, (int)loci.size(), o.data(), l.data(), h.data(), n.data()), ctx_);
+  }
+  // Up to DKB_MAX_MULTI streams, (stream, sample), in ONE scan launch (a trio step); the streams
+  // must outlive the next sync()
+  void submit_multi(const std::vector<std::pair<const Stream *, int>> &batches) {
+    std::vector<const uint32_t *> b, m;
+    std::vector<uint64_t> n;
+    std::vector<int> smp;
+    for (const auto &x : batches) {
+      b.push_back(x.first->bases2.data());
+      m.push_back(x.first->mask1.data());
+      n.push_back(x.first->n_positions);
+      smp.push_back(x.second);
+    }
+    check(dkb_batch_submit_multi(ctx_, (int)batches.size(), b.data(), m.data(), n.data(), smp.data()), ctx_);
   }
   void sync() { check(dkb_sync(ctx_), ctx_); }
   void reset_counts() { check(dkb_counts_reset(ctx_), ctx_); }
