@@ -187,13 +187,12 @@ void free_table(dkb_ctx *c) {
 }
 
 // Words of the L2-resident seed filter: 64 bits per seed, between the shared-memory size
-// and 32 MB (it shares L2 with the tables and the stream; DKB_L2_FILTER_MAX_WORDS overrides).
+// and 32 MB (it shares L2 with the tables and the stream).
 // Measured on the 100 000-candidate WGS shard (6 M seeds): 4 / 8 / 16 / 32 / 48 MB -> 2.89 / 3.65 /
 // 3.86 / 3.92 / 3.91 Tbases/s: below 16 MB the filter's false positives (each a DRAM access
 // into the 1.5 GB slot table) cost more than the filter's own L2 misses.
 uint32_t l2_filter_words(double seeds) {
-  double cap = 8.0 * 1024 * 1024;  // 32 MB
-  if (const char *e = getenv("DKB_L2_FILTER_MAX_WORDS")) cap = atof(e);
+  const double cap = 8.0 * 1024 * 1024;  // 32 MB
   double w = seeds * 2.0;
   if (w > cap) w = cap;
   if (w < BLOOM_WORDS) w = BLOOM_WORDS;
@@ -448,7 +447,6 @@ int launch_scan(dkb_ctx *ctx, int n_seg, const uint32_t *const *d_bases, const u
   if (!fn) return fail(ctx, DKB_EINVAL, "no scan kernel for this tuning");
   size_t smem_bytes = !ctx->gf ? SCAN_SMEM_BYTES
                       : ctx->pre_words ? SCAN_SMEM_BYTES_PRE + (size_t)ctx->pre_words * 4 : SCAN_SMEM_BYTES_GF;
-  if (ctx->D >= 8) smem_bytes += SCAN_TMA_BYTES;  // TMA builds: the per-warp stream ring of the macro path
   {
     std::lock_guard<std::mutex> lk(g_smem_mu);
     auto it = g_smem_set.find({ctx->device, (const void *)fn});
@@ -999,9 +997,7 @@ int dkb_table_build(dkb_ctx *ctx, const uint64_t *keys, const uint32_t *variant_
   ctx->n_entries = n;
   ctx->n_variants = n_variants;
   const size_t n1 = n ? n : 1, nv1 = n_variants ? n_variants : 1, ns = ctx->n_samples;
-  int slots_per_entry = 8;
-  if (const char *e = getenv("DKB_KEY_SLOTS_PER_ENTRY")) slots_per_entry = atoi(e) > 0 ? atoi(e) : 8;
-  ctx->table_slots = pow2_at_least((uint64_t)slots_per_entry * n + 2);  // <= 0.25 entries per 2-slot bucket
+  ctx->table_slots = pow2_at_least(8 * (uint64_t)n + 2);  // <= 0.25 entries per 2-slot bucket
   uint16_t *d_wi = nullptr, *d_wc = nullptr;
   uint32_t *d_slot_of = nullptr;
   uint32_t *d_set = nullptr, *d_cov = nullptr;
@@ -1071,13 +1067,12 @@ int dkb_table_build(dkb_ctx *ctx, const uint64_t *keys, const uint32_t *variant_
     // size.  Only occupied slots are ever touched by true hits, so the hot set is 32 B per seed
     // and orientation; an absent seed (a filter false positive) lands on a slot marked
     // ST_MOVED_BIT - a second load - about one time in 8.
-    double per_seed = 4.0;  // (2.0: 3 % slower on configs[1] - displaced seeds cost a dependent load per step)
-    if (const char *e = getenv("DKB_SEED_SLOTS_PER_SEED")) per_seed = atof(e) >= 1.1 ? atof(e) : per_seed;
+    const double per_seed = 4.0;  // (2.0: 3 % slower on configs[1] - displaced seeds cost a dependent load per step)
     const double want_slots = per_seed * n_seeds + 64;
     if (want_slots >= 4294967295.0) return fail(ctx, DKB_EINVAL, "too many seeds for the seed table");
     ctx->seed_slots = (uint32_t)want_slots;
     CU(cudaMalloc(&ctx->d_sslots, (size_t)ctx->seed_slots * 64));
-    if (!ctx->gf && !getenv("DKB_NO_PROBE_ARRAY")) {  // probe array: 8 words per seed (dkb_device.cuh)
+    if (!ctx->gf) {  // probe array: 8 words per seed (dkb_device.cuh)
       const double want_probe = 8.0 * n_seeds + 64;
       if (want_probe >= 4294967295.0) return fail(ctx, DKB_EINVAL, "too many seeds for the probe array");
       ctx->probe_slots = (uint32_t)want_probe;
@@ -1125,26 +1120,6 @@ int dkb_table_build(dkb_ctx *ctx, const uint64_t *keys, const uint32_t *variant_
     CU(cudaStreamSynchronize(st));
     ctx->bloom_bits_set = h_stats[0];
     ctx->n_live = (size_t)h_stats[1];
-    // Optional (DKB_L2_PERSIST_MB=n): set n MB of L2 aside for persisting lines and mark the
-    // L2 filter as such for everything launched on the scan stream.
-    if (const char *e = getenv("DKB_L2_PERSIST_MB")) {
-      const size_t want = (size_t)atol(e) << 20;
-      cudaStreamAttrValue av;
-      memset(&av, 0, sizeof(av));
-      if (want && ctx->gf) {
-        CU(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, want));
-        size_t bytes = (size_t)ctx->bloom_words * 4;
-        int max_win = 0;
-        CU(cudaDeviceGetAttribute(&max_win, cudaDevAttrMaxAccessPolicyWindowSize, ctx->device));
-        if (bytes > (size_t)max_win) bytes = (size_t)max_win;
-        av.accessPolicyWindow.base_ptr = ctx->d_bloom;
-        av.accessPolicyWindow.num_bytes = bytes;
-        av.accessPolicyWindow.hitRatio = bytes <= want ? 1.0f : (float)want / (float)bytes;
-        av.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-        av.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-      }
-      CU(cudaStreamSetAttribute(ctx->s_scan, cudaStreamAttributeAccessPolicyWindow, &av));
-    }
     return DKB_OK;
   }();
   cleanup();

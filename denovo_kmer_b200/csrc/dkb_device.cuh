@@ -14,11 +14,7 @@ constexpr int SCAN_WARPS = SCAN_THREADS / 32;
 constexpr int CHUNK = 64;                  // stream positions per lane per tile (4 words)
 constexpr int WTILE = 32 * CHUNK;          // positions per warp tile (512 B of bases)
 constexpr int WTILE_WORDS = WTILE / 16;    // 128 uint32 words of bases per warp tile
-#ifndef DKB_STREAM_LD
-#define DKB_STREAM_LD 1
-#endif
-// 202 KB seed filter resident in shared memory (136 KB in TMA builds, whose stream ring needs 66 KB)
-constexpr int BLOOM_WORDS = DKB_STREAM_LD == 2 ? 34816 : 51712;
+constexpr int BLOOM_WORDS = 51712;         // 202 KB seed filter resident in shared memory
 // per-warp list of the filter-hit ids of one (macro) tile; denser tiles take several passes.
 // Behind the pre-filter (mode 2) a macro tile has a handful of hits: 32 ids do, and the 6 KB go
 // to the pre-filter instead (configs[1] 7.09 -> 7.23 Tbases/s; k = 21 at stride 8 4.14 -> 4.04).
@@ -39,24 +35,7 @@ constexpr size_t SCAN_SMEM_BYTES = (size_t)BLOOM_WORDS * 4 + scan_lists_bytes(0)
 // random loads per clock against 1.0 with a large one: scripts/micro/l2_gather.cu).
 constexpr size_t SCAN_SMEM_BYTES_GF = scan_lists_bytes(1);       // L2 filter, no pre-filter
 constexpr size_t SCAN_SMEM_BYTES_PRE = scan_lists_bytes(2);      // + pre_words * 4
-
-// DKB_STREAM_LD: how the macro path (strides 8, 16) reads the base stream.
-//   0  read-only loads at normal L2 priority        3  evict-first loads
-//   1  (default) normal priority in the shared-memory filter mode, evict-first in the L2 modes
-//   2  TMA: one lane per warp issues a 1-D bulk copy (cp.async.bulk) of each group of
-//      sub-tiles into a per-warp shared-memory ring, completion on an mbarrier; the stream
-//      never touches the LSU/L1 path the filter lookups need
-#ifndef DKB_STREAM_LD
-#define DKB_STREAM_LD 1
-#endif
-#ifndef DKB_TMA_STAGES
-#define DKB_TMA_STAGES 2
-#endif
 constexpr int MACRO_GS = 2;  // sub-tiles per group of the macro path
-constexpr int TMA_NST = DKB_TMA_STAGES;
-constexpr uint32_t TMA_STAGE_BYTES = MACRO_GS * 512 + 16;  // + the 16 bytes that hold the halo word
-constexpr size_t SCAN_TMA_BYTES =
-    DKB_STREAM_LD == 2 ? (size_t)SCAN_WARPS * TMA_NST * (TMA_STAGE_BYTES + 8) : 0;  // ring + mbarriers
 
 constexpr int MAX_SEED_LEN = 15;             // 30 bits: leaves SEED_EMPTY outside the seed space
 constexpr uint32_t SEED_MULT = 0x9E3779B1u;  // odd multiplier of the filter hash
@@ -111,14 +90,10 @@ __host__ __device__ __forceinline__ uint32_t bloom_bits(uint32_t seed, uint32_t 
 
 __host__ __device__ __forceinline__ uint64_t kmer_mask(int k) { return (1ull << (2 * k)) - 1; }
 
-// DKB_CANON: which filter modes key their seeds by the strand-canonical form of the s-mer,
-// min(s-mer, its reverse complement): 0 none, 1 the L2 filter modes (default), 2 all.  Both
-// orientations of a haplotype then share their seeds: half the seeds in the filters and the
-// seed table, for ~7 more instructions per lookup.
-#ifndef DKB_CANON
-#define DKB_CANON 1
-#endif
-__host__ __device__ constexpr bool canon_for_mode(int fm) { return DKB_CANON == 2 || (DKB_CANON == 1 && fm > 0); }
+// The L2 filter modes key their seeds by the strand-canonical form of the s-mer, min(s-mer,
+// its reverse complement).  Both orientations of a haplotype then share their seeds: half the
+// seeds in the filters and the seed table, for ~7 more instructions per lookup.
+__host__ __device__ constexpr bool canon_for_mode(int fm) { return fm > 0; }
 
 // Reverse complement of an s-mer held in the low 2s bits (stream order either way: first base
 // least significant), cshift = 32 - 2s; x must be masked to its 2s bits.
@@ -151,16 +126,6 @@ __device__ __forceinline__ uint64_t base_reverse(uint64_t v, int k) {
 __device__ __forceinline__ uint64_t l2_policy_evict_last() {
   uint64_t p;
   asm("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-__device__ __forceinline__ uint64_t l2_policy_normal() {
-  uint64_t p;
-  asm("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-  uint64_t p;
-  asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
   return p;
 }
 __device__ __forceinline__ uint4 ldg_v4_hint(const void *ptr, uint64_t pol) {

@@ -17,12 +17,6 @@
 #pragma once
 #include "dkb_device.cuh"
 
-#ifndef DKB_X
-// Timing experiments only, wrong counts (scripts/ab_build.sh; DESIGN.md §4 "where the time goes"):
-// 1 rounds without their load, 2 no rounds, 6 no stage C, 7 no hit handling at all (macro path).
-#define DKB_X 0
-#endif
-
 namespace dkb {
 
 // FM = filter mode (dkb_device.cuh): 0 seed filter in shared memory, 1 in L2, 2 in L2 behind a
@@ -311,9 +305,6 @@ struct ScanWarp {
 
   // Queue the lanes' verified seeds (2 * seed-table slot + read orientation, stream position) for stage C.
   __device__ __forceinline__ void push_verified(bool found, uint32_t slot, uint32_t p) {
-#if DKB_X == 6
-    found = found && p == 0xFFFFFFFFu;  // timing experiment: no stage C
-#endif
     const uint32_t bal = __ballot_sync(FULL_MASK, found);
     if (bal == 0) return;
     if (found) cq[(ct + __popc(bal & lt_mask)) & (CQ_CAP - 1)] = (uint64_t)slot << 32 | p;
@@ -402,9 +393,7 @@ struct ScanWarp {
         uint32_t flip;
         const uint32_t x = canon(cut_seed(w, b), flip);
         lx[r] = x;
-#if DKB_X != 1
         if (has) lv[r] = ld_slot_word(vhome(x));
-#endif
         lidx |= ((b & 31) | flip << 7) << (8 * r);
       }
       if (!__any_sync(FULL_MASK, a != 0)) break;
@@ -646,16 +635,9 @@ struct ScanWarp {
       asm("mad.wide.u32 %0, %1, 4, %2;" : "=l"(ga) : "r"((uint32_t)(prod >> 32)), "l"(P.bloom));
       // (no L1 allocation: the filter is far larger than L1, and leaving L1 to the loads
       // that need it is worth 4 %; the same hint on stream or table loads costs 1-2 %)
-#ifndef DKB_FILTER_POLICY
-#define DKB_FILTER_POLICY 0  // experiment: 0 evict-last hint, 1 no hint
-#endif
       if (pass) {
-#if DKB_FILTER_POLICY == 0
         asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.u32 %0, [%1], %2;"
                      : "=r"(word[i]) : "l"(ga), "l"(keep));
-#else
-        asm volatile("ld.global.nc.L1::no_allocate.u32 %0, [%1];" : "=r"(word[i]) : "l"(ga));
-#endif
       }
     }
 #pragma unroll
@@ -767,55 +749,14 @@ struct ScanWarp {
   }
 };
 
-// ---- stream loads (DKB_STREAM_LD: dkb_device.cuh) -------------------------------------
+// ---- stream loads of the macro path ----------------------------------------------------
 // Shared-memory filter mode: normal L2 priority - its filter hits are frequent and re-read
 // their bases from L2 right after (evict-first costs 6 % at 250 candidates).  L2 filter modes:
 // evict-first - hits are rare there, and the stream must not push the filter and the tables out.
 template <int FM>
 __device__ __forceinline__ uint4 ld_stream_v4(const uint32_t *p) {
-#if DKB_STREAM_LD == 0
-  return __ldg(reinterpret_cast<const uint4 *>(p));
-#elif DKB_STREAM_LD == 3
-  return __ldcs(reinterpret_cast<const uint4 *>(p));
-#else
   if (FM == 0) return __ldg(reinterpret_cast<const uint4 *>(p));
   return __ldcs(reinterpret_cast<const uint4 *>(p));
-#endif
-}
-
-// TMA pieces: mbarrier + 1-D bulk copy global -> shared (shared addresses as 32-bit values)
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAIT_%=:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra DONE_%=;\n"
-      "bra WAIT_%=;\n"
-      "DONE_%=:\n"
-      "}" ::"r"(bar), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar,
-                                         uint64_t policy) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;"
-      ::"r"(dst), "l"(src), "r"(bytes), "r"(bar), "l"(policy) : "memory");
-}
-__device__ __forceinline__ uint4 lds_v4(uint32_t addr) {
-  uint4 v;
-  asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr));
-  return v;
-}
-__device__ __forceinline__ uint32_t lds_u32(uint32_t addr) {
-  uint32_t v;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
-  return v;
 }
 
 // tile -> registers.  Streaming (evict-first) loads: the stream is read once
@@ -937,86 +878,6 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) k_scan(const ScanParams P) {
         acc = acc << LPT | W.stage_a_sub(w, mk[j]);
       }
     };
-#if DKB_STREAM_LD == 2
-    // ---- TMA staging: per warp a ring of TMA_NST stages, one group (GS sub-tiles + the halo
-    // word's 16 bytes) each, filled by 1-D bulk copies that lane 0 issues and an mbarrier per
-    // stage completes.  The copy of the group TMA_NST ahead is issued when a stage has been
-    // consumed, so nothing of the stream is held in registers across a group and no stream
-    // load occupies an L1 line or a scoreboard of this warp.
-    uint8_t *ring_base = reinterpret_cast<uint8_t *>(hl_all + SCAN_WARPS * HL_CAP);
-    const uint32_t ring_a = (uint32_t)__cvta_generic_to_shared(ring_base) + warp * TMA_NST * TMA_STAGE_BYTES;
-    const uint32_t bar_a = (uint32_t)__cvta_generic_to_shared(ring_base) +
-                           SCAN_WARPS * TMA_NST * TMA_STAGE_BYTES + warp * TMA_NST * 8;
-    if (lane == 0) {
-#pragma unroll
-      for (int i = 0; i < TMA_NST; i++) mbar_init(bar_a + 8 * i, 1);
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    const uint64_t stream_pol = l2_policy_evict_first();
-    struct GroupCursor {
-      UnitCursor u;
-      int g;
-    };
-    auto advance = [&](GroupCursor &q) {
-      if (++q.g == GPM) { q.u.unit += n_warps; q.u.settle_seg(P); q.g = 0; }
-    };
-    GroupCursor pc{c, 0}, cc{c, 0};
-    uint32_t direct = 0, phase = 0;  // one bit per stage: read word by word / mbarrier parity
-    auto issue = [&](int st) {       // the group at pc -> stage st
-      const ScanSegment &S = P.seg[pc.u.seg];
-      const uint32_t t0 = pc.u.local(P) * SUB + pc.g * GS;
-      if ((t0 + GS) * WTILE_WORDS + 4 <= S.n_bwords) {
-        direct &= ~(1u << st);
-        if (lane == 0) {
-          constexpr uint32_t bytes = HALO ? TMA_STAGE_BYTES : GS * 512;
-          mbar_expect_tx(bar_a + 8 * st, bytes);
-          bulk_g2s(ring_a + st * TMA_STAGE_BYTES, S.bases + (size_t)t0 * WTILE_WORDS, bytes, bar_a + 8 * st,
-                   stream_pol);
-        }
-      } else {
-        direct |= 1u << st;
-      }
-    };
-#pragma unroll
-    for (int i = 0; i < TMA_NST; i++)
-      if (pc.u.live(P)) { issue(i); advance(pc); }
-    int st = 0;
-    while (cc.u.live(P)) {
-      uint4 v[GS];
-      uint32_t edge = 0;
-      if ((direct >> st) & 1) {
-        load_group_tail(P.seg[cc.u.seg], cc.u.local(P) * SUB + cc.g * GS, v, edge);
-      } else {
-        mbar_wait(bar_a + 8 * st, (phase >> st) & 1);
-        phase ^= 1u << st;
-        const uint32_t sa = ring_a + st * TMA_STAGE_BYTES;
-#pragma unroll
-        for (int j = 0; j < GS; j++) v[j] = lds_v4(sa + j * 512 + lane * 16);
-        if (HALO) edge = lds_u32(sa + GS * 512);
-      }
-      uint2 mk[GS];
-      load_flags(P.seg[cc.u.seg], cc.u.local(P) * SUB + cc.g * GS, mk);
-      const uint32_t cur_macro = cc.u.local(P);
-      const bool last_group = cc.g == GPM - 1;
-      advance(cc);
-      filter_group(v, edge, mk);
-      // the stage's words have been used (stage A depends on them), so it can be refilled
-      __syncwarp();
-      if (pc.u.live(P)) { issue(st); advance(pc); }
-      st = st + 1 == TMA_NST ? 0 : st + 1;
-      if (last_group) {
-        W.consume_pending(acc);
-        const uint32_t w0[5] = {0, 0, 0, 0, 0};
-        W.handle_hits(acc, 0, w0, cur_macro * SUB * WTILE);
-        acc = 0;
-        if (cc.u.live(P) && cc.u.seg != W.cur) {  // the warp's next unit lies in another stream
-          W.drain();
-          W.cur = cc.u.seg;
-        }
-      }
-    }
-#else
     auto load_group = [&](const ScanSegment &S, uint32_t t0, uint4 (&v)[GS], uint32_t &edge) {
       const uint32_t wb = t0 * WTILE_WORDS + lane * 4;
       if ((t0 + GS) * WTILE_WORDS + 4 <= S.n_bwords) {
@@ -1060,11 +921,7 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) k_scan(const ScanParams P) {
         }
         asm volatile("" : "+r"(nxt_edge));
         const uint32_t w0[5] = {0, 0, 0, 0, 0};
-#if DKB_X != 7  // (7: timing / traffic experiment without any hit handling)
         W.handle_hits(acc, 0, w0, cur_macro * SUB * WTILE);
-#else
-        asm volatile("" ::"r"(acc));  // the lookups stay
-#endif
         acc = 0;
         if (c.live(P) && c.seg != W.cur) {  // the warp's next unit lies in another stream
           W.drain();
@@ -1072,7 +929,6 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) k_scan(const ScanParams P) {
         }
       }
     }
-#endif
   } else {
   uint32_t nxt[5];
   if (c.live(P)) load_tile(P.seg[c.seg], c.local(P), lane, nxt);
@@ -1092,9 +948,7 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) k_scan(const ScanParams P) {
         acc_prev = 0;
         W.cur = c.seg;
       }
-#if DKB_X != 2
       W.start_local(acc_prev, w, base_prev);
-#endif
 #pragma unroll
       for (int i = 0; i < 5; i++) w[i] = nxt[i];
       base_prev = c.local(P) * WTILE;

@@ -1,9 +1,8 @@
 // dkb_scan_inst.cu - the instantiations of kernel 2 for ONE probe stride (DKB_INST_D = 1, 2,
 // 4, 8 or 16), compiled as its own translation unit so that the strides build in parallel.
 // Shared-memory filter: 1..4 filter bits; L2 filter with and without the pre-filter (strides
-// 2..16): 1..2 bits; each with and
-// without the profiling counters, and in region mode (RG, DESIGN.md §2) without them.
-// DKB_AB_BUILD (scripts/ab_build.sh): 2 filter bits only.
+// 2..16): 1..2 bits; each with and without the profiling counters, and in region mode (RG,
+// DESIGN.md §2) without them.
 #include "dkb_scan.cuh"
 
 #ifndef DKB_INST_D
@@ -31,14 +30,12 @@ scan_fn DKB_CAT(pick_scan_d, DKB_INST_D)(int NH, int fm, bool prof, bool rg) {
 #if DKB_INST_D >= 8
   PICK(2, 3) PICK(2, 4)
 #endif
-#ifndef DKB_AB_BUILD
   PICK(1, 0) PICK(3, 0) PICK(4, 0)
 #if DKB_INST_D >= 2
   PICK(1, 1) PICK(1, 2)
 #endif
 #if DKB_INST_D >= 8
   PICK(1, 3) PICK(1, 4)
-#endif
 #endif
 #undef PICK
   return nullptr;
