@@ -26,6 +26,18 @@
 using namespace dkb;
 static_assert(DKB_MAX_MULTI == dkb::MAX_SEGMENTS, "ABI and kernel disagree on the batches per launch");
 
+// A device buffer and its capacity, in elements.
+template <typename T>
+struct DevBuf {
+  T *p = nullptr;
+  size_t cap = 0;
+  void free() {
+    if (p) cudaFree(p);
+    p = nullptr;
+    cap = 0;
+  }
+};
+
 struct dkb_ctx {
   int device = 0;
   int k = 0;
@@ -75,21 +87,39 @@ struct dkb_ctx {
   double scan_ms_total = 0.0;
   uint64_t scan_launches_timed = 0;
   float last_scan_ms = 0.f;
-  struct Stage {
-    uint32_t *bases = nullptr, *mask = nullptr;
-    size_t bases_cap = 0, mask_cap = 0;  // in words
+  // A staging slot: device buffers one launch's inputs are copied into.  Slots come in rings of
+  // two, so that the copies for one launch overlap the scan of the previous one (stage_slot).
+  struct Slot {
+    cudaEvent_t copied = nullptr, freed = nullptr;  // on the copy / scan stream
+    bool in_use = false;                            // a scan reads the slot until `freed`
+    void free() {
+      if (copied) cudaEventDestroy(copied);
+      if (freed) cudaEventDestroy(freed);
+      copied = freed = nullptr;
+    }
+  };
+  template <typename S>
+  struct Ring {
+    S slot[2];
+    int next = 0;
+  };
+  // host batches of every host submit form
+  struct Stage : Slot {
+    DevBuf<uint32_t> bases, mask;
     // raw reads for the device-side packer (dkb_batch_submit_reads)
-    uint8_t *seq = nullptr, *qual = nullptr;
-    uint64_t *offsets = nullptr, *nib = nullptr;
-    size_t seq_cap = 0, qual_cap = 0, off_cap = 0, nib_cap = 0;  // bytes / elements
+    DevBuf<uint8_t> seq, qual;
+    DevBuf<uint64_t> offsets, nib;
     // zero list of dkb_batch_submit_sparse
-    uint32_t *zoff = nullptr;
-    uint8_t *zbytes = nullptr;
-    size_t zoff_cap = 0, zbytes_cap = 0;
-    cudaEvent_t copied = nullptr, freed = nullptr;
-    bool in_use = false;
-  } stage[2];
-  int next_stage = 0;
+    DevBuf<uint32_t> zoff;
+    DevBuf<uint8_t> zbytes;
+    void free() {
+      bases.free(); mask.free();
+      seq.free(); qual.free(); offsets.free(); nib.free();
+      zoff.free(); zbytes.free();
+      Slot::free();
+    }
+  };
+  Ring<Stage> stage;
   uint64_t scan_launches = 0, positions_scanned = 0;
   // multi-GPU: the communicator and the overlapped count reduction (dkb_reduce_push)
   void *comm = nullptr;  // ncclComm_t
@@ -108,22 +138,24 @@ struct dkb_ctx {
     const uint64_t *offsets = nullptr, *lo = nullptr, *hi = nullptr;
     size_t n_reads = 0;
     uint64_t n_pos = 0;
-    bool set = false;
-  } loci, mloci[DKB_MAX_MULTI];
-  int mloci_n = 0;
-  bool mloci_set = false;
+  } loci[DKB_MAX_MULTI];
+  int loci_n = 0;           // batches the pending loci are for
+  bool loci_set = false;    // loci are pending
+  bool loci_multi = false;  // ... from dkb_batch_set_loci_multi
   // the read-locus index of one launch's batches on the device (concatenated, one segment per
-  // batch with reads), double-buffered like `stage`
-  struct LociStage {
-    uint64_t *offsets = nullptr, *lo = nullptr, *hi = nullptr;
-    uint32_t *start = nullptr, *tile = nullptr;
-    ulonglong2 *span = nullptr;
-    size_t off_cap = 0, lo_cap = 0, hi_cap = 0, start_cap = 0, tile_cap = 0, span_cap = 0;
+  // batch with reads)
+  struct LociStage : Slot {
+    DevBuf<uint64_t> offsets, lo, hi;
+    DevBuf<uint32_t> start, tile;
+    DevBuf<ulonglong2> span;
     uint32_t tile_base[DKB_MAX_MULTI] = {}, n_tiles[DKB_MAX_MULTI] = {};  // per batch of the submit
-    cudaEvent_t copied = nullptr, freed = nullptr;
-    bool in_use = false;
-  } lstage[2];
-  int next_lstage = 0;
+    void free() {
+      offsets.free(); lo.free(); hi.free();
+      start.free(); tile.free(); span.free();
+      Slot::free();
+    }
+  };
+  Ring<LociStage> lstage;
 };
 
 namespace {
@@ -164,10 +196,7 @@ void dfree(T *&p) {
 }
 
 // Forget whatever loci are pending, single-batch or multi-batch.
-void drop_loci(dkb_ctx *c) {
-  c->loci.set = false;
-  c->mloci_set = false;
-}
+void drop_loci(dkb_ctx *c) { c->loci_set = false; }
 
 void free_table(dkb_ctx *c) {
   dfree(c->d_keys); dfree(c->d_variant); dfree(c->d_allele); dfree(c->d_dead);
@@ -386,22 +415,34 @@ scan_fn pick_scan(int D, int NH, int fm, bool prof, bool rg) {
   return nullptr;
 }
 
-// One scan launch over n_seg device-resident packed streams (each into its sample's counters).
+// The batches of one submit: batch i has n_positions[i] stream positions and is counted into
+// the counters of samples[i].  Its packed streams are at d_bases[i] / d_mask[i] on the device:
+// the caller's for the device forms, a staging slot's for the host forms (their staging step
+// sets them).
+struct Batches {
+  bool multi;  // a multi-batch submit: it takes the loci of dkb_batch_set_loci_multi
+  int n;
+  const uint64_t *n_positions;
+  const int *samples;
+  const uint32_t *const *d_bases, *const *d_mask;
+};
+
+// One scan launch over the batches (each into its sample's counters).
 // Region mode: ls is the read-locus index of all of them (stage_loci).
-int launch_scan(dkb_ctx *ctx, int n_seg, const uint32_t *const *d_bases, const uint32_t *const *d_mask,
-                const uint64_t *n_positions, const int *samples, dkb_ctx::LociStage *ls) {
+int launch_scan(dkb_ctx *ctx, const Batches &b, dkb_ctx::LociStage *ls) {
+  const uint64_t *n_positions = b.n_positions;
   ScanParams P;
   memset(&P, 0, sizeof(P));
   // work units: tiles, or macro tiles of 4-8 tiles at strides 8/16
   const uint32_t per_unit = ctx->D >= 8 ? 32u / (64u / ctx->D) : 1u;
   uint64_t units = 0, total_pos = 0;
   P.n_seg = 0;
-  for (int i = 0; i < n_seg; i++) {
+  for (int i = 0; i < b.n; i++) {
     if (n_positions[i] == 0) continue;
     ScanSegment &S = P.seg[P.n_seg++];
-    S.bases = d_bases[i];
-    S.mask = d_mask[i];
-    S.counts = ctx->d_counts + (size_t)samples[i] * ctx->n_entries;
+    S.bases = b.d_bases[i];
+    S.mask = b.d_mask[i];
+    S.counts = ctx->d_counts + (size_t)b.samples[i] * ctx->n_entries;
     S.n_pos = (uint32_t)n_positions[i];
     S.n_bwords = (uint32_t)dkb_stream_bases_words(n_positions[i]);
     S.n_mwords = (uint32_t)dkb_stream_mask_words(n_positions[i]);
@@ -436,9 +477,9 @@ int launch_scan(dkb_ctx *ctx, int n_seg, const uint32_t *const *d_bases, const u
   const bool rg = ctx->regions;
   if (rg) {
     if (!ls) return fail(ctx, DKB_ESTATE, "region mode scans batches with their loci");
-    P.read_start = ls->start;
-    P.tile_read = ls->tile;
-    P.read_span = ls->span;
+    P.read_start = ls->start.p;
+    P.tile_read = ls->tile.p;
+    P.read_span = ls->span.p;
     P.entry_win = ctx->d_entry_win;
   }
   scan_fn fn = pick_scan(ctx->D, ctx->NH, ctx->gf ? (ctx->pre_words ? 2 : 1) + (ctx->gate ? 2 : 0) : 0, ctx->prof, rg);
@@ -479,123 +520,119 @@ int launch_scan(dkb_ctx *ctx, int n_seg, const uint32_t *const *d_bases, const u
   CU(cudaGetLastError());
   CU(cudaEventRecord(ev.second, ctx->s_scan));
   ctx->ev_pending.push_back(ev);
-  if (rg) {
-    CU(cudaEventRecord(ls->freed, ctx->s_scan));
-    ls->in_use = true;
-  }
   ctx->scan_launches++;
   ctx->positions_scanned += total_pos;
   ctx->finalised = false;
   return DKB_OK;
 }
 
-int launch_scan(dkb_ctx *ctx, const uint32_t *d_bases, const uint32_t *d_mask, uint64_t n_positions,
-                int sample, dkb_ctx::LociStage *ls) {
-  return launch_scan(ctx, 1, &d_bases, &d_mask, &n_positions, &sample, ls);
-}
-
-// Grow a staging buffer (elements of T); the caller has made sure no kernel still reads it.
-template <typename T>
-int grow(dkb_ctx *ctx, T *&p, size_t &cap, size_t need) {
-  if (cap >= need) return DKB_OK;
-  dfree(p);
-  cap = 0;  // a failed allocation must not leave a capacity behind a null pointer
-  const size_t want = need + need / 8 + 256;
-  T *q = nullptr;
-  CU(cudaMalloc(&q, want * sizeof(T)));
-  p = q;
-  cap = want;
-  return DKB_OK;
-}
-
-// Copy n host-resident batches into one staging buffer, each at a 16-byte-aligned offset, on
-// the copy stream; the scan stream waits for the copies.  d_bases / d_mask get the batches'
-// device addresses.  After launching the scan the caller records st->freed and sets in_use.
-int stage_batches(dkb_ctx *ctx, int n, const uint32_t *const *bases2, const uint32_t *const *mask1,
-                  const uint64_t *n_positions, const uint32_t **d_bases, const uint32_t **d_mask,
-                  dkb_ctx::Stage *&out) {
-  size_t bo[DKB_MAX_MULTI], mo[DKB_MAX_MULTI], bw = 0, mw = 0;
-  for (int i = 0; i < n; i++) {
-    bo[i] = bw;
-    mo[i] = mw;
-    bw += (dkb_stream_bases_words(n_positions[i]) + 3) / 4 * 4;
-    mw += (dkb_stream_mask_words(n_positions[i]) + 3) / 4 * 4;
-  }
-  dkb_ctx::Stage &st = ctx->stage[ctx->next_stage];
-  ctx->next_stage ^= 1;
+// The slot protocol of both staging rings.  stage_slot takes the ring's next slot; fill(slot)
+// grows its buffers (grow) and queues the copies of one launch's inputs into them on the copy
+// stream, which first waits until the slot's last scan is done with them; the scan stream then
+// waits for the copies.  release() hands the slots of a launch back once its scan is queued.
+template <typename S, typename Fill>
+int stage_slot(dkb_ctx *ctx, dkb_ctx::Ring<S> &ring, S *&out, Fill fill) {
+  S &st = ring.slot[ring.next];
+  ring.next ^= 1;
   if (st.in_use) CU(cudaStreamWaitEvent(ctx->s_copy, st.freed, 0));
-  if (st.bases_cap < bw || st.mask_cap < mw) {
-    // the previous scan may still read the old buffers
-    if (st.in_use) CU(cudaEventSynchronize(st.freed));
-    int rc;
-    if ((rc = grow(ctx, st.bases, st.bases_cap, bw)) != DKB_OK) return rc;
-    if ((rc = grow(ctx, st.mask, st.mask_cap, mw)) != DKB_OK) return rc;
-  }
-  for (int i = 0; i < n; i++) {
-    d_bases[i] = st.bases + bo[i];
-    d_mask[i] = st.mask + mo[i];
-    if (n_positions[i] == 0) continue;
-    CU(cudaMemcpyAsync(st.bases + bo[i], bases2[i], dkb_stream_bases_words(n_positions[i]) * 4,
-                       cudaMemcpyHostToDevice, ctx->s_copy));
-    CU(cudaMemcpyAsync(st.mask + mo[i], mask1[i], dkb_stream_mask_words(n_positions[i]) * 4, cudaMemcpyHostToDevice,
-                       ctx->s_copy));
-  }
+  int rc = fill(st);
+  if (rc != DKB_OK) return rc;
   CU(cudaEventRecord(st.copied, ctx->s_copy));
   CU(cudaStreamWaitEvent(ctx->s_scan, st.copied, 0));
   out = &st;
   return DKB_OK;
 }
 
-const char *const NO_PROF_REGIONS = "region mode has no scan kernel with profiling counters (dkb_profile_counters 0)";
-
-// Region mode: the loci dkb_batch_set_loci left for this submit (consumed whatever the outcome;
-// out->set stays false in whole-stream mode).
-int take_loci(dkb_ctx *ctx, uint64_t n_positions, dkb_ctx::Loci *out) {
-  *out = dkb_ctx::Loci{};
-  if (!ctx->regions) return DKB_OK;
-  const dkb_ctx::Loci l = ctx->loci;
-  const bool multi = ctx->mloci_set;
-  drop_loci(ctx);
-  if (multi) return fail(ctx, DKB_ESTATE, "region mode: multi-batch loci are pending, but this is a single-batch submit");
-  if (!l.set) return fail(ctx, DKB_ESTATE, "region mode: dkb_batch_set_loci must come before every single-batch submit");
-  if (ctx->prof) return fail(ctx, DKB_ESTATE, NO_PROF_REGIONS);
-  if (l.n_pos != n_positions)
-    return fail(ctx, DKB_EINVAL, "the loci's reads cover " + std::to_string(l.n_pos) + " stream positions, the batch " +
-                                     std::to_string(n_positions));
-  *out = l;
+// Grow a buffer of slot st to at least `need` elements.  The slot's last scan may still read
+// the old buffer, so the host waits for that scan first - only when the buffer must grow.
+template <typename T>
+int grow(dkb_ctx *ctx, dkb_ctx::Slot &st, DevBuf<T> &b, size_t need) {
+  if (b.cap >= need) return DKB_OK;
+  if (st.in_use) CU(cudaEventSynchronize(st.freed));
+  b.free();  // a failed allocation must not leave a capacity behind a null pointer
+  const size_t want = need + need / 8 + 256;
+  T *q = nullptr;
+  CU(cudaMalloc(&q, want * sizeof(T)));
+  b.p = q;
+  b.cap = want;
   return DKB_OK;
 }
 
-// The same for a multi-batch submit: the loci dkb_batch_set_loci_multi left, one set per batch.
-int take_loci_multi(dkb_ctx *ctx, int n_batches, const uint64_t *n_positions, dkb_ctx::Loci *out) {
-  for (int i = 0; i < DKB_MAX_MULTI; i++) out[i] = dkb_ctx::Loci{};
-  if (!ctx->regions) return DKB_OK;
-  const bool single = ctx->loci.set, multi = ctx->mloci_set;
-  const int n = ctx->mloci_n;
+int release(dkb_ctx *ctx, std::initializer_list<dkb_ctx::Slot *> slots) {
+  for (dkb_ctx::Slot *st : slots) {
+    if (!st) continue;
+    CU(cudaEventRecord(st->freed, ctx->s_scan));
+    st->in_use = true;
+  }
+  return DKB_OK;
+}
+
+// Copy n host-resident batches into one staging buffer, each at a 16-byte-aligned offset.
+// d_bases / d_mask get the batches' device addresses.
+int stage_batches(dkb_ctx *ctx, const Batches &b, const uint32_t *const *bases2, const uint32_t *const *mask1,
+                  const uint32_t **d_bases, const uint32_t **d_mask, dkb_ctx::Stage *&out) {
+  const uint64_t *n_positions = b.n_positions;
+  size_t bo[DKB_MAX_MULTI], mo[DKB_MAX_MULTI], bw = 0, mw = 0;
+  for (int i = 0; i < b.n; i++) {
+    bo[i] = bw;
+    mo[i] = mw;
+    bw += (dkb_stream_bases_words(n_positions[i]) + 3) / 4 * 4;
+    mw += (dkb_stream_mask_words(n_positions[i]) + 3) / 4 * 4;
+  }
+  return stage_slot(ctx, ctx->stage, out, [&](dkb_ctx::Stage &st) -> int {
+    int rc;
+    if ((rc = grow(ctx, st, st.bases, bw)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st, st.mask, mw)) != DKB_OK) return rc;
+    for (int i = 0; i < b.n; i++) {
+      d_bases[i] = st.bases.p + bo[i];
+      d_mask[i] = st.mask.p + mo[i];
+      if (n_positions[i] == 0) continue;
+      CU(cudaMemcpyAsync(st.bases.p + bo[i], bases2[i], dkb_stream_bases_words(n_positions[i]) * 4,
+                         cudaMemcpyHostToDevice, ctx->s_copy));
+      CU(cudaMemcpyAsync(st.mask.p + mo[i], mask1[i], dkb_stream_mask_words(n_positions[i]) * 4,
+                         cudaMemcpyHostToDevice, ctx->s_copy));
+    }
+    return DKB_OK;
+  });
+}
+
+const char *const NO_PROF_REGIONS = "region mode has no scan kernel with profiling counters (dkb_profile_counters 0)";
+
+// Region mode: take the loci pending for this submit, whatever its outcome - dkb_batch_set_loci's
+// for a single-batch submit, dkb_batch_set_loci_multi's for a multi-batch one - into l[0, n).
+int take_loci(dkb_ctx *ctx, bool multi, dkb_ctx::Loci *l, int &n) {
+  const bool set = ctx->loci_set;
+  n = ctx->loci_n;
+  for (int i = 0; i < n; i++) l[i] = ctx->loci[i];
   drop_loci(ctx);
-  if (single) return fail(ctx, DKB_ESTATE, "region mode: single-batch loci are pending, but this is a multi-batch submit");
-  if (!multi)
-    return fail(ctx, DKB_ESTATE, "region mode: dkb_batch_set_loci_multi must come before every multi-batch submit");
+  if (set && ctx->loci_multi != multi)
+    return fail(ctx, DKB_ESTATE, multi ? "region mode: single-batch loci are pending, but this is a multi-batch submit"
+                                       : "region mode: multi-batch loci are pending, but this is a single-batch submit");
+  if (!set)
+    return fail(ctx, DKB_ESTATE, multi ? "region mode: dkb_batch_set_loci_multi must come before every multi-batch submit"
+                                       : "region mode: dkb_batch_set_loci must come before every single-batch submit");
   if (ctx->prof) return fail(ctx, DKB_ESTATE, NO_PROF_REGIONS);
-  if (n != n_batches)
+  return DKB_OK;
+}
+
+// Region mode: the taken loci must be for the submit's batches and cover their positions.
+int check_loci_positions(dkb_ctx *ctx, const Batches &b, const dkb_ctx::Loci *l, int n) {
+  if (n != b.n)
     return fail(ctx, DKB_EINVAL, "the loci are for " + std::to_string(n) + " batches, the submit has " +
-                                     std::to_string(n_batches));
-  if (n && !n_positions) return fail(ctx, DKB_EINVAL, "null argument");
+                                     std::to_string(b.n));
   for (int i = 0; i < n; i++)
-    if (ctx->mloci[i].n_pos != n_positions[i])
-      return fail(ctx, DKB_EINVAL, "batch " + std::to_string(i) + ": the loci's reads cover " +
-                                       std::to_string(ctx->mloci[i].n_pos) + " stream positions, the batch " +
-                                       std::to_string(n_positions[i]));
-  for (int i = 0; i < n; i++) out[i] = ctx->mloci[i];
+    if (l[i].n_pos != b.n_positions[i])
+      return fail(ctx, DKB_EINVAL, (b.multi ? "batch " + std::to_string(i) + ": " : std::string()) +
+                                       "the loci's reads cover " + std::to_string(l[i].n_pos) +
+                                       " stream positions, the batch " + std::to_string(b.n_positions[i]));
   return DKB_OK;
 }
 
 // Copy the loci of a launch's n batches (copy stream) into one LociStage, concatenated, and
 // build their read-locus index with one launch of each index kernel (scan stream, ahead of the
-// scan).  ls = nullptr in whole-stream mode, and when no batch has reads (nothing to scan).
+// scan).  ls = nullptr when no batch has reads (nothing to scan).
 int stage_loci(dkb_ctx *ctx, int n, const dkb_ctx::Loci *l, dkb_ctx::LociStage *&ls) {
   ls = nullptr;
-  if (n == 0 || !l[0].set) return DKB_OK;
   LociSegments S;
   memset(&S, 0, sizeof(S));
   uint32_t tile_base[DKB_MAX_MULTI], n_tiles[DKB_MAX_MULTI];
@@ -616,38 +653,33 @@ int stage_loci(dkb_ctx *ctx, int n, const dkb_ctx::Loci *l, dkb_ctx::LociStage *
   S.read_base[S.n_seg] = (uint32_t)nr;
   S.tile_base[S.n_seg] = (uint32_t)nt;
   const size_t no = nr + S.n_seg;  // offsets: n_reads + 1 per segment
-  dkb_ctx::LociStage &st = ctx->lstage[ctx->next_lstage];
-  ctx->next_lstage ^= 1;
-  if (st.in_use) CU(cudaStreamWaitEvent(ctx->s_copy, st.freed, 0));
-  if (st.off_cap < no || st.lo_cap < nr || st.hi_cap < nr || st.start_cap < nr || st.span_cap < nr ||
-      st.tile_cap < nt) {
-    if (st.in_use) CU(cudaEventSynchronize(st.freed));  // the previous scan may still read the old index
+  int rc = stage_slot(ctx, ctx->lstage, ls, [&](dkb_ctx::LociStage &st) -> int {
     int rc;
-    if ((rc = grow(ctx, st.offsets, st.off_cap, no)) != DKB_OK) return rc;
-    if ((rc = grow(ctx, st.lo, st.lo_cap, nr)) != DKB_OK) return rc;
-    if ((rc = grow(ctx, st.hi, st.hi_cap, nr)) != DKB_OK) return rc;
-    if ((rc = grow(ctx, st.start, st.start_cap, nr)) != DKB_OK) return rc;
-    if ((rc = grow(ctx, st.span, st.span_cap, nr)) != DKB_OK) return rc;
-    if ((rc = grow(ctx, st.tile, st.tile_cap, nt)) != DKB_OK) return rc;
-  }
-  for (uint32_t j = 0; j < S.n_seg; j++) {
-    const dkb_ctx::Loci &b = l[batch_of[j]];
-    const size_t r0 = S.read_base[j];
-    CU(cudaMemcpyAsync(st.offsets + r0 + j, b.offsets, (b.n_reads + 1) * 8, cudaMemcpyHostToDevice, ctx->s_copy));
-    CU(cudaMemcpyAsync(st.lo + r0, b.lo, b.n_reads * 8, cudaMemcpyHostToDevice, ctx->s_copy));
-    CU(cudaMemcpyAsync(st.hi + r0, b.hi, b.n_reads * 8, cudaMemcpyHostToDevice, ctx->s_copy));
-  }
-  CU(cudaEventRecord(st.copied, ctx->s_copy));
-  CU(cudaStreamWaitEvent(ctx->s_scan, st.copied, 0));
+    if ((rc = grow(ctx, st, st.offsets, no)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st, st.lo, nr)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st, st.hi, nr)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st, st.start, nr)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st, st.span, nr)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st, st.tile, nt)) != DKB_OK) return rc;
+    for (uint32_t j = 0; j < S.n_seg; j++) {
+      const dkb_ctx::Loci &b = l[batch_of[j]];
+      const size_t r0 = S.read_base[j];
+      CU(cudaMemcpyAsync(st.offsets.p + r0 + j, b.offsets, (b.n_reads + 1) * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+      CU(cudaMemcpyAsync(st.lo.p + r0, b.lo, b.n_reads * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+      CU(cudaMemcpyAsync(st.hi.p + r0, b.hi, b.n_reads * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+    }
+    return DKB_OK;
+  });
+  if (rc != DKB_OK) return rc;
   const int TB = 256;
-  k_read_loci<<<(uint32_t)((nr + TB - 1) / TB), TB, 0, ctx->s_scan>>>(S, st.offsets, st.lo, st.hi, st.start, st.span);
-  k_tile_reads<<<(uint32_t)((nt + TB - 1) / TB), TB, 0, ctx->s_scan>>>(S, st.start, st.tile);
+  k_read_loci<<<(uint32_t)((nr + TB - 1) / TB), TB, 0, ctx->s_scan>>>(S, ls->offsets.p, ls->lo.p, ls->hi.p,
+                                                                     ls->start.p, ls->span.p);
+  k_tile_reads<<<(uint32_t)((nt + TB - 1) / TB), TB, 0, ctx->s_scan>>>(S, ls->start.p, ls->tile.p);
   CU(cudaGetLastError());
   for (int i = 0; i < n; i++) {
-    st.tile_base[i] = tile_base[i];
-    st.n_tiles[i] = n_tiles[i];
+    ls->tile_base[i] = tile_base[i];
+    ls->n_tiles[i] = n_tiles[i];
   }
-  ls = &st;
   return DKB_OK;
 }
 
@@ -794,19 +826,56 @@ int check_sample(dkb_ctx *ctx, int sample) {
                                    : "sample must be in [0, " + std::to_string(ctx->n_samples) + ")");
 }
 
-// Checks shared by the multi-batch submits, after their loci have been taken.
-int check_multi(dkb_ctx *ctx, int n_batches, const void *bases2, const void *mask1, const uint64_t *n_positions,
-                const int *samples) {
-  if (n_batches < 0 || n_batches > DKB_MAX_MULTI) return fail(ctx, DKB_EINVAL, "n_batches out of range");
-  if (n_batches && (!bases2 || !mask1 || !n_positions || !samples)) return fail(ctx, DKB_EINVAL, "null argument");
-  for (int i = 0; i < n_batches; i++) {
-    if (check_sample(ctx, samples[i]) != DKB_OK) return DKB_EINVAL;
-    if (n_positions[i] > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
+// The checks of the packed-stream forms (dkb_batch_submit, _device and their multi forms):
+// n_batches and the arrays of a multi-batch submit, then the stream pointers of every batch
+// with positions, which on the device must be aligned too.
+int check_streams(dkb_ctx *ctx, const Batches &b, const uint32_t *const *bases2, const uint32_t *const *mask1,
+                  bool device) {
+  if (b.multi && (b.n < 0 || b.n > DKB_MAX_MULTI)) return fail(ctx, DKB_EINVAL, "n_batches out of range");
+  if (b.multi && b.n && (!bases2 || !mask1 || !b.n_positions || !b.samples))
+    return fail(ctx, DKB_EINVAL, "null argument");
+  for (int i = 0; i < b.n; i++) {
+    if (b.n_positions[i] == 0) continue;
+    if (!bases2[i] || !mask1[i]) return fail(ctx, DKB_EINVAL, "null stream pointer");
+    if (device && ((uintptr_t)bases2[i] & 15)) return fail(ctx, DKB_EINVAL, "d_bases2 must be 16-byte aligned");
+    if (device && ((uintptr_t)mask1[i] & 3)) return fail(ctx, DKB_EINVAL, "d_mask1 must be 4-byte aligned");
   }
   return DKB_OK;
 }
 
-// One batch's loci, as dkb_batch_set_loci takes them, checked and kept in *out (out->set untouched).
+// The path every submit form takes.  check() is the form's own argument checks; stage(st) is
+// the device step of a host form: it puts the batches on the device (in staging slot st) and
+// sets b.d_bases / b.d_mask.  The pending loci are used up whatever the outcome.
+template <typename Check, typename StageFn>
+int submit(dkb_ctx *ctx, const Batches &b, Check check, StageFn stage) {
+  if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
+  if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
+  dkb_ctx::Loci loci[DKB_MAX_MULTI];
+  int n_loci = 0, rc;
+  if (ctx->regions && (rc = take_loci(ctx, b.multi, loci, n_loci)) != DKB_OK) return rc;
+  if ((rc = check()) != DKB_OK) return rc;
+  bool any = false;
+  for (int i = 0; i < b.n; i++) {
+    if (check_sample(ctx, b.samples[i]) != DKB_OK) return DKB_EINVAL;
+    if (b.n_positions[i] > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
+    any |= b.n_positions[i] != 0;
+  }
+  // (after the form's checks: dkb_batch_submit_reads knows its positions once its offsets are checked)
+  if (ctx->regions && (rc = check_loci_positions(ctx, b, loci, n_loci)) != DKB_OK) return rc;
+  if (!any) return DKB_OK;
+  CU(cudaSetDevice(ctx->device));
+  dkb_ctx::Stage *st = nullptr;
+  dkb_ctx::LociStage *ls = nullptr;
+  if ((rc = stage(st)) != DKB_OK) return rc;
+  if (ctx->regions && (rc = stage_loci(ctx, b.n, loci, ls)) != DKB_OK) return rc;
+  if ((rc = launch_scan(ctx, b, ls)) != DKB_OK) return rc;
+  return release(ctx, {ls, st});
+}
+
+// The device step of the device forms: none.
+int on_device(dkb_ctx::Stage *&) { return DKB_OK; }
+
+// One batch's loci, as dkb_batch_set_loci takes them, checked and kept in *out.
 int check_loci(dkb_ctx *ctx, const uint64_t *offsets, const uint64_t *lo, const uint64_t *hi, size_t n_reads,
                dkb_ctx::Loci *out) {
   if ((uint64_t)n_reads >= 0x100000000ull) return fail(ctx, DKB_EINVAL, "too many reads in one batch (max 2^32 - 1)");
@@ -883,11 +952,11 @@ int dkb_ctx_create_family(int device, int k, int n_children, dkb_ctx **out) {
     CU(cudaSetDevice(device));
     CU(cudaStreamCreateWithFlags(&ctx->s_scan, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&ctx->s_copy, cudaStreamNonBlocking));
-    for (auto &st : ctx->stage) {
+    for (auto &st : ctx->stage.slot) {
       CU(cudaEventCreateWithFlags(&st.copied, cudaEventDisableTiming));
       CU(cudaEventCreateWithFlags(&st.freed, cudaEventDisableTiming));
     }
-    for (auto &st : ctx->lstage) {
+    for (auto &st : ctx->lstage.slot) {
       CU(cudaEventCreateWithFlags(&st.copied, cudaEventDisableTiming));
       CU(cudaEventCreateWithFlags(&st.freed, cudaEventDisableTiming));
     }
@@ -910,28 +979,8 @@ int dkb_ctx_destroy(dkb_ctx *ctx) {
   cudaDeviceSynchronize();
   free_table(ctx);
   dfree(ctx->d_prof);
-  for (auto &st : ctx->stage) {
-    dfree(st.bases);
-    dfree(st.mask);
-    dfree(st.seq);
-    dfree(st.qual);
-    dfree(st.offsets);
-    dfree(st.nib);
-    dfree(st.zoff);
-    dfree(st.zbytes);
-    if (st.copied) cudaEventDestroy(st.copied);
-    if (st.freed) cudaEventDestroy(st.freed);
-  }
-  for (auto &st : ctx->lstage) {
-    dfree(st.offsets);
-    dfree(st.lo);
-    dfree(st.hi);
-    dfree(st.start);
-    dfree(st.tile);
-    dfree(st.span);
-    if (st.copied) cudaEventDestroy(st.copied);
-    if (st.freed) cudaEventDestroy(st.freed);
-  }
+  for (auto &st : ctx->stage.slot) st.free();
+  for (auto &st : ctx->lstage.slot) st.free();
   for (auto *v : {&ctx->ev_pool, &ctx->ev_pending})
     for (auto &pr : *v) {
       cudaEventDestroy(pr.first);
@@ -1129,219 +1178,145 @@ int dkb_table_build(dkb_ctx *ctx, const uint64_t *keys, const uint32_t *variant_
 
 int dkb_batch_submit_device(dkb_ctx *ctx, const uint32_t *d_bases2, const uint32_t *d_mask1,
                             uint64_t n_positions, int sample) {
-  if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
-  if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
-  if (check_sample(ctx, sample) != DKB_OK) return DKB_EINVAL;
-  dkb_ctx::Loci loci;
-  int rc = take_loci(ctx, n_positions, &loci);
-  if (rc != DKB_OK) return rc;
-  if (n_positions == 0) return DKB_OK;
-  if (n_positions > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
-  if (!d_bases2 || !d_mask1) return fail(ctx, DKB_EINVAL, "null stream pointer");
-  if ((uintptr_t)d_bases2 & 15) return fail(ctx, DKB_EINVAL, "d_bases2 must be 16-byte aligned");
-  if ((uintptr_t)d_mask1 & 3) return fail(ctx, DKB_EINVAL, "d_mask1 must be 4-byte aligned");
-  CU(cudaSetDevice(ctx->device));
-  dkb_ctx::LociStage *ls;
-  if ((rc = stage_loci(ctx, 1, &loci, ls)) != DKB_OK) return rc;
-  return launch_scan(ctx, d_bases2, d_mask1, n_positions, sample, ls);
+  const Batches b{false, 1, &n_positions, &sample, &d_bases2, &d_mask1};
+  return submit(ctx, b, [&]() -> int { return check_streams(ctx, b, &d_bases2, &d_mask1, true); }, on_device);
 }
 
 int dkb_batch_submit_device_multi(dkb_ctx *ctx, int n_batches, const uint32_t *const *d_bases2,
                                   const uint32_t *const *d_mask1, const uint64_t *n_positions,
                                   const int *samples) {
-  if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
-  if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
-  dkb_ctx::Loci loci[DKB_MAX_MULTI];
-  int rc = take_loci_multi(ctx, n_batches, n_positions, loci);
-  if (rc != DKB_OK) return rc;
-  if ((rc = check_multi(ctx, n_batches, d_bases2, d_mask1, n_positions, samples)) != DKB_OK) return rc;
-  for (int i = 0; i < n_batches; i++) {
-    if (n_positions[i] == 0) continue;
-    if (!d_bases2[i] || !d_mask1[i]) return fail(ctx, DKB_EINVAL, "null stream pointer");
-    if ((uintptr_t)d_bases2[i] & 15) return fail(ctx, DKB_EINVAL, "d_bases2 must be 16-byte aligned");
-    if ((uintptr_t)d_mask1[i] & 3) return fail(ctx, DKB_EINVAL, "d_mask1 must be 4-byte aligned");
-  }
-  CU(cudaSetDevice(ctx->device));
-  dkb_ctx::LociStage *ls;
-  if ((rc = stage_loci(ctx, n_batches, loci, ls)) != DKB_OK) return rc;
-  return launch_scan(ctx, n_batches, d_bases2, d_mask1, n_positions, samples, ls);
+  const Batches b{true, n_batches, n_positions, samples, d_bases2, d_mask1};
+  return submit(ctx, b, [&]() -> int { return check_streams(ctx, b, d_bases2, d_mask1, true); }, on_device);
 }
 
 int dkb_batch_submit_multi(dkb_ctx *ctx, int n_batches, const uint32_t *const *bases2,
                            const uint32_t *const *mask1, const uint64_t *n_positions, const int *samples) {
-  if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
-  if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
-  dkb_ctx::Loci loci[DKB_MAX_MULTI];
-  int rc = take_loci_multi(ctx, n_batches, n_positions, loci);
-  if (rc != DKB_OK) return rc;
-  if ((rc = check_multi(ctx, n_batches, bases2, mask1, n_positions, samples)) != DKB_OK) return rc;
-  bool any = false;
-  for (int i = 0; i < n_batches; i++) {
-    if (n_positions[i] == 0) continue;
-    if (!bases2[i] || !mask1[i]) return fail(ctx, DKB_EINVAL, "null stream pointer");
-    any = true;
-  }
-  if (!any) return DKB_OK;
-  CU(cudaSetDevice(ctx->device));
   const uint32_t *d_bases[DKB_MAX_MULTI], *d_mask[DKB_MAX_MULTI];
-  dkb_ctx::Stage *st;
-  if ((rc = stage_batches(ctx, n_batches, bases2, mask1, n_positions, d_bases, d_mask, st)) != DKB_OK) return rc;
-  dkb_ctx::LociStage *ls;
-  if ((rc = stage_loci(ctx, n_batches, loci, ls)) != DKB_OK) return rc;
-  rc = launch_scan(ctx, n_batches, d_bases, d_mask, n_positions, samples, ls);
-  if (rc != DKB_OK) return rc;
-  CU(cudaEventRecord(st->freed, ctx->s_scan));
-  st->in_use = true;
-  return DKB_OK;
+  const Batches b{true, n_batches, n_positions, samples, d_bases, d_mask};
+  return submit(ctx, b, [&]() -> int { return check_streams(ctx, b, bases2, mask1, false); },
+                [&](dkb_ctx::Stage *&st) { return stage_batches(ctx, b, bases2, mask1, d_bases, d_mask, st); });
 }
 
 int dkb_batch_submit(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t *mask1,
                      uint64_t n_positions, int sample) {
-  if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
-  if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
-  if (check_sample(ctx, sample) != DKB_OK) return DKB_EINVAL;
-  dkb_ctx::Loci loci;
-  int rc = take_loci(ctx, n_positions, &loci);
-  if (rc != DKB_OK) return rc;
-  if (n_positions == 0) return DKB_OK;
-  if (n_positions > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
-  if (!bases2 || !mask1) return fail(ctx, DKB_EINVAL, "null stream pointer");
-  CU(cudaSetDevice(ctx->device));
   const uint32_t *d_bases, *d_mask;
-  dkb_ctx::Stage *st;
-  if ((rc = stage_batches(ctx, 1, &bases2, &mask1, &n_positions, &d_bases, &d_mask, st)) != DKB_OK) return rc;
-  dkb_ctx::LociStage *ls;
-  if ((rc = stage_loci(ctx, 1, &loci, ls)) != DKB_OK) return rc;
-  rc = launch_scan(ctx, d_bases, d_mask, n_positions, sample, ls);
-  if (rc != DKB_OK) return rc;
-  CU(cudaEventRecord(st->freed, ctx->s_scan));
-  st->in_use = true;
-  return DKB_OK;
+  const Batches b{false, 1, &n_positions, &sample, &d_bases, &d_mask};
+  return submit(ctx, b, [&]() -> int { return check_streams(ctx, b, &bases2, &mask1, false); },
+                [&](dkb_ctx::Stage *&st) { return stage_batches(ctx, b, &bases2, &mask1, &d_bases, &d_mask, st); });
 }
 
 int dkb_batch_submit_sparse(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t *zoff,
                             const uint8_t *zbytes, size_t zbytes_used, uint64_t n_positions, int sample) {
-  if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
-  if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
-  if (check_sample(ctx, sample) != DKB_OK) return DKB_EINVAL;
-  dkb_ctx::Loci loci;
-  int rc = take_loci(ctx, n_positions, &loci);
-  if (rc != DKB_OK) return rc;
-  if (n_positions == 0) return DKB_OK;
-  if (n_positions > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
-  if (!bases2 || !zoff || (zbytes_used && !zbytes)) return fail(ctx, DKB_EINVAL, "null stream pointer");
-  const size_t nb = dkb_zero_list_blocks(n_positions);
-  if ((zoff[nb] & 0x7FFFFFFFu) != zbytes_used) return fail(ctx, DKB_EINVAL, "zoff[n_blocks] != zbytes_used");
-  // the expander trusts the offsets: they must ascend inside zbytes, a plain-bits block is 256 bytes
-  for (size_t b = 0; b < nb; b++) {
-    const uint32_t cur = zoff[b] & 0x7FFFFFFFu, nxt = zoff[b + 1] & 0x7FFFFFFFu;
-    if (nxt < cur || nxt > zbytes_used || ((zoff[b] & 0x80000000u) && nxt - cur != 256u))
-      return fail(ctx, DKB_EINVAL, "malformed zero list (block offsets)");
-  }
-  CU(cudaSetDevice(ctx->device));
-  const size_t bw = dkb_stream_bases_words(n_positions), mw = dkb_stream_mask_words(n_positions);
-  dkb_ctx::Stage &st = ctx->stage[ctx->next_stage];
-  ctx->next_stage ^= 1;
-  const size_t zb1 = zbytes_used ? zbytes_used : 1;
-  if (st.in_use) CU(cudaStreamWaitEvent(ctx->s_copy, st.freed, 0));
-  if (st.bases_cap < bw || st.mask_cap < mw || st.zoff_cap < nb + 1 || st.zbytes_cap < zb1) {
-    if (st.in_use) CU(cudaEventSynchronize(st.freed));  // the previous scan may still read the old buffers
-    if ((rc = grow(ctx, st.bases, st.bases_cap, bw)) != DKB_OK) return rc;
-    if ((rc = grow(ctx, st.mask, st.mask_cap, mw)) != DKB_OK) return rc;
-    if ((rc = grow(ctx, st.zoff, st.zoff_cap, nb + 1)) != DKB_OK) return rc;
-    if ((rc = grow(ctx, st.zbytes, st.zbytes_cap, zb1)) != DKB_OK) return rc;
-  }
-  CU(cudaMemcpyAsync(st.bases, bases2, bw * 4, cudaMemcpyHostToDevice, ctx->s_copy));
-  CU(cudaMemcpyAsync(st.zoff, zoff, (nb + 1) * 4, cudaMemcpyHostToDevice, ctx->s_copy));
-  if (zbytes_used) CU(cudaMemcpyAsync(st.zbytes, zbytes, zbytes_used, cudaMemcpyHostToDevice, ctx->s_copy));
-  CU(cudaEventRecord(st.copied, ctx->s_copy));
-  CU(cudaStreamWaitEvent(ctx->s_scan, st.copied, 0));
-  k_expand_zero_list<<<(uint32_t)((nb + 7) / 8), 256, 0, ctx->s_scan>>>(st.zoff, st.zbytes, (uint32_t)nb,
-                                                                      (uint32_t)mw, st.mask);
-  CU(cudaGetLastError());
-  dkb_ctx::LociStage *ls;
-  if ((rc = stage_loci(ctx, 1, &loci, ls)) != DKB_OK) return rc;
-  rc = launch_scan(ctx, st.bases, st.mask, n_positions, sample, ls);
-  if (rc != DKB_OK) return rc;
-  CU(cudaEventRecord(st.freed, ctx->s_scan));
-  st.in_use = true;
-  return DKB_OK;
+  const uint32_t *d_bases, *d_mask;
+  const Batches b{false, 1, &n_positions, &sample, &d_bases, &d_mask};
+  auto check = [&]() -> int {
+    if (n_positions && (!bases2 || !zoff || (zbytes_used && !zbytes)))
+      return fail(ctx, DKB_EINVAL, "null stream pointer");
+    return DKB_OK;
+  };
+  return submit(ctx, b, check, [&](dkb_ctx::Stage *&slot) -> int {
+    // the zero list is checked here, once the batch's length is: its size follows from n_positions
+    const size_t nb = dkb_zero_list_blocks(n_positions);
+    if ((zoff[nb] & 0x7FFFFFFFu) != zbytes_used) return fail(ctx, DKB_EINVAL, "zoff[n_blocks] != zbytes_used");
+    // the expander trusts the offsets: they must ascend inside zbytes, a plain-bits block is 256 bytes
+    for (size_t i = 0; i < nb; i++) {
+      const uint32_t cur = zoff[i] & 0x7FFFFFFFu, nxt = zoff[i + 1] & 0x7FFFFFFFu;
+      if (nxt < cur || nxt > zbytes_used || ((zoff[i] & 0x80000000u) && nxt - cur != 256u))
+        return fail(ctx, DKB_EINVAL, "malformed zero list (block offsets)");
+    }
+    const size_t bw = dkb_stream_bases_words(n_positions), mw = dkb_stream_mask_words(n_positions);
+    const size_t zb1 = zbytes_used ? zbytes_used : 1;
+    int rc = stage_slot(ctx, ctx->stage, slot, [&](dkb_ctx::Stage &st) -> int {
+      int rc;
+      if ((rc = grow(ctx, st, st.bases, bw)) != DKB_OK) return rc;
+      if ((rc = grow(ctx, st, st.mask, mw)) != DKB_OK) return rc;
+      if ((rc = grow(ctx, st, st.zoff, nb + 1)) != DKB_OK) return rc;
+      if ((rc = grow(ctx, st, st.zbytes, zb1)) != DKB_OK) return rc;
+      CU(cudaMemcpyAsync(st.bases.p, bases2, bw * 4, cudaMemcpyHostToDevice, ctx->s_copy));
+      CU(cudaMemcpyAsync(st.zoff.p, zoff, (nb + 1) * 4, cudaMemcpyHostToDevice, ctx->s_copy));
+      if (zbytes_used) CU(cudaMemcpyAsync(st.zbytes.p, zbytes, zbytes_used, cudaMemcpyHostToDevice, ctx->s_copy));
+      return DKB_OK;
+    });
+    if (rc != DKB_OK) return rc;
+    k_expand_zero_list<<<(uint32_t)((nb + 7) / 8), 256, 0, ctx->s_scan>>>(slot->zoff.p, slot->zbytes.p, (uint32_t)nb,
+                                                                        (uint32_t)mw, slot->mask.p);
+    CU(cudaGetLastError());
+    d_bases = slot->bases.p;
+    d_mask = slot->mask.p;
+    return DKB_OK;
+  });
 }
 
 int dkb_batch_submit_reads(dkb_ctx *ctx, const uint8_t *seq, int seq_format, const uint8_t *qual,
                            const uint64_t *offsets, size_t n_reads, int min_baseq, int sample) {
-  if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
-  if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
-  if (check_sample(ctx, sample) != DKB_OK) return DKB_EINVAL;
-  if (seq_format != 0 && seq_format != 1) return fail(ctx, DKB_EINVAL, "seq_format must be 0 (ASCII) or 1 (BAM 4-bit)");
-  dkb_ctx::Loci loci;
-  if (n_reads == 0) return take_loci(ctx, 0, &loci);
-  if (!seq || !offsets) return fail(ctx, DKB_EINVAL, "null read buffer");
-  if (n_reads >= 0xFFFFFFFFull) return fail(ctx, DKB_EINVAL, "too many reads in one batch");
-  for (size_t r = 0; r < n_reads; r++)
-    if (offsets[r + 1] < offsets[r]) return fail(ctx, DKB_EINVAL, "offsets must not decrease");
-  const uint64_t n_pos = dkb_stream_positions(offsets, n_reads);
-  int rc = take_loci(ctx, n_pos, &loci);
-  if (rc != DKB_OK) return rc;
-  if (n_pos > 0xFFFFF000ull) return fail(ctx, DKB_EINVAL, "batch too long (max 2^32 - 4096 positions)");
-  const uint64_t n_bases = offsets[n_reads] - offsets[0];
-  CU(cudaSetDevice(ctx->device));
-  const size_t bw = dkb_stream_bases_words(n_pos), mw = dkb_stream_mask_words(n_pos);
-  // BAM keeps every read's 4-bit codes byte-aligned: (len + 1) / 2 bytes per read
-  std::vector<uint64_t> nib;
-  uint64_t seq_bytes = n_bases;
-  if (seq_format == 1) {
-    nib.resize(n_reads);
-    uint64_t b = 0;
-    for (size_t r = 0; r < n_reads; r++) {
-      nib[r] = b;
-      b += (offsets[r + 1] - offsets[r] + 1) / 2;
+  uint64_t n_pos = 0;  // known once the offsets are checked
+  const uint32_t *d_bases, *d_mask;
+  const Batches b{false, 1, &n_pos, &sample, &d_bases, &d_mask};
+  auto check = [&]() -> int {
+    if (seq_format != 0 && seq_format != 1) return fail(ctx, DKB_EINVAL, "seq_format must be 0 (ASCII) or 1 (BAM 4-bit)");
+    if (n_reads == 0) return DKB_OK;
+    if (!seq || !offsets) return fail(ctx, DKB_EINVAL, "null read buffer");
+    if (n_reads >= 0xFFFFFFFFull) return fail(ctx, DKB_EINVAL, "too many reads in one batch");
+    for (size_t r = 0; r < n_reads; r++)
+      if (offsets[r + 1] < offsets[r]) return fail(ctx, DKB_EINVAL, "offsets must not decrease");
+    n_pos = dkb_stream_positions(offsets, n_reads);
+    return DKB_OK;
+  };
+  return submit(ctx, b, check, [&](dkb_ctx::Stage *&slot) -> int {
+    const uint64_t n_bases = offsets[n_reads] - offsets[0];
+    const size_t bw = dkb_stream_bases_words(n_pos), mw = dkb_stream_mask_words(n_pos);
+    // BAM keeps every read's 4-bit codes byte-aligned: (len + 1) / 2 bytes per read
+    std::vector<uint64_t> nib;
+    uint64_t seq_bytes = n_bases;
+    if (seq_format == 1) {
+      nib.resize(n_reads);
+      uint64_t bytes = 0;
+      for (size_t r = 0; r < n_reads; r++) {
+        nib[r] = bytes;
+        bytes += (offsets[r + 1] - offsets[r] + 1) / 2;
+      }
+      seq_bytes = bytes;
     }
-    seq_bytes = b;
-  }
-  dkb_ctx::Stage &st = ctx->stage[ctx->next_stage];
-  ctx->next_stage ^= 1;
-  if (st.in_use) CU(cudaEventSynchronize(st.freed));  // buffers may be regrown below
-  if ((rc = grow(ctx, st.bases, st.bases_cap, bw)) != DKB_OK) return rc;
-  if ((rc = grow(ctx, st.mask, st.mask_cap, mw)) != DKB_OK) return rc;
-  if ((rc = grow(ctx, st.seq, st.seq_cap, (size_t)seq_bytes)) != DKB_OK) return rc;
-  if (qual && (rc = grow(ctx, st.qual, st.qual_cap, (size_t)n_bases)) != DKB_OK) return rc;
-  if ((rc = grow(ctx, st.offsets, st.off_cap, n_reads + 1)) != DKB_OK) return rc;
-  if (seq_format == 1 && (rc = grow(ctx, st.nib, st.nib_cap, n_reads)) != DKB_OK) return rc;
-  // the reads of this batch start at offsets[0] in the caller's arrays; device copies start at 0
-  const uint8_t *seq0 = seq_format == 1 ? seq : seq + offsets[0];
-  CU(cudaMemcpyAsync(st.seq, seq0, seq_bytes, cudaMemcpyHostToDevice, ctx->s_copy));
-  if (qual) CU(cudaMemcpyAsync(st.qual, qual + offsets[0], n_bases, cudaMemcpyHostToDevice, ctx->s_copy));
-  CU(cudaMemcpyAsync(st.offsets, offsets, (n_reads + 1) * 8, cudaMemcpyHostToDevice, ctx->s_copy));
-  if (seq_format == 1) {
-    CU(cudaMemcpyAsync(st.nib, nib.data(), n_reads * 8, cudaMemcpyHostToDevice, ctx->s_copy));
-    CU(cudaStreamSynchronize(ctx->s_copy));  // nib is a local vector
-  }
-  CU(cudaEventRecord(st.copied, ctx->s_copy));
-  CU(cudaStreamWaitEvent(ctx->s_scan, st.copied, 0));
-  PackParams Q;
-  Q.seq = st.seq;
-  Q.qual = qual ? st.qual : nullptr;
-  Q.offsets = st.offsets;
-  Q.nib_start = st.nib;
-  Q.n_reads = (uint32_t)n_reads;
-  Q.n_pos = n_pos;
-  Q.n_bwords = (uint32_t)bw;
-  Q.n_mwords = (uint32_t)mw;
-  Q.min_baseq = min_baseq;
-  Q.four_bit = seq_format;
-  Q.bases2 = st.bases;
-  Q.mask1 = st.mask;
-  const int TB = 256;
-  k_pack<<<(uint32_t)((mw + TB - 1) / TB), TB, 0, ctx->s_scan>>>(Q);
-  CU(cudaGetLastError());
-  dkb_ctx::LociStage *ls;
-  if ((rc = stage_loci(ctx, 1, &loci, ls)) != DKB_OK) return rc;
-  rc = launch_scan(ctx, st.bases, st.mask, n_pos, sample, ls);
-  if (rc != DKB_OK) return rc;
-  CU(cudaEventRecord(st.freed, ctx->s_scan));
-  st.in_use = true;
-  return DKB_OK;
+    int rc = stage_slot(ctx, ctx->stage, slot, [&](dkb_ctx::Stage &st) -> int {
+      int rc;
+      if ((rc = grow(ctx, st, st.bases, bw)) != DKB_OK) return rc;
+      if ((rc = grow(ctx, st, st.mask, mw)) != DKB_OK) return rc;
+      if ((rc = grow(ctx, st, st.seq, (size_t)seq_bytes)) != DKB_OK) return rc;
+      if (qual && (rc = grow(ctx, st, st.qual, (size_t)n_bases)) != DKB_OK) return rc;
+      if ((rc = grow(ctx, st, st.offsets, n_reads + 1)) != DKB_OK) return rc;
+      if (seq_format == 1 && (rc = grow(ctx, st, st.nib, n_reads)) != DKB_OK) return rc;
+      // the reads of this batch start at offsets[0] in the caller's arrays; device copies start at 0
+      const uint8_t *seq0 = seq_format == 1 ? seq : seq + offsets[0];
+      CU(cudaMemcpyAsync(st.seq.p, seq0, seq_bytes, cudaMemcpyHostToDevice, ctx->s_copy));
+      if (qual) CU(cudaMemcpyAsync(st.qual.p, qual + offsets[0], n_bases, cudaMemcpyHostToDevice, ctx->s_copy));
+      CU(cudaMemcpyAsync(st.offsets.p, offsets, (n_reads + 1) * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+      if (seq_format == 1) {
+        CU(cudaMemcpyAsync(st.nib.p, nib.data(), n_reads * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+        CU(cudaStreamSynchronize(ctx->s_copy));  // nib is a local vector
+      }
+      return DKB_OK;
+    });
+    if (rc != DKB_OK) return rc;
+    PackParams Q;
+    Q.seq = slot->seq.p;
+    Q.qual = qual ? slot->qual.p : nullptr;
+    Q.offsets = slot->offsets.p;
+    Q.nib_start = slot->nib.p;
+    Q.n_reads = (uint32_t)n_reads;
+    Q.n_pos = n_pos;
+    Q.n_bwords = (uint32_t)bw;
+    Q.n_mwords = (uint32_t)mw;
+    Q.min_baseq = min_baseq;
+    Q.four_bit = seq_format;
+    Q.bases2 = slot->bases.p;
+    Q.mask1 = slot->mask.p;
+    const int TB = 256;
+    k_pack<<<(uint32_t)((mw + TB - 1) / TB), TB, 0, ctx->s_scan>>>(Q);
+    CU(cudaGetLastError());
+    d_bases = slot->bases.p;
+    d_mask = slot->mask.p;
+    return DKB_OK;
+  });
 }
 
 int dkb_table_set_regions(dkb_ctx *ctx, const uint64_t *lo, const uint64_t *hi, uint32_t n_variants) {
@@ -1385,9 +1360,11 @@ int dkb_batch_set_loci(dkb_ctx *ctx, const uint64_t *offsets, const uint64_t *lo
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
   drop_loci(ctx);
   if (!ctx->regions) return fail(ctx, DKB_ESTATE, "dkb_batch_set_loci needs region mode (dkb_table_set_regions)");
-  int rc = check_loci(ctx, offsets, lo, hi, n_reads, &ctx->loci);
+  int rc = check_loci(ctx, offsets, lo, hi, n_reads, &ctx->loci[0]);
   if (rc != DKB_OK) return rc;
-  ctx->loci.set = true;
+  ctx->loci_n = 1;
+  ctx->loci_multi = false;
+  ctx->loci_set = true;
   return DKB_OK;
 }
 
@@ -1400,14 +1377,14 @@ int dkb_batch_set_loci_multi(dkb_ctx *ctx, int n_batches, const uint64_t *const 
   if (n_batches && (!offsets || !lo || !hi || !n_reads)) return fail(ctx, DKB_EINVAL, "null argument");
   uint64_t total = 0;  // reads are numbered across the launch's batches in 32 bits
   for (int i = 0; i < n_batches; i++) {
-    int rc = check_loci(ctx, offsets[i], lo[i], hi[i], n_reads[i], &ctx->mloci[i]);
+    int rc = check_loci(ctx, offsets[i], lo[i], hi[i], n_reads[i], &ctx->loci[i]);
     if (rc != DKB_OK) return rc;
     total += n_reads[i];
   }
   if (total >= 0x100000000ull) return fail(ctx, DKB_EINVAL, "too many reads in one launch (max 2^32 - 1)");
-  for (int i = 0; i < n_batches; i++) ctx->mloci[i].set = true;
-  ctx->mloci_n = n_batches;
-  ctx->mloci_set = true;
+  ctx->loci_n = n_batches;
+  ctx->loci_multi = true;
+  ctx->loci_set = true;
   return DKB_OK;
 }
 

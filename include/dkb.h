@@ -241,10 +241,10 @@ int dkb_table_set_regions(dkb_ctx *ctx, const uint64_t *lo, const uint64_t *hi, 
  * that submit with the batch; the buffers follow the submit's validity rule (dkb_batch_submit:
  * valid until dkb_sync; for _device too).  In region mode a single-batch submit without loci
  * returns DKB_ESTATE, and one whose loci cover a different number of stream positions
- * (dkb_stream_positions(offsets, n_reads) != n_positions) DKB_EINVAL; either way the loci are
- * used up.  DKB_ESTATE in whole-stream mode; DKB_EINVAL for descending offsets or
- * n_reads >= 2^32.  Region mode has no profiling counters: with dkb_profile_counters on, a
- * submit returns DKB_ESTATE. */
+ * (dkb_stream_positions(offsets, n_reads) != n_positions) DKB_EINVAL; every submit uses up the
+ * pending loci whatever its outcome.  DKB_ESTATE in whole-stream mode; DKB_EINVAL for descending
+ * offsets or n_reads >= 2^32.  Region mode has no profiling counters: with dkb_profile_counters
+ * on, a submit returns DKB_ESTATE. */
 int dkb_batch_set_loci(dkb_ctx *ctx, const uint64_t *offsets, const uint64_t *lo,
                        const uint64_t *hi, size_t n_reads);
 /* Region mode: the read loci of the NEXT multi-batch submit (dkb_batch_submit_multi or

@@ -15,7 +15,7 @@ import region_oracle as ro
 from denovo_kmer_b200 import synth
 from family_oracle import family_results
 from helpers import oracle_counts
-from test_gpu_regions import TUNINGS, _trimmed
+from test_gpu_regions import TUNINGS, _submit, _trimmed
 
 pytestmark = pytest.mark.gpu
 
@@ -24,12 +24,16 @@ MIN_BQ = 20
 
 
 def _split(dkb, fam, samples, parts, min_bq=MIN_BQ):
-    """Per sample, its reads cut into `parts` batches: [(sample, stream, loci, seq, qual, off)]."""
+    """Per sample, its reads cut into `parts` batches - that many even ones, or a list of the
+    batches' relative sizes: [(sample, stream, loci, seq, qual, off)]."""
     out = []
     for smp in samples:
         seq, qual, off = fam.reads[smp]
         lo, hi = fam.loci[smp]
-        cuts = np.linspace(0, len(off) - 1, parts + 1).astype(int)
+        if np.isscalar(parts):
+            cuts = np.linspace(0, len(off) - 1, parts + 1).astype(int)
+        else:
+            cuts = (np.cumsum([0] + list(parts)) / sum(parts) * (len(off) - 1)).astype(int)
         for a, b in zip(cuts[:-1], cuts[1:]):
             a0, b0 = int(off[a]), int(off[b])
             boff = off[a:b + 1] - off[a]
@@ -305,16 +309,23 @@ def test_every_region_twin_with_several_segments(dkb, adv_input, monkeypatch):
 
 
 # ---- pipelining ----------------------------------------------------------------------------
-@pytest.mark.parametrize("regions", [False, True])
-def test_multi_pipelined(dkb, orc, regions):
-    """Eight multi submits in a row without dkb_sync, interleaved with single submits (host and
-    device), so both staging buffers and both locus stages are reused; then the same steps with
-    reduce_push / reduce_flush after each on one GPU."""
+SINGLE_FORMS = ("submit", "sparse", "reads", "reads4")
+UNEVEN = (1, 6, 1, 10, 10, 10, 1, 6)
+
+
+@pytest.mark.parametrize("regions, parts", [pytest.param(r, p, id=f"{r}{'-uneven' if p == UNEVEN else ''}")
+                                            for p in (10, UNEVEN) for r in (False, True)])
+def test_multi_pipelined(dkb, orc, regions, parts):
+    """Multi submits in a row without dkb_sync, interleaved with single submits (host and
+    device multi; dkb_batch_submit, _sparse, _reads from ASCII and from 4-bit codes), so that
+    every form shares both staging buffers and both locus stages; then the same steps with
+    reduce_push / reduce_flush after each on one GPU.  The uneven split makes each staging
+    buffer and each locus stage grow while the other one's scan is queued."""
     k = 31
     trio = _trimmed(synth.make_trio_host(200_000, 12, 30, k, seed=45))
     entries = dkb.variant_kmers(trio.variant_tuples(), k)
     vlo, vhi = ro.windows(trio.variants, 400)
-    batches = _split(dkb, trio, range(3), 10)
+    batches = _split(dkb, trio, range(3), parts)
     if regions:
         want = _region_want(orc, entries, batches, vlo, vhi, k, 3)
     else:
@@ -323,30 +334,36 @@ def test_multi_pipelined(dkb, orc, regions):
         for smp in range(3):
             ks.count_reads(*trio.reads[smp], k, MIN_BQ, counts=want[smp])
     steps = _steps(batches, 3)
-    assert len(steps) == 10
+    assert len(steps) == (parts if np.isscalar(parts) else len(parts))
     for reduce in (False, True):
         keep = []
         with dkb.KmerCounter(k) as kc:
             kc.build_table(entries)
             if regions:
                 kc.set_regions(vlo, vhi)
-            n_multi = 0
+            l0 = kc.stats()["scan_launches"]
+            n_multi = n_single = launches = 0
             for i, step in enumerate(steps):
-                if i % 4 == 3:  # a single-batch submit per batch of this step
-                    for smp, st, loci, *_ in step:
-                        kc.submit(st, smp, loci=loci if regions else None)
+                if i % 4 == 3:  # a single-batch submit per batch of this step, the forms in turn
+                    for smp, st, loci, seq, qual, off in step:
+                        _submit(dkb, kc, SINGLE_FORMS[n_single % 4], seq, qual, off, smp, MIN_BQ,
+                                loci if regions else None)
+                        n_single += 1
+                        launches += st.n_positions > 0
                 else:
                     _submit_step(dkb, kc, step, "device" if i % 4 == 2 else "host", regions, keep)
                     n_multi += 1
+                    launches += any(b[1].n_positions > 0 for b in step)
                 if reduce:
                     kc.reduce_push(THR)
-            assert n_multi >= 6
+            assert n_multi >= 6 and n_single >= len(SINGLE_FORMS)
             if reduce:
                 kc.reduce_flush(THR)
                 red = kc.reduced_counts().copy()
                 _, _, _, calls = kc.results()
             kc.sync()
             keep.clear()
+            assert kc.stats()["scan_launches"] - l0 == launches
             got = kc.entry_counts().copy()
             assert np.array_equal(got.astype(np.uint64), want), (regions, reduce)
             if reduce:

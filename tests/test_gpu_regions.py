@@ -338,6 +338,14 @@ def test_region_refusals(dkb):
         n = (C.c_uint64 * 1)(st.n_positions)
         assert L.dkb_batch_submit_device_multi(h, 1, (C.c_void_p * 1)(b2.data_ptr()), (C.c_void_p * 1)(m1.data_ptr()),
                                                n, (C.c_int * 1)(0)) == _lib.ESTATE
+        # every single-batch form: a submit refused for a bad sample uses up its loci, and without
+        # loci a bad sample is refused for the missing loci
+        for form in ("submit", "sparse", "reads", "reads4", "device"):
+            for smp, loci, code in ((3, dkb.ReadLoci(off, lo, hi), _lib.EINVAL), (0, None, _lib.ESTATE),
+                                    (3, None, _lib.ESTATE)):
+                with pytest.raises(dkb.DkbError) as ei:
+                    _submit(dkb, kc, form, seq, qual, off, smp, 20, loci)
+                assert ei.value.code == code, (form, smp, loci is not None)
         kc.profile_counters(True)  # region mode has no profiling kernels: refused, never ungated
         assert L.dkb_batch_set_loci(h, u64(off), u64(lo), u64(hi), len(off) - 1) == _lib.OK
         assert L.dkb_batch_submit(h, st.bases2.ctypes.data, st.mask1.ctypes.data, st.n_positions, 0) == _lib.ESTATE
