@@ -21,6 +21,7 @@ pub struct DkbStats {
     pub bloom_hits: u64, pub seed_hits: u64, pub windows_probed: u64, pub window_hits: u64,
     pub scan_launches_timed: u64,
     pub scan_ms_total: f64, pub last_scan_ms: f32, pub prefilter_words: u32, pub gated_lookups: u32,
+    pub occupied_halves: u64, pub direct_halves: u64,
 }
 
 pub const DKB_ABI_VERSION: c_int = 1;

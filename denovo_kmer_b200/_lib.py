@@ -34,7 +34,7 @@ class Stats(C.Structure):
         "bloom_bits_set", "scan_launches", "positions_scanned", "bloom_hits", "seed_hits",
         "windows_probed", "window_hits", "scan_launches_timed")] + [
         ("scan_ms_total", C.c_double), ("last_scan_ms", C.c_float), ("prefilter_words", C.c_uint32),
-        ("gated_lookups", C.c_uint32)]
+        ("gated_lookups", C.c_uint32), ("occupied_halves", C.c_uint64), ("direct_halves", C.c_uint64)]
 
 
 # every symbol include/dkb.h declares: (restype, argtypes)

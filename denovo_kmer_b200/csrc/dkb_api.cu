@@ -72,6 +72,7 @@ struct dkb_ctx {
   uint32_t pre_words = 0;  // shared-memory pre-filter of the L2 filter mode
   bool want_pre = false;   // the tuner's choice
   uint64_t bloom_bits_set = 0;
+  uint64_t occupied_halves = 0, direct_halves = 0;  // seed-record halves with a designation; direct ones
   // counters and results
   uint32_t *d_counts = nullptr;  // [n_samples][n_entries]
   uint32_t *d_hits = nullptr, *d_distinct = nullptr, *d_nkmers = nullptr;
@@ -210,6 +211,7 @@ void free_table(dkb_ctx *c) {
   c->regions = false;  // a new table counts the whole stream until dkb_table_set_regions
   drop_loci(c);
   c->n_entries = c->n_live = 0;
+  c->occupied_halves = c->direct_halves = 0;
   c->n_variants = 0;
   c->finalised = false;
   c->red_pending = c->red_last = -1;  // snapshots of the old table's counters are void
@@ -1049,12 +1051,13 @@ int dkb_table_build(dkb_ctx *ctx, const uint64_t *keys, const uint32_t *variant_
   ctx->table_slots = pow2_at_least(8 * (uint64_t)n + 2);  // <= 0.25 entries per 2-slot bucket
   uint16_t *d_wi = nullptr, *d_wc = nullptr;
   uint32_t *d_slot_of = nullptr;
-  uint32_t *d_set = nullptr, *d_cov = nullptr;
+  uint32_t *d_set = nullptr, *d_cov = nullptr, *d_dir = nullptr;
   unsigned int *d_nseeds = nullptr;
   unsigned long long *d_stats = nullptr;
   cudaStream_t st = ctx->s_scan;
   auto cleanup = [&]() {
-    dfree(d_wi); dfree(d_wc); dfree(d_slot_of); dfree(d_set); dfree(d_cov); dfree(d_nseeds); dfree(d_stats);
+    dfree(d_wi); dfree(d_wc); dfree(d_slot_of); dfree(d_set); dfree(d_cov); dfree(d_dir); dfree(d_nseeds);
+    dfree(d_stats);
   };
   rc = [&]() -> int {
     CU(cudaMalloc(&ctx->d_keys, n1 * 8));
@@ -1105,13 +1108,15 @@ int dkb_table_build(dkb_ctx *ctx, const uint64_t *keys, const uint32_t *variant_
       k_mark_repeats<<<g1, TB, 0, st>>>(B);
       k_apply_dead<<<g1, TB, 0, st>>>(B);
       k_assign_seeds<<<g2, TB, 0, st>>>(B, ASSIGN_COUNT, d_set, set_slots - 1, d_nseeds, SeedTable{},
-                                        nullptr, nullptr, 0, nullptr, 0, seed_mult, ctx->NH);
+                                        nullptr, nullptr, 0, nullptr, 0, seed_mult, ctx->NH, nullptr);
       CU(cudaGetLastError());
     }
     unsigned int n_seeds = 0;
     CU(cudaMemcpyAsync(&n_seeds, d_nseeds, 4, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     ctx->n_seeds = n_seeds;
+    dfree(d_set);  // done with: the direct-record scratch below takes its place
+    d_set = nullptr;
     // Seed table: 64-byte slots (seed + a 32-byte record per read orientation), a quarter full, any
     // size.  Only occupied slots are ever touched by true hits, so the hot set is 32 B per seed
     // and orientation; an absent seed (a filter false positive) lands on a slot marked
@@ -1130,6 +1135,9 @@ int dkb_table_build(dkb_ctx *ctx, const uint64_t *keys, const uint32_t *variant_
     }
     CU(cudaMalloc(&d_cov, (size_t)ctx->seed_slots * 24));
     CU(cudaMemsetAsync(d_cov, 0, (size_t)ctx->seed_slots * 24, st));
+    const size_t dir_bytes = (size_t)ctx->seed_slots * 2 * DIR_WORDS * 4;  // per record half
+    CU(cudaMalloc(&d_dir, dir_bytes));
+    CU(cudaMemsetAsync(d_dir, 0, dir_bytes, st));
     ctx->bloom_words = ctx->gf ? l2_filter_words((double)n_seeds) / 4 * 4 : (uint32_t)BLOOM_WORDS;
     CU(cudaMalloc(&ctx->d_bloom, (size_t)ctx->bloom_words * 4));
     CU(cudaMemsetAsync(ctx->d_bloom, 0, (size_t)ctx->bloom_words * 4, st));
@@ -1150,25 +1158,33 @@ int dkb_table_build(dkb_ctx *ctx, const uint64_t *keys, const uint32_t *variant_
     }
     const SeedTable T = seed_table(ctx);
     k_init_slots<<<(uint32_t)((4 * (size_t)ctx->seed_slots + TB - 1) / TB), TB, 0, st>>>(T);
+    // build statistics, counted on the device (the filter can be 16 MB): filter bits set, live
+    // entries, occupied record halves, direct ones
+    CU(cudaMalloc(&d_stats, 32));
+    CU(cudaMemsetAsync(d_stats, 0, 32, st));
     if (n) {
       k_assign_seeds<<<g2, TB, 0, st>>>(B, ASSIGN_INSERT, nullptr, 0, nullptr, T, nullptr,
                                         ctx->d_bloom, ctx->bloom_words, ctx->d_pre, ctx->pre_words,
-                                        seed_mult, ctx->NH);
+                                        seed_mult, ctx->NH, nullptr);
       k_assign_seeds<<<g2, TB, 0, st>>>(B, ASSIGN_RECORD, nullptr, 0, nullptr, T, d_cov,
                                         ctx->d_bloom, ctx->bloom_words, ctx->d_pre, ctx->pre_words,
-                                        seed_mult, ctx->NH);
-      k_finish_records<<<(uint32_t)((2 * (size_t)ctx->seed_slots + TB - 1) / TB), TB, 0, st>>>(T, d_cov);
+                                        seed_mult, ctx->NH, nullptr);
+      const uint32_t gh = (uint32_t)((2 * (size_t)ctx->seed_slots + TB - 1) / TB);
+      k_finish_records<<<gh, TB, 0, st>>>(T, d_cov);
+      k_assign_seeds<<<g2, TB, 0, st>>>(B, ASSIGN_DIRECT, nullptr, 0, nullptr, T, d_cov,
+                                        ctx->d_bloom, ctx->bloom_words, ctx->d_pre, ctx->pre_words,
+                                        seed_mult, ctx->NH, d_dir);
+      k_finish_direct<<<gh, TB, 0, st>>>(T, d_cov, d_dir, ctx->k, ctx->s, d_stats + 2);
     }
-    // build statistics, counted on the device (the filter can be 16 MB)
-    CU(cudaMalloc(&d_stats, 16));
-    CU(cudaMemsetAsync(d_stats, 0, 16, st));
     k_build_stats<<<296, 256, 0, st>>>(ctx->d_bloom, ctx->bloom_words, ctx->d_dead, (uint32_t)n, d_stats);
     CU(cudaGetLastError());
-    unsigned long long h_stats[2] = {0, 0};
-    CU(cudaMemcpyAsync(h_stats, d_stats, 16, cudaMemcpyDeviceToHost, st));
+    unsigned long long h_stats[4] = {0, 0, 0, 0};
+    CU(cudaMemcpyAsync(h_stats, d_stats, 32, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     ctx->bloom_bits_set = h_stats[0];
     ctx->n_live = (size_t)h_stats[1];
+    ctx->occupied_halves = h_stats[2];
+    ctx->direct_halves = h_stats[3];
     return DKB_OK;
   }();
   cleanup();
@@ -1625,6 +1641,8 @@ int dkb_stats_get(dkb_ctx *ctx, dkb_stats *out) {
   out->last_scan_ms = ctx->last_scan_ms;
   out->prefilter_words = ctx->gf ? ctx->pre_words : 0;
   out->gated_lookups = ctx->gate ? 1u : 0u;
+  out->occupied_halves = ctx->occupied_halves;
+  out->direct_halves = ctx->direct_halves;
   return DKB_OK;
 }
 

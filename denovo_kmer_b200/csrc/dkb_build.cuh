@@ -165,6 +165,108 @@ __global__ void k_finish_records(const SeedTable T, const uint32_t *cov) {
   }
 }
 
+// ---- direct records (dkb_device.cuh; the proof is in DESIGN.md §4) ----------------------
+// Build scratch per record half, 8 words, zeroed: what its designations have in common.
+//   0     variant + 1                  1, 2  allele 0: e - j + 32, e + j + 1 (entry e, offset j)
+//   3, 4  the same for allele 1        5, 6  A0, A1: offsets designated by allele 0, 1
+//   7     flags: bit 4a + b = a window of allele a shows base b at X; DIRF_* below
+// Words 0-4 keep the first value written; a later designation with another value sets a flag.
+constexpr int DIR_WORDS = 8;
+constexpr uint32_t DIRF_REJECT = 1u << 8;    // a key with a second live owner, or a window without X
+constexpr uint32_t DIRF_VARIANT = 1u << 9;   // more than one variant
+constexpr uint32_t DIRF_SLOPE = 1u << 10;    // << 2a: e - j varies in allele a; << 2a + 1: e + j varies
+
+__device__ __forceinline__ void dir_same(uint32_t *w, uint32_t v, uint32_t *flags, uint32_t bit) {
+  const uint32_t old = atomicCAS(w, 0u, v);
+  if (old != 0u && old != v) atomicOr(flags, bit);
+}
+
+// Bases of a finished record (words 5-7 = wild) that are wild inside the covered range, i.e.
+// disputed by the designating windows: their number, and x = the first of them.
+__device__ __forceinline__ int disputed_bases(const uint32_t *rec, const uint32_t *cov, int &x) {
+  int n = 0;
+  x = 0;
+  for (int w = 2; w >= 0; w--) {
+    const uint32_t d = rec[5 + w] & cov[w];
+    n += __popc(d);
+    if (d) x = 16 * w + ((__ffs(d) - 1) >> 1);
+  }
+  return n >> 1;
+}
+
+// One designation (entry e of variant `var`, allele a, offset j, window v in stream order) into
+// the scratch d of its record half; `shared` = another live entry has e's key.
+__device__ __forceinline__ void direct_add(const uint32_t *rec, const uint32_t *cov, uint32_t *d,
+                                           uint32_t e, uint32_t var, int a, int j, uint64_t v, int k,
+                                           int E, bool shared) {
+  uint32_t *const flags = d + 7;
+  if (shared) atomicOr(flags, DIRF_REJECT);
+  atomicOr(d + 5 + a, 1u << j);
+  dir_same(d, var + 1, flags, DIRF_VARIANT);
+  dir_same(d + 1 + 2 * a, e - j + 32, flags, DIRF_SLOPE << (2 * a));
+  dir_same(d + 2 + 2 * a, e + j + 1, flags, DIRF_SLOPE << (2 * a + 1));
+  if (E + k > NB_BASES) return;  // no neighbourhood: never direct
+  int x;
+  if (disputed_bases(rec, cov, x) != 1) return;  // none, or too many (k_finish_direct decides)
+  const int o = E - j;                            // first base of the window in the neighbourhood
+  if (x < o || x >= o + k) atomicOr(flags, DIRF_REJECT);
+  else atomicOr(flags, 1u << (4 * a + (uint32_t)((v >> (2 * (x - o))) & 3)));
+}
+
+// One thread per record half: make the half direct where its designations allow it.
+// stats[0] += occupied halves, stats[1] += direct ones.
+__global__ void k_finish_direct(const SeedTable T, const uint32_t *cov, const uint32_t *dir, int k,
+                                int s, unsigned long long *stats) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;  // one thread per half
+  const int E = k - s;
+  bool occ = false, direct = false;
+  if (i < 2 * (size_t)T.n_slots && !(*slot_word(T, (uint32_t)(i >> 1), 0) & ST_FREE_BIT)) {
+    uint32_t *r = slot_word(T, (uint32_t)(i >> 1), 0, (int)(i & 1));
+    occ = r[1] != 0;
+    const uint32_t *d = dir + i * DIR_WORDS;
+    const uint32_t A0 = d[5], A1 = d[6], f = d[7];
+    const uint32_t seen0 = f & 0xFu, seen1 = (f >> 4) & 0xFu;
+    int x;
+    const int nx = disputed_bases(r, cov + i * 3, x);
+    direct = occ && E + k <= NB_BASES && !(f & (DIRF_REJECT | DIRF_VARIANT));
+    uint32_t pick0 = 0xFu, pick1 = 0xFu;
+    if (A0 && A1) {  // an SNV's two alleles: the same offsets, and one disputed base each shows its own way
+      direct = direct && A0 == A1 && nx == 1 && __popc(seen0) == 1 && __popc(seen1) == 1 && seen0 != seen1;
+      pick0 = seen0;
+      pick1 = seen1;
+    } else {  // one allele: no disputed base; X = the seed's first base, which every read matches
+      direct = direct && nx == 0;
+      x = E;
+      if (!A0) pick0 = 0;
+      if (!A1) pick1 = 0;
+    }
+    uint32_t c[2] = {0, 0}, neg = 0;
+    for (int a = 0; a < 2; a++) {
+      if (!(a ? A1 : A0)) continue;
+      if (!(f & (DIRF_SLOPE << (2 * a)))) {
+        c[a] = d[1 + 2 * a] - 32;  // e = c + j
+      } else if (!(f & (DIRF_SLOPE << (2 * a + 1)))) {
+        c[a] = d[2 + 2 * a] - 1;   // e = c - j
+        neg |= 1u << a;
+      } else {
+        direct = false;
+      }
+    }
+    if (direct) {
+      r[5] = c[0];
+      r[6] = c[1];
+      r[7] = (uint32_t)x | pick0 << DIR_PICK0 | pick1 << DIR_PICK1 | (neg & 1u) << DIR_NEG0 |
+             (neg >> 1) << DIR_NEG1;
+      r[1] |= INFO_DIRECT;
+    }
+  }
+  const uint32_t n_occ = __popc(__ballot_sync(FULL_MASK, occ)), n_dir = __popc(__ballot_sync(FULL_MASK, direct));
+  if ((threadIdx.x & 31) == 0) {
+    if (n_occ) atomicAdd(stats, (unsigned long long)n_occ);
+    if (n_dir) atomicAdd(stats + 1, (unsigned long long)n_dir);
+  }
+}
+
 // popcount of n words / number of zero bytes, for the build statistics (out[0], out[1])
 __global__ void k_build_stats(const uint32_t *words, uint32_t n_words, const uint8_t *dead,
                               uint32_t n_dead, unsigned long long *out) {
@@ -207,15 +309,16 @@ __device__ __forceinline__ void seedset_insert(uint32_t *set, uint32_t mask, uin
 //     G = floor((k-s+1)/D)*D along the haplotype, so neighbouring windows share
 //     them (2 seeds per SNV haplotype strand and class at k=31, s<=15);
 //   min-hash rule (no hints): the s-mer of the class with the smallest hash.
-// Three passes (the choice of offsets is the same in each):
+// Four passes (the choice of offsets is the same in each):
 //   ASSIGN_COUNT   add the seeds to `set` (sizing);
 //   ASSIGN_INSERT  record the offsets in the entry's slot, insert the seeds, set their filter bits;
-//   ASSIGN_RECORD  add offset and window to the record in the seed's slot.
-enum { ASSIGN_COUNT = 0, ASSIGN_INSERT = 1, ASSIGN_RECORD = 2 };
+//   ASSIGN_RECORD  add offset and window to the record in the seed's slot;
+//   ASSIGN_DIRECT  (after k_finish_records) add the designation to the direct-record scratch `dir`.
+enum { ASSIGN_COUNT = 0, ASSIGN_INSERT = 1, ASSIGN_RECORD = 2, ASSIGN_DIRECT = 3 };
 __global__ void k_assign_seeds(const BuildParams B, int pass, uint32_t *set, uint32_t set_mask,
                                unsigned int *n_seeds, const SeedTable T, uint32_t *cov,
                                uint32_t *bloom, uint32_t bloom_words, uint32_t *pre,
-                               uint32_t pre_words, uint32_t seed_mult, int n_hashes) {
+                               uint32_t pre_words, uint32_t seed_mult, int n_hashes, uint32_t *dir) {
   const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
   const uint32_t i = t >> 1;
   const int ori = t & 1;
@@ -236,6 +339,18 @@ __global__ void k_assign_seeds(const BuildParams B, int pass, uint32_t *set, uin
     const int hap_ori = (wi >> 15) & 1;  // orientation whose string reads along the haplotype
     u = wi & 0x7FFFu;
     if (ori != hap_ori) u = nwin - 1 - u;  // same window seen on the other strand
+  }
+  bool shared = false;  // ASSIGN_DIRECT: another live entry has this key (k_mark_repeats' walk)
+  if (pass == ASSIGN_DIRECT) {
+    uint32_t b = key_bucket(key, B.kt.bucket_mask);
+    for (bool open = false; !open && !shared; b = (b + 1) & B.kt.bucket_mask) {
+      for (int q = 0; q < KBUCKET; q++) {
+        const uint4 sl = B.kt.slots[b * KBUCKET + q];
+        const uint64_t tk = slot_key(sl);
+        if (tk == KEY_EMPTY) open = true;
+        else if (tk == key && sl.z != ENTRY_DEAD && sl.z != i) shared = true;
+      }
+    }
   }
   uint32_t offs = 0;
   const int W = 32 / (2 * D);  // bits per packed offset field
@@ -277,7 +392,12 @@ __global__ void k_assign_seeds(const BuildParams B, int pass, uint32_t *set, uin
       atomicOr(bloom + bloom_word(h, bloom_words), bloom_bits(seed, h, bloom_words, n_hashes));
     } else {
       const uint32_t slot = seedtab_find(T, seed);
-      record_add(slot_word(T, slot, 0, (int)flip), cov + ((size_t)slot * 2 + flip) * 3, j, v, k, E);
+      const size_t h = (size_t)slot * 2 + flip;
+      if (pass == ASSIGN_RECORD)
+        record_add(slot_word(T, slot, 0, (int)flip), cov + h * 3, j, v, k, E);
+      else
+        direct_add(slot_word(T, slot, 0, (int)flip), cov + h * 3, dir + h * DIR_WORDS, i, B.variant[i],
+                   B.allele[i], j, v, k, E, shared);
     }
   }
   if (pass == ASSIGN_INSERT) atomicOr(&B.kt.slots[B.slot_of[i]].w, offs);

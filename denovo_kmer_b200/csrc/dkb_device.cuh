@@ -155,10 +155,21 @@ __device__ __forceinline__ uint64_t ldg_u64_hint(const void *ptr, uint64_t pol) 
 //   word 0   (half 0 only) bits 0..29 the seed, bit 30 = slot is free, bit 31 = some seed whose
 //            home is this slot lives further along (a miss must walk on); see ST_*
 //   word 1   info: bit j = some key designates this seed at offset j (its window starts j
-//            bases before the seed)
+//            bases before the seed); bit 31 (INFO_DIRECT) = a DIRECT record, below
 //   word 2-4 nb, the NEIGHBOURHOOD: the 48 bases from E = k - s before the seed, 2 bits each,
 //            stream order - the union of all windows that designate the seed (2k - s <= 48)
 //   word 5-7 wild: both bits of a base set where the designating keys disagree, or none covers it
+// A DIRECT record (the build proves it, DESIGN.md §4) has every designation from one variant, at
+// most one per (offset j, allele), entry = c_a + sigma_a * j within allele a, and its windows agree
+// on every covered base except at most one, X (an SNV's base), which each allele shows one way.
+// Its wild mask is "not covered, or X": the covered range follows from info's lowest and highest
+// offset, so words 5-7 carry instead
+//   word 5, 6  c_0, c_1
+//   word 7     bits 0..5 X; bits 6..9: read bases at X that pick allele 0 (bit 6 + base);
+//              bits 10..13: those that pick allele 1; bit 14 / 15: sigma_0 / sigma_1 = -1
+// (a record that only one allele designates has no X: that allele takes every base at X = E, the
+// seed's first base, which the read matches anyway).  Stage C counts its windows straight from
+// the record, without the key table.
 // A lookup is ONE 4-byte load of word 0 unless the home slot carries ST_MOVED_BIT: a seed
 // absent from an unmarked home slot is absent from the table.
 // A read window can equal a designating key only if the read equals nb on the window's
@@ -182,6 +193,9 @@ __host__ __device__ __forceinline__ uint32_t seed_next(uint32_t slot, uint32_t n
   return slot + 1 == n_slots ? 0u : slot + 1;
 }
 constexpr int NB_BASES = 48;
+constexpr uint32_t INFO_DIRECT = 0x80000000u;  // info bit of a direct record (offsets j <= k - s <= 23)
+constexpr uint32_t INFO_OFFSETS = 0x00FFFFFFu;
+constexpr int DIR_PICK0 = 6, DIR_PICK1 = 10, DIR_NEG0 = 14, DIR_NEG1 = 15;  // word 7 of a direct record
 // Key table: 16-byte slots {key lo, key hi, entry index, packed designated
 // offsets}, buckets of 2 slots = one 32-byte L2 sector (two LDG.128), a
 // multimap: one slot per (key, owner) entry; a full bucket spills into the next.

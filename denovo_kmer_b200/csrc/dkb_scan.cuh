@@ -14,6 +14,8 @@
 // run is canonicalised and probed in the key table, one window per lane (stage C).  A slot
 // is counted only when its own designated offset for class (j % D) equals j, so a matching
 // window is counted exactly once however many seeds it contains (proof in DESIGN.md §4).
+// A direct record (an isolated SNV's seed, dkb_device.cuh) names its windows' entries itself:
+// its windows are counted in phase 1 without the key table.
 #pragma once
 #include "dkb_device.cuh"
 
@@ -130,6 +132,7 @@ struct ScanWarp {
   // longer cost one dependent L2 round trip each inside a single lane.
   // Region mode resolves the seed's read once here: a counted window contains the seed and
   // no separator, so it lies in the seed's read; phase 2 takes it from the owner lane.
+  // A direct record's windows are counted in phase 1 and leave no tasks for phase 2.
   __device__ __forceinline__ void stage_c(uint32_t n) {
     const int k = P.k, s = P.s, E = k - s;
     const uint64_t km = kmer_mask(k);
@@ -145,14 +148,27 @@ struct ScanWarp {
       // the sector stage B already touched)
       const uint4 *rp = P.st.slots + 2 * (size_t)(uint32_t)(e >> 32);  // e >> 32 = 2 * slot + flip
       const uint4 r0 = ldg_v4_hint(rp, keep), r1 = ldg_v4_hint(rp + 1, keep);
-      const uint32_t nb0 = r0.z, nb1 = r0.w, nb2 = r1.x, wd0 = r1.y, wd1 = r1.z, wd2 = r1.w;
+      const uint32_t nb0 = r0.z, nb1 = r0.w, nb2 = r1.x;
+      uint32_t wd0 = r1.y, wd1 = r1.z, wd2 = r1.w;
       uint32_t b[5], m[3];
 #pragma unroll
       for (int i = 0; i < 5; i++) b[i] = ld_bases(bw0 + i);
 #pragma unroll
       for (int i = 0; i < 3; i++) m[i] = ld_mask(mw0 + i);
-      info = r0.y;
+      info = r0.y & INFO_OFFSETS;
+      const bool direct = (r0.y & INFO_DIRECT) != 0;
       if (p >= (uint32_t)E && E + k <= NB_BASES) {
+        if (direct) {
+          // a direct record's wild mask: the bases no designated window covers (window j covers
+          // [E - j, E - j + k)), and X
+          const int lo = 2 * (E - (31 - __clz(info))), hi = 2 * (E + k - (__ffs(info) - 1));
+          const unsigned __int128 one = 1;
+          const unsigned __int128 wild =
+              ~(((one << hi) - 1) ^ ((one << lo) - 1)) | (unsigned __int128)3 << (2 * (r1.w & 63));
+          wd0 = (uint32_t)wild;
+          wd1 = (uint32_t)(wild >> 32);
+          wd2 = (uint32_t)(wild >> 64);
+        }
         // the read's neighbourhood (base 0 = p - E) and its mismatches, 2 bits per base
         const uint32_t sh = 2 * (start & 15);
         rn0 = __funnelshift_r(b[0], b[1], sh);
@@ -180,8 +196,28 @@ struct ScanWarp {
         const int jlo = E + k - R > 0 ? E + k - R : 0, jhi = E - Lm - 1;
         info = jhi >= jlo ? info & ((2u << jhi) - 1u) & ~((1u << jlo) - 1u) : 0u;
         if ((inv >> E) & ((1ull << s) - 1)) info = 0;  // an invalid base inside the seed itself
+        // Direct record: a window left here equals the key of allele a's designation at its offset
+        // j exactly when the read's base at X is one allele a shows there (DESIGN.md §4), and that
+        // key's only live entry is c_a + sigma_a * j: count it here, no key-table probe.
+        const uint32_t x = r1.w & 63;
+        const uint32_t rb = ((x < 16 ? rn0 : x < 32 ? rn1 : rn2) >> (2 * (x & 15))) & 3;
+        const bool a1 = (r1.w >> (DIR_PICK1 + rb)) & 1;
+        if (PROF && direct) n_probe += __popc(info);  // the windows the key table would have been asked about
+        if (direct && !a1 && !((r1.w >> (DIR_PICK0 + rb)) & 1)) info = 0;
         if constexpr (RG) {
           if (info) rd = find_read(p);  // (a chance seed match needs no read)
+        }
+        if (direct) {
+          const uint32_t c = a1 ? r1.z : r1.y;
+          const bool neg = (r1.w >> (a1 ? DIR_NEG1 : DIR_NEG0)) & 1;
+          uint32_t *const counts = P.seg[cur].counts;
+          while (info) {
+            const uint32_t j = __ffs(info) - 1;
+            info &= info - 1;
+            const uint32_t e = neg ? c - j : c + j;
+            if (in_region(rd, e)) atomicAdd(counts + e, 1u);
+            if (PROF) n_hit++;
+          }
         }
       } else {
         // no usable neighbourhood (stream start, or 2k - s > NB_BASES): every designated
@@ -208,6 +244,11 @@ struct ScanWarp {
       }
     }
     // ---- phase 2 ----
+    if (!__any_sync(FULL_MASK, info != 0)) {  // every window was counted in phase 1, or none survived
+      ch += n;
+      __syncwarp();
+      return;
+    }
     uint32_t cnt = __popc(info), incl = cnt;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {

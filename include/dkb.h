@@ -334,6 +334,9 @@ typedef struct dkb_stats {
   uint32_t prefilter_words;  /* L2 filter mode: words of the shared-memory pre-filter, 0 = none */
   uint32_t gated_lookups;    /* 1: the scan also reads the flag stream in full and skips the lookups of
                                 seeds that hold an unusable base (env DKB_GATE=0/1 overrides) */
+  uint64_t occupied_halves;  /* seed-record halves (one per seed and read orientation) with a designation */
+  uint64_t direct_halves;    /* of those, the ones whose windows the scan counts straight from the
+                                record, without the key table (DESIGN.md §4) */
 } dkb_stats;
 int dkb_stats_get(dkb_ctx *ctx, dkb_stats *out);
 int dkb_profile_counters(dkb_ctx *ctx, int enable);
