@@ -90,6 +90,13 @@ extern "C" {
                               n_reads: usize) -> c_int;
     pub fn dkb_batch_submit_multi(ctx: *mut DkbCtx, n_batches: c_int, bases2: *const *const u32,
                                   mask1: *const *const u32, n_positions: *const u64, samples: *const c_int) -> c_int;
+    pub fn dkb_batch_submit_sparse_multi(ctx: *mut DkbCtx, n_batches: c_int, bases2: *const *const u32,
+                                         zoff: *const *const u32, zbytes: *const *const u8,
+                                         zbytes_used: *const usize, n_positions: *const u64,
+                                         samples: *const c_int) -> c_int;
+    pub fn dkb_batch_submit_reads_multi(ctx: *mut DkbCtx, n_batches: c_int, seq: *const *const u8, seq_format: c_int,
+                                        qual: *const *const u8, offsets: *const *const u64, n_reads: *const usize,
+                                        min_baseq: c_int, samples: *const c_int) -> c_int;
     pub fn dkb_batch_set_loci_multi(ctx: *mut DkbCtx, n_batches: c_int, offsets: *const *const u64,
                                     lo: *const *const u64, hi: *const *const u64, n_reads: *const usize) -> c_int;
     pub fn dkb_sync(ctx: *mut DkbCtx) -> c_int;

@@ -81,6 +81,8 @@ pub fn run_trio(device: i32, k: i32, min_baseq: i32, thr: Thresholds, cands: &[C
                 let (seq, qual, off, _, _) = &bufs[i];
                 batches.push((p.next(seq, false, Some(qual.as_slice()), off)?, srcs[i].0 as i32));
             }
+            // the packers made zero lists of the flags, so this one launch also sends the smaller
+            // zero lists over PCIe (dkb_batch_submit_sparse_multi), as `submit` does below
             kc.submit_multi(&batches)?;
             in_flight += 1;
         }

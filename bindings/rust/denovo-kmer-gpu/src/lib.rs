@@ -186,12 +186,23 @@ impl Counter {
     /// launch: a trio step is one call.  Each batch must not be repacked before
     /// [`Counter::sync`], as for [`Counter::submit`] (one [`BatchPacker`] per sample keeps that
     /// rule when `sync` is called every second step).  Region mode: [`Counter::set_loci_multi`] first.
+    /// When every batch carries a zero list of its flags (as [`BatchPacker::next`] makes), the
+    /// zero lists cross PCIe instead of the dense flags, as in [`Counter::submit`].
     pub fn submit_multi(&mut self, batches: &[(&PinnedBatch, i32)]) -> Result<()> {
         let b: Vec<*const u32> = batches.iter().map(|(x, _)| x.bases2 as *const u32).collect();
-        let m: Vec<*const u32> = batches.iter().map(|(x, _)| x.mask1 as *const u32).collect();
         let n: Vec<u64> = batches.iter().map(|(x, _)| x.n_positions).collect();
         let s: Vec<c_int> = batches.iter().map(|(_, smp)| *smp).collect();
         let nb = c_int::try_from(batches.len()).unwrap_or(c_int::MAX);
+        if !batches.is_empty() && batches.iter().all(|(x, _)| x.zbytes_used != usize::MAX) {
+            let z: Vec<*const u32> = batches.iter().map(|(x, _)| x.zoff as *const u32).collect();
+            let zb: Vec<*const u8> = batches.iter().map(|(x, _)| x.zbytes as *const u8).collect();
+            let used: Vec<usize> = batches.iter().map(|(x, _)| x.zbytes_used).collect();
+            return self.ck(unsafe {
+                sys::dkb_batch_submit_sparse_multi(self.ctx, nb, b.as_ptr(), z.as_ptr(), zb.as_ptr(), used.as_ptr(),
+                                                   n.as_ptr(), s.as_ptr())
+            });
+        }
+        let m: Vec<*const u32> = batches.iter().map(|(x, _)| x.mask1 as *const u32).collect();
         self.ck(unsafe { sys::dkb_batch_submit_multi(self.ctx, nb, b.as_ptr(), m.as_ptr(), n.as_ptr(), s.as_ptr()) })
     }
 
@@ -202,6 +213,24 @@ impl Counter {
             sys::dkb_batch_submit_reads(self.ctx, seq.as_ptr(), four_bit as c_int,
                                         qual.map_or(ptr::null(), |q| q.as_ptr()), offsets.as_ptr(),
                                         offsets.len().saturating_sub(1), min_baseq, sample)
+        })
+    }
+
+    /// Kernel 0 + 2 on up to [`sys::DKB_MAX_MULTI`] batches of decoded reads,
+    /// `(seq, qual, offsets, sample)`, packed in one launch and scanned in ONE: one `four_bit` and
+    /// one `min_baseq` for all of them.  The buffers must stay unchanged until [`Counter::sync`].
+    /// Region mode: [`Counter::set_loci_multi`] first.
+    pub fn submit_reads_multi(&mut self, batches: &[(&[u8], Option<&[u8]>, &[u64], i32)], four_bit: bool,
+                              min_baseq: i32) -> Result<()> {
+        let seq: Vec<*const u8> = batches.iter().map(|b| b.0.as_ptr()).collect();
+        let qual: Vec<*const u8> = batches.iter().map(|b| b.1.map_or(ptr::null(), |q| q.as_ptr())).collect();
+        let off: Vec<*const u64> = batches.iter().map(|b| b.2.as_ptr()).collect();
+        let nr: Vec<usize> = batches.iter().map(|b| b.2.len().saturating_sub(1)).collect();
+        let s: Vec<c_int> = batches.iter().map(|b| b.3).collect();
+        let nb = c_int::try_from(batches.len()).unwrap_or(c_int::MAX);
+        self.ck(unsafe {
+            sys::dkb_batch_submit_reads_multi(self.ctx, nb, seq.as_ptr(), four_bit as c_int, qual.as_ptr(),
+                                              off.as_ptr(), nr.as_ptr(), min_baseq, s.as_ptr())
         })
     }
 

@@ -75,6 +75,12 @@ SYMBOLS = {
     "dkb_batch_set_loci": (C.c_int, [C.c_void_p, u64p, u64p, u64p, C.c_size_t]),
     "dkb_batch_submit_multi": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), u64p,
                                          C.POINTER(C.c_int)]),
+    "dkb_batch_submit_sparse_multi": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
+                                                C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), u64p,
+                                                C.POINTER(C.c_int)]),
+    "dkb_batch_submit_reads_multi": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p), C.c_int,
+                                               C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
+                                               C.POINTER(C.c_size_t), C.c_int, C.POINTER(C.c_int)]),
     "dkb_batch_set_loci_multi": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(u64p), C.POINTER(u64p), C.POINTER(u64p),
                                            C.POINTER(C.c_size_t)]),
     "dkb_sync": (C.c_int, [C.c_void_p]),

@@ -320,6 +320,45 @@ class KmerCounter:
         smp = (C.c_int * n)(*[int(x) for x in samples])
         self._ck(self._L.dkb_batch_submit_multi(self._h, n, b, m, npos, smp))
 
+    def submit_sparse_multi(self, batches, samples, loci=None):
+        """Up to 4 host batches with their flags as zero lists (mask_to_zero_list), expanded by
+        one launch and scanned by one: batches[i] = (bases2, zoff, zbytes, n_positions) goes into
+        the counters of samples[i].  loci: region mode, one ReadLoci per batch.  Buffers are kept
+        alive until sync()."""
+        n = len(batches)
+        if len(samples) != n:
+            raise ValueError("submit_sparse_multi: one sample per batch")
+        batches = [(np.ascontiguousarray(b, dtype=np.uint32), np.ascontiguousarray(z, dtype=np.uint32),
+                    np.ascontiguousarray(zb, dtype=np.uint8), int(npos)) for b, z, zb, npos in batches]
+        self._set_loci_multi(loci, n)
+        self._keep.append(batches)
+        ptrs = lambda j: (C.c_void_p * n)(*[x[j].ctypes.data for x in batches])  # noqa: E731
+        used = (C.c_size_t * n)(*[len(x[2]) for x in batches])
+        npos = (C.c_uint64 * n)(*[x[3] for x in batches])
+        smp = (C.c_int * n)(*[int(x) for x in samples])
+        self._ck(self._L.dkb_batch_submit_sparse_multi(self._h, n, ptrs(0), ptrs(1), ptrs(2), used, npos, smp))
+
+    def submit_reads_multi(self, reads, samples, min_baseq: int = DEFAULT_MIN_BASEQ, four_bit: bool = False,
+                           loci=None):
+        """Up to 4 batches of decoded reads (ASCII, or BAM 4-bit codes when four_bit) packed by
+        one launch and scanned by one: reads[i] = (seq, qual, offsets), qual may be None, goes
+        into the counters of samples[i].  loci: region mode, one ReadLoci per batch.  Buffers
+        are kept alive until sync()."""
+        n = len(reads)
+        if len(samples) != n:
+            raise ValueError("submit_reads_multi: one sample per batch")
+        reads = [(np.ascontiguousarray(s, dtype=np.uint8), None if q is None else np.ascontiguousarray(q, dtype=np.uint8),
+                  np.ascontiguousarray(o, dtype=np.uint64)) for s, q, o in reads]
+        self._set_loci_multi(loci, n)
+        self._keep.append(reads)
+        seq = (C.c_void_p * n)(*[x[0].ctypes.data for x in reads])
+        qual = (C.c_void_p * n)(*[None if x[1] is None else x[1].ctypes.data for x in reads])
+        offs = (C.c_void_p * n)(*[x[2].ctypes.data for x in reads])
+        nr = (C.c_size_t * n)(*[len(x[2]) - 1 for x in reads])
+        smp = (C.c_int * n)(*[int(x) for x in samples])
+        self._ck(self._L.dkb_batch_submit_reads_multi(self._h, n, seq, int(four_bit), qual, offs, nr, min_baseq,
+                                                      smp))
+
     def submit_device_multi(self, batches, loci=None):
         """batches: up to 4 tuples (d_bases2, d_mask1, n_positions, sample) of resident
         streams, scanned in ONE kernel launch (e.g. the three samples of a trio, or the four of

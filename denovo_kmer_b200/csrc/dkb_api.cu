@@ -38,6 +38,18 @@ struct DevBuf {
   }
 };
 
+// Page-locked host scratch and its capacity, in elements (grow_host).
+template <typename T>
+struct HostBuf {
+  T *p = nullptr;
+  size_t cap = 0;
+  void free() {
+    if (p) cudaFreeHost(p);
+    p = nullptr;
+    cap = 0;
+  }
+};
+
 struct dkb_ctx {
   int device = 0;
   int k = 0;
@@ -107,15 +119,18 @@ struct dkb_ctx {
   // host batches of every host submit form
   struct Stage : Slot {
     DevBuf<uint32_t> bases, mask;
-    // raw reads for the device-side packer (dkb_batch_submit_reads)
+    // raw reads for the device-side packer (dkb_batch_submit_reads and its multi form), each
+    // array the batches' concatenated; the 4-bit form's nibble starts are computed into
+    // nib_host and copied from there
     DevBuf<uint8_t> seq, qual;
     DevBuf<uint64_t> offsets, nib;
-    // zero list of dkb_batch_submit_sparse
+    HostBuf<uint64_t> nib_host;
+    // zero lists of dkb_batch_submit_sparse and its multi form, concatenated
     DevBuf<uint32_t> zoff;
     DevBuf<uint8_t> zbytes;
     void free() {
       bases.free(); mask.free();
-      seq.free(); qual.free(); offsets.free(); nib.free();
+      seq.free(); qual.free(); offsets.free(); nib.free(); nib_host.free();
       zoff.free(); zbytes.free();
       Slot::free();
     }
@@ -569,33 +584,220 @@ int release(dkb_ctx *ctx, std::initializer_list<dkb_ctx::Slot *> slots) {
   return DKB_OK;
 }
 
-// Copy n host-resident batches into one staging buffer, each at a 16-byte-aligned offset.
-// d_bases / d_mask get the batches' device addresses.
-int stage_batches(dkb_ctx *ctx, const Batches &b, const uint32_t *const *bases2, const uint32_t *const *mask1,
-                  const uint32_t **d_bases, const uint32_t **d_mask, dkb_ctx::Stage *&out) {
-  const uint64_t *n_positions = b.n_positions;
+// Grow a slot's page-locked host scratch to at least `need` elements.  The caller has waited
+// for the slot's last copies (its `copied` event): they may still read the old scratch.
+template <typename T>
+int grow_host(dkb_ctx *ctx, HostBuf<T> &b, size_t need) {
+  if (b.cap >= need) return DKB_OK;
+  b.free();
+  const size_t want = need + need / 8 + 256;
+  T *q = nullptr;
+  CU(cudaMallocHost(&q, want * sizeof(T)));
+  b.p = q;
+  b.cap = want;
+  return DKB_OK;
+}
+
+// Where a submit's packed streams go in a staging slot: batch i's at bases.p + bo[i] and
+// mask.p + mo[i], each at a 16-byte-aligned offset; bw / mw words in all.
+struct StreamLayout {
   size_t bo[DKB_MAX_MULTI], mo[DKB_MAX_MULTI], bw = 0, mw = 0;
-  for (int i = 0; i < b.n; i++) {
-    bo[i] = bw;
-    mo[i] = mw;
-    bw += (dkb_stream_bases_words(n_positions[i]) + 3) / 4 * 4;
-    mw += (dkb_stream_mask_words(n_positions[i]) + 3) / 4 * 4;
+  explicit StreamLayout(const Batches &b) {
+    for (int i = 0; i < b.n; i++) {
+      bo[i] = bw;
+      mo[i] = mw;
+      bw += (dkb_stream_bases_words(b.n_positions[i]) + 3) / 4 * 4;
+      mw += (dkb_stream_mask_words(b.n_positions[i]) + 3) / 4 * 4;
+    }
   }
-  return stage_slot(ctx, ctx->stage, out, [&](dkb_ctx::Stage &st) -> int {
+  // grow the slot's stream buffers to hold the layout
+  int grow_slot(dkb_ctx *ctx, dkb_ctx::Stage &st) const {
     int rc;
     if ((rc = grow(ctx, st, st.bases, bw)) != DKB_OK) return rc;
-    if ((rc = grow(ctx, st, st.mask, mw)) != DKB_OK) return rc;
+    return grow(ctx, st, st.mask, mw);
+  }
+  // the batches' device addresses, for launch_scan
+  void place(const Batches &b, const dkb_ctx::Stage &st, const uint32_t **d_bases, const uint32_t **d_mask) const {
     for (int i = 0; i < b.n; i++) {
       d_bases[i] = st.bases.p + bo[i];
       d_mask[i] = st.mask.p + mo[i];
+    }
+  }
+};
+
+// Copy n host-resident batches into one staging buffer (StreamLayout).  d_bases / d_mask get
+// the batches' device addresses.
+int stage_batches(dkb_ctx *ctx, const Batches &b, const uint32_t *const *bases2, const uint32_t *const *mask1,
+                  const uint32_t **d_bases, const uint32_t **d_mask, dkb_ctx::Stage *&out) {
+  const uint64_t *n_positions = b.n_positions;
+  const StreamLayout L(b);
+  return stage_slot(ctx, ctx->stage, out, [&](dkb_ctx::Stage &st) -> int {
+    int rc;
+    if ((rc = L.grow_slot(ctx, st)) != DKB_OK) return rc;
+    L.place(b, st, d_bases, d_mask);
+    for (int i = 0; i < b.n; i++) {
       if (n_positions[i] == 0) continue;
-      CU(cudaMemcpyAsync(st.bases.p + bo[i], bases2[i], dkb_stream_bases_words(n_positions[i]) * 4,
+      CU(cudaMemcpyAsync(st.bases.p + L.bo[i], bases2[i], dkb_stream_bases_words(n_positions[i]) * 4,
                          cudaMemcpyHostToDevice, ctx->s_copy));
-      CU(cudaMemcpyAsync(st.mask.p + mo[i], mask1[i], dkb_stream_mask_words(n_positions[i]) * 4,
+      CU(cudaMemcpyAsync(st.mask.p + L.mo[i], mask1[i], dkb_stream_mask_words(n_positions[i]) * 4,
                          cudaMemcpyHostToDevice, ctx->s_copy));
     }
     return DKB_OK;
   });
+}
+
+// "batch i: " in front of a refusal that concerns one batch of a multi-batch submit
+std::string batch_prefix(const Batches &b, int i) {
+  return b.multi ? "batch " + std::to_string(i) + ": " : std::string();
+}
+
+// Host batches with their flags as zero lists: the bases and the zero lists are copied into
+// one staging slot, concatenated, and ONE k_expand_zero_list launch writes every batch's flags
+// into the slot's stream buffer (StreamLayout) ahead of the scan.
+int stage_sparse(dkb_ctx *ctx, const Batches &b, const uint32_t *const *bases2, const uint32_t *const *zoff,
+                 const uint8_t *const *zbytes, const size_t *zbytes_used, const uint32_t **d_bases,
+                 const uint32_t **d_mask, dkb_ctx::Stage *&slot) {
+  // the zero lists are checked here, once the batches' lengths are: their sizes follow from n_positions
+  size_t nb[DKB_MAX_MULTI], zo[DKB_MAX_MULTI], zbo[DKB_MAX_MULTI], n_zoff = 0, n_zbytes = 0;
+  for (int i = 0; i < b.n; i++) {
+    nb[i] = dkb_zero_list_blocks(b.n_positions[i]);
+    zo[i] = n_zoff;
+    zbo[i] = n_zbytes;
+    if (b.n_positions[i] == 0) continue;
+    const uint32_t *z = zoff[i];
+    if ((z[nb[i]] & 0x7FFFFFFFu) != zbytes_used[i])
+      return fail(ctx, DKB_EINVAL, batch_prefix(b, i) + "zoff[n_blocks] != zbytes_used");
+    // the expander trusts the offsets: they must ascend inside zbytes, a plain-bits block is 256 bytes
+    for (size_t j = 0; j < nb[i]; j++) {
+      const uint32_t cur = z[j] & 0x7FFFFFFFu, nxt = z[j + 1] & 0x7FFFFFFFu;
+      if (nxt < cur || nxt > zbytes_used[i] || ((z[j] & 0x80000000u) && nxt - cur != 256u))
+        return fail(ctx, DKB_EINVAL, batch_prefix(b, i) + "malformed zero list (block offsets)");
+    }
+    n_zoff += nb[i] + 1;
+    n_zbytes += zbytes_used[i];
+  }
+  const StreamLayout L(b);
+  int rc = stage_slot(ctx, ctx->stage, slot, [&](dkb_ctx::Stage &st) -> int {
+    int rc;
+    if ((rc = L.grow_slot(ctx, st)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st, st.zoff, n_zoff)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st, st.zbytes, n_zbytes ? n_zbytes : 1)) != DKB_OK) return rc;
+    for (int i = 0; i < b.n; i++) {
+      if (b.n_positions[i] == 0) continue;
+      CU(cudaMemcpyAsync(st.bases.p + L.bo[i], bases2[i], dkb_stream_bases_words(b.n_positions[i]) * 4,
+                         cudaMemcpyHostToDevice, ctx->s_copy));
+      CU(cudaMemcpyAsync(st.zoff.p + zo[i], zoff[i], (nb[i] + 1) * 4, cudaMemcpyHostToDevice, ctx->s_copy));
+      if (zbytes_used[i])
+        CU(cudaMemcpyAsync(st.zbytes.p + zbo[i], zbytes[i], zbytes_used[i], cudaMemcpyHostToDevice, ctx->s_copy));
+    }
+    return DKB_OK;
+  });
+  if (rc != DKB_OK) return rc;
+  ZeroListParams Z;
+  memset(&Z, 0, sizeof(Z));
+  for (int i = 0; i < b.n; i++) {
+    if (b.n_positions[i] == 0) continue;
+    ZeroListSegment &S = Z.seg[Z.n_seg++];
+    S.zoff = slot->zoff.p + zo[i];
+    S.zbytes = slot->zbytes.p + zbo[i];
+    S.mask1 = slot->mask.p + L.mo[i];
+    S.b_begin = Z.n_blocks;
+    S.n_blocks = (uint32_t)nb[i];
+    S.n_mwords = (uint32_t)dkb_stream_mask_words(b.n_positions[i]);
+    Z.n_blocks += (uint32_t)nb[i];
+  }
+  k_expand_zero_list<<<(Z.n_blocks + 7) / 8, 256, 0, ctx->s_scan>>>(Z);
+  CU(cudaGetLastError());
+  L.place(b, *slot, d_bases, d_mask);
+  return DKB_OK;
+}
+
+// Host batches of decoded reads: their bases, qualities and offsets are copied into one staging
+// slot, concatenated, and ONE k_pack launch packs every batch into the slot's stream buffer
+// (StreamLayout) ahead of the scan.  seq[i] points at batch i's first 4-bit byte (seq_format 1)
+// or at the base its offsets count from (0); qual (may be null) and qual[i] (may be null) alike.
+int stage_reads(dkb_ctx *ctx, const Batches &b, const uint8_t *const *seq, int seq_format,
+                const uint8_t *const *qual, const uint64_t *const *offsets, const size_t *n_reads,
+                int min_baseq, const uint32_t **d_bases, const uint32_t **d_mask, dkb_ctx::Stage *&slot) {
+  const bool four_bit = seq_format == 1;
+  // per batch with positions: its bases and where its seq / qual / offsets / nibble starts go
+  uint64_t n_bases[DKB_MAX_MULTI], seq_bytes[DKB_MAX_MULTI];
+  size_t so[DKB_MAX_MULTI], qo[DKB_MAX_MULTI], oo[DKB_MAX_MULTI], no[DKB_MAX_MULTI];
+  size_t n_seq = 0, n_qual = 0, n_off = 0, n_nib = 0;
+  for (int i = 0; i < b.n; i++) {
+    so[i] = n_seq; qo[i] = n_qual; oo[i] = n_off; no[i] = n_nib;
+    if (b.n_positions[i] == 0) continue;
+    n_bases[i] = offsets[i][n_reads[i]] - offsets[i][0];
+    seq_bytes[i] = n_bases[i];
+    if (four_bit) {  // BAM keeps every read's 4-bit codes byte-aligned: (len + 1) / 2 bytes per read
+      seq_bytes[i] = 0;
+      for (size_t r = 0; r < n_reads[i]; r++) seq_bytes[i] += (offsets[i][r + 1] - offsets[i][r] + 1) / 2;
+      n_nib += n_reads[i];
+    }
+    n_seq += seq_bytes[i];
+    if (qual && qual[i]) n_qual += n_bases[i];
+    n_off += n_reads[i] + 1;
+  }
+  const StreamLayout L(b);
+  int rc = stage_slot(ctx, ctx->stage, slot, [&](dkb_ctx::Stage &st) -> int {
+    int rc;
+    if ((rc = L.grow_slot(ctx, st)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st, st.seq, n_seq ? n_seq : 1)) != DKB_OK) return rc;
+    if (n_qual && (rc = grow(ctx, st, st.qual, n_qual)) != DKB_OK) return rc;
+    if ((rc = grow(ctx, st, st.offsets, n_off)) != DKB_OK) return rc;
+    if (four_bit) {
+      if ((rc = grow(ctx, st, st.nib, n_nib)) != DKB_OK) return rc;
+      // the nibble starts go through the slot's page-locked scratch, which the slot's last
+      // copies may still read: wait for those copies (not for any scan) before rewriting it
+      CU(cudaEventSynchronize(st.copied));
+      if ((rc = grow_host(ctx, st.nib_host, n_nib)) != DKB_OK) return rc;
+    }
+    for (int i = 0; i < b.n; i++) {
+      if (b.n_positions[i] == 0) continue;
+      const uint64_t *off = offsets[i];
+      // the reads of a batch start at off[0] in the caller's arrays; device copies start at the batch's segment
+      CU(cudaMemcpyAsync(st.seq.p + so[i], four_bit ? seq[i] : seq[i] + off[0], seq_bytes[i], cudaMemcpyHostToDevice,
+                         ctx->s_copy));
+      if (qual && qual[i])
+        CU(cudaMemcpyAsync(st.qual.p + qo[i], qual[i] + off[0], n_bases[i], cudaMemcpyHostToDevice, ctx->s_copy));
+      CU(cudaMemcpyAsync(st.offsets.p + oo[i], off, (n_reads[i] + 1) * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+      if (four_bit) {
+        uint64_t *nib = st.nib_host.p + no[i], bytes = 0;
+        for (size_t r = 0; r < n_reads[i]; r++) {
+          nib[r] = bytes;
+          bytes += (off[r + 1] - off[r] + 1) / 2;
+        }
+        CU(cudaMemcpyAsync(st.nib.p + no[i], nib, n_reads[i] * 8, cudaMemcpyHostToDevice, ctx->s_copy));
+      }
+    }
+    return DKB_OK;
+  });
+  if (rc != DKB_OK) return rc;
+  PackParams Q;
+  memset(&Q, 0, sizeof(Q));
+  for (int i = 0; i < b.n; i++) {
+    if (b.n_positions[i] == 0) continue;
+    PackSegment &S = Q.seg[Q.n_seg++];
+    S.seq = slot->seq.p + so[i];
+    S.qual = qual && qual[i] ? slot->qual.p + qo[i] : nullptr;
+    S.offsets = slot->offsets.p + oo[i];
+    S.nib_start = four_bit ? slot->nib.p + no[i] : nullptr;
+    S.bases2 = slot->bases.p + L.bo[i];
+    S.mask1 = slot->mask.p + L.mo[i];
+    S.m_begin = Q.n_mwords;
+    S.n_pos = b.n_positions[i];
+    S.n_reads = (uint32_t)n_reads[i];
+    S.n_bwords = (uint32_t)dkb_stream_bases_words(b.n_positions[i]);
+    S.n_mwords = (uint32_t)dkb_stream_mask_words(b.n_positions[i]);
+    Q.n_mwords += S.n_mwords;
+  }
+  Q.min_baseq = min_baseq;
+  Q.four_bit = seq_format;
+  const int TB = 256;
+  k_pack<<<(uint32_t)((Q.n_mwords + TB - 1) / TB), TB, 0, ctx->s_scan>>>(Q);
+  CU(cudaGetLastError());
+  L.place(b, *slot, d_bases, d_mask);
+  return DKB_OK;
 }
 
 const char *const NO_PROF_REGIONS = "region mode has no scan kernel with profiling counters (dkb_profile_counters 0)";
@@ -624,8 +826,7 @@ int check_loci_positions(dkb_ctx *ctx, const Batches &b, const dkb_ctx::Loci *l,
                                      std::to_string(b.n));
   for (int i = 0; i < n; i++)
     if (l[i].n_pos != b.n_positions[i])
-      return fail(ctx, DKB_EINVAL, (b.multi ? "batch " + std::to_string(i) + ": " : std::string()) +
-                                       "the loci's reads cover " + std::to_string(l[i].n_pos) +
+      return fail(ctx, DKB_EINVAL, batch_prefix(b, i) + "the loci's reads cover " + std::to_string(l[i].n_pos) +
                                        " stream positions, the batch " + std::to_string(b.n_positions[i]));
   return DKB_OK;
 }
@@ -841,6 +1042,38 @@ int check_streams(dkb_ctx *ctx, const Batches &b, const uint32_t *const *bases2,
     if (!bases2[i] || !mask1[i]) return fail(ctx, DKB_EINVAL, "null stream pointer");
     if (device && ((uintptr_t)bases2[i] & 15)) return fail(ctx, DKB_EINVAL, "d_bases2 must be 16-byte aligned");
     if (device && ((uintptr_t)mask1[i] & 3)) return fail(ctx, DKB_EINVAL, "d_mask1 must be 4-byte aligned");
+  }
+  return DKB_OK;
+}
+
+// The checks of the zero-list forms (dkb_batch_submit_sparse and its multi form); the zero
+// lists themselves are checked by stage_sparse.
+int check_sparse(dkb_ctx *ctx, const Batches &b, const uint32_t *const *bases2, const uint32_t *const *zoff,
+                 const uint8_t *const *zbytes, const size_t *zbytes_used) {
+  if (b.multi && (b.n < 0 || b.n > DKB_MAX_MULTI)) return fail(ctx, DKB_EINVAL, "n_batches out of range");
+  if (b.multi && b.n && (!bases2 || !zoff || !zbytes || !zbytes_used || !b.n_positions || !b.samples))
+    return fail(ctx, DKB_EINVAL, "null argument");
+  for (int i = 0; i < b.n; i++)
+    if (b.n_positions[i] && (!bases2[i] || !zoff[i] || (zbytes_used[i] && !zbytes[i])))
+      return fail(ctx, DKB_EINVAL, batch_prefix(b, i) + "null stream pointer");
+  return DKB_OK;
+}
+
+// The checks of the decoded-read forms (dkb_batch_submit_reads and its multi form).  Sets each
+// batch's stream positions, n_pos[i] (0 for a batch without reads).
+int check_reads(dkb_ctx *ctx, const Batches &b, const uint8_t *const *seq, int seq_format,
+                const uint64_t *const *offsets, const size_t *n_reads, uint64_t *n_pos) {
+  if (b.multi && (b.n < 0 || b.n > DKB_MAX_MULTI)) return fail(ctx, DKB_EINVAL, "n_batches out of range");
+  if (seq_format != 0 && seq_format != 1) return fail(ctx, DKB_EINVAL, "seq_format must be 0 (ASCII) or 1 (BAM 4-bit)");
+  if (b.multi && b.n && (!seq || !offsets || !n_reads || !b.samples)) return fail(ctx, DKB_EINVAL, "null argument");
+  for (int i = 0; i < b.n; i++) {
+    if (n_reads[i] == 0) continue;
+    if (!seq[i] || !offsets[i]) return fail(ctx, DKB_EINVAL, batch_prefix(b, i) + "null read buffer");
+    if (n_reads[i] >= 0xFFFFFFFFull) return fail(ctx, DKB_EINVAL, batch_prefix(b, i) + "too many reads in one batch");
+    for (size_t r = 0; r < n_reads[i]; r++)
+      if (offsets[i][r + 1] < offsets[i][r])
+        return fail(ctx, DKB_EINVAL, batch_prefix(b, i) + "offsets must not decrease");
+    n_pos[i] = dkb_stream_positions(offsets[i], n_reads[i]);
   }
   return DKB_OK;
 }
@@ -1225,42 +1458,21 @@ int dkb_batch_submit_sparse(dkb_ctx *ctx, const uint32_t *bases2, const uint32_t
                             const uint8_t *zbytes, size_t zbytes_used, uint64_t n_positions, int sample) {
   const uint32_t *d_bases, *d_mask;
   const Batches b{false, 1, &n_positions, &sample, &d_bases, &d_mask};
-  auto check = [&]() -> int {
-    if (n_positions && (!bases2 || !zoff || (zbytes_used && !zbytes)))
-      return fail(ctx, DKB_EINVAL, "null stream pointer");
-    return DKB_OK;
-  };
-  return submit(ctx, b, check, [&](dkb_ctx::Stage *&slot) -> int {
-    // the zero list is checked here, once the batch's length is: its size follows from n_positions
-    const size_t nb = dkb_zero_list_blocks(n_positions);
-    if ((zoff[nb] & 0x7FFFFFFFu) != zbytes_used) return fail(ctx, DKB_EINVAL, "zoff[n_blocks] != zbytes_used");
-    // the expander trusts the offsets: they must ascend inside zbytes, a plain-bits block is 256 bytes
-    for (size_t i = 0; i < nb; i++) {
-      const uint32_t cur = zoff[i] & 0x7FFFFFFFu, nxt = zoff[i + 1] & 0x7FFFFFFFu;
-      if (nxt < cur || nxt > zbytes_used || ((zoff[i] & 0x80000000u) && nxt - cur != 256u))
-        return fail(ctx, DKB_EINVAL, "malformed zero list (block offsets)");
-    }
-    const size_t bw = dkb_stream_bases_words(n_positions), mw = dkb_stream_mask_words(n_positions);
-    const size_t zb1 = zbytes_used ? zbytes_used : 1;
-    int rc = stage_slot(ctx, ctx->stage, slot, [&](dkb_ctx::Stage &st) -> int {
-      int rc;
-      if ((rc = grow(ctx, st, st.bases, bw)) != DKB_OK) return rc;
-      if ((rc = grow(ctx, st, st.mask, mw)) != DKB_OK) return rc;
-      if ((rc = grow(ctx, st, st.zoff, nb + 1)) != DKB_OK) return rc;
-      if ((rc = grow(ctx, st, st.zbytes, zb1)) != DKB_OK) return rc;
-      CU(cudaMemcpyAsync(st.bases.p, bases2, bw * 4, cudaMemcpyHostToDevice, ctx->s_copy));
-      CU(cudaMemcpyAsync(st.zoff.p, zoff, (nb + 1) * 4, cudaMemcpyHostToDevice, ctx->s_copy));
-      if (zbytes_used) CU(cudaMemcpyAsync(st.zbytes.p, zbytes, zbytes_used, cudaMemcpyHostToDevice, ctx->s_copy));
-      return DKB_OK;
-    });
-    if (rc != DKB_OK) return rc;
-    k_expand_zero_list<<<(uint32_t)((nb + 7) / 8), 256, 0, ctx->s_scan>>>(slot->zoff.p, slot->zbytes.p, (uint32_t)nb,
-                                                                        (uint32_t)mw, slot->mask.p);
-    CU(cudaGetLastError());
-    d_bases = slot->bases.p;
-    d_mask = slot->mask.p;
-    return DKB_OK;
-  });
+  return submit(ctx, b, [&]() -> int { return check_sparse(ctx, b, &bases2, &zoff, &zbytes, &zbytes_used); },
+                [&](dkb_ctx::Stage *&st) {
+                  return stage_sparse(ctx, b, &bases2, &zoff, &zbytes, &zbytes_used, &d_bases, &d_mask, st);
+                });
+}
+
+int dkb_batch_submit_sparse_multi(dkb_ctx *ctx, int n_batches, const uint32_t *const *bases2,
+                                  const uint32_t *const *zoff, const uint8_t *const *zbytes,
+                                  const size_t *zbytes_used, const uint64_t *n_positions, const int *samples) {
+  const uint32_t *d_bases[DKB_MAX_MULTI], *d_mask[DKB_MAX_MULTI];
+  const Batches b{true, n_batches, n_positions, samples, d_bases, d_mask};
+  return submit(ctx, b, [&]() -> int { return check_sparse(ctx, b, bases2, zoff, zbytes, zbytes_used); },
+                [&](dkb_ctx::Stage *&st) {
+                  return stage_sparse(ctx, b, bases2, zoff, zbytes, zbytes_used, d_bases, d_mask, st);
+                });
 }
 
 int dkb_batch_submit_reads(dkb_ctx *ctx, const uint8_t *seq, int seq_format, const uint8_t *qual,
@@ -1268,71 +1480,23 @@ int dkb_batch_submit_reads(dkb_ctx *ctx, const uint8_t *seq, int seq_format, con
   uint64_t n_pos = 0;  // known once the offsets are checked
   const uint32_t *d_bases, *d_mask;
   const Batches b{false, 1, &n_pos, &sample, &d_bases, &d_mask};
-  auto check = [&]() -> int {
-    if (seq_format != 0 && seq_format != 1) return fail(ctx, DKB_EINVAL, "seq_format must be 0 (ASCII) or 1 (BAM 4-bit)");
-    if (n_reads == 0) return DKB_OK;
-    if (!seq || !offsets) return fail(ctx, DKB_EINVAL, "null read buffer");
-    if (n_reads >= 0xFFFFFFFFull) return fail(ctx, DKB_EINVAL, "too many reads in one batch");
-    for (size_t r = 0; r < n_reads; r++)
-      if (offsets[r + 1] < offsets[r]) return fail(ctx, DKB_EINVAL, "offsets must not decrease");
-    n_pos = dkb_stream_positions(offsets, n_reads);
-    return DKB_OK;
-  };
-  return submit(ctx, b, check, [&](dkb_ctx::Stage *&slot) -> int {
-    const uint64_t n_bases = offsets[n_reads] - offsets[0];
-    const size_t bw = dkb_stream_bases_words(n_pos), mw = dkb_stream_mask_words(n_pos);
-    // BAM keeps every read's 4-bit codes byte-aligned: (len + 1) / 2 bytes per read
-    std::vector<uint64_t> nib;
-    uint64_t seq_bytes = n_bases;
-    if (seq_format == 1) {
-      nib.resize(n_reads);
-      uint64_t bytes = 0;
-      for (size_t r = 0; r < n_reads; r++) {
-        nib[r] = bytes;
-        bytes += (offsets[r + 1] - offsets[r] + 1) / 2;
-      }
-      seq_bytes = bytes;
-    }
-    int rc = stage_slot(ctx, ctx->stage, slot, [&](dkb_ctx::Stage &st) -> int {
-      int rc;
-      if ((rc = grow(ctx, st, st.bases, bw)) != DKB_OK) return rc;
-      if ((rc = grow(ctx, st, st.mask, mw)) != DKB_OK) return rc;
-      if ((rc = grow(ctx, st, st.seq, (size_t)seq_bytes)) != DKB_OK) return rc;
-      if (qual && (rc = grow(ctx, st, st.qual, (size_t)n_bases)) != DKB_OK) return rc;
-      if ((rc = grow(ctx, st, st.offsets, n_reads + 1)) != DKB_OK) return rc;
-      if (seq_format == 1 && (rc = grow(ctx, st, st.nib, n_reads)) != DKB_OK) return rc;
-      // the reads of this batch start at offsets[0] in the caller's arrays; device copies start at 0
-      const uint8_t *seq0 = seq_format == 1 ? seq : seq + offsets[0];
-      CU(cudaMemcpyAsync(st.seq.p, seq0, seq_bytes, cudaMemcpyHostToDevice, ctx->s_copy));
-      if (qual) CU(cudaMemcpyAsync(st.qual.p, qual + offsets[0], n_bases, cudaMemcpyHostToDevice, ctx->s_copy));
-      CU(cudaMemcpyAsync(st.offsets.p, offsets, (n_reads + 1) * 8, cudaMemcpyHostToDevice, ctx->s_copy));
-      if (seq_format == 1) {
-        CU(cudaMemcpyAsync(st.nib.p, nib.data(), n_reads * 8, cudaMemcpyHostToDevice, ctx->s_copy));
-        CU(cudaStreamSynchronize(ctx->s_copy));  // nib is a local vector
-      }
-      return DKB_OK;
-    });
-    if (rc != DKB_OK) return rc;
-    PackParams Q;
-    Q.seq = slot->seq.p;
-    Q.qual = qual ? slot->qual.p : nullptr;
-    Q.offsets = slot->offsets.p;
-    Q.nib_start = slot->nib.p;
-    Q.n_reads = (uint32_t)n_reads;
-    Q.n_pos = n_pos;
-    Q.n_bwords = (uint32_t)bw;
-    Q.n_mwords = (uint32_t)mw;
-    Q.min_baseq = min_baseq;
-    Q.four_bit = seq_format;
-    Q.bases2 = slot->bases.p;
-    Q.mask1 = slot->mask.p;
-    const int TB = 256;
-    k_pack<<<(uint32_t)((mw + TB - 1) / TB), TB, 0, ctx->s_scan>>>(Q);
-    CU(cudaGetLastError());
-    d_bases = slot->bases.p;
-    d_mask = slot->mask.p;
-    return DKB_OK;
-  });
+  return submit(ctx, b, [&]() -> int { return check_reads(ctx, b, &seq, seq_format, &offsets, &n_reads, &n_pos); },
+                [&](dkb_ctx::Stage *&st) {
+                  return stage_reads(ctx, b, &seq, seq_format, &qual, &offsets, &n_reads, min_baseq, &d_bases,
+                                     &d_mask, st);
+                });
+}
+
+int dkb_batch_submit_reads_multi(dkb_ctx *ctx, int n_batches, const uint8_t *const *seq, int seq_format,
+                                 const uint8_t *const *qual, const uint64_t *const *offsets,
+                                 const size_t *n_reads, int min_baseq, const int *samples) {
+  uint64_t n_pos[DKB_MAX_MULTI] = {};  // known once the offsets are checked
+  const uint32_t *d_bases[DKB_MAX_MULTI], *d_mask[DKB_MAX_MULTI];
+  const Batches b{true, n_batches, n_pos, samples, d_bases, d_mask};
+  return submit(ctx, b, [&]() -> int { return check_reads(ctx, b, seq, seq_format, offsets, n_reads, n_pos); },
+                [&](dkb_ctx::Stage *&st) {
+                  return stage_reads(ctx, b, seq, seq_format, qual, offsets, n_reads, min_baseq, d_bases, d_mask, st);
+                });
 }
 
 int dkb_table_set_regions(dkb_ctx *ctx, const uint64_t *lo, const uint64_t *hi, uint32_t n_variants) {

@@ -222,6 +222,25 @@ int dkb_batch_submit_device_multi(dkb_ctx *ctx, int n_batches, const uint32_t *c
  * first. */
 int dkb_batch_submit_multi(dkb_ctx *ctx, int n_batches, const uint32_t *const *bases2,
                            const uint32_t *const *mask1, const uint64_t *n_positions, const int *samples);
+/* dkb_batch_submit_sparse for up to DKB_MAX_MULTI host-resident batches: batch i is bases2[i]
+ * with its flags as the zero list zoff[i] / zbytes[i] / zbytes_used[i], n_positions[i] long, into
+ * the counters of samples[i].  Every zero list is checked as dkb_batch_submit_sparse checks it;
+ * one launch expands them all, then one scan launch counts them.  The call follows the rules of
+ * dkb_batch_submit_multi (n_batches in [0, DKB_MAX_MULTI], empty batches skipped, buffers valid
+ * until dkb_sync, the loci of dkb_batch_set_loci_multi in region mode).  A refusal that concerns
+ * one batch names it ("batch i: ..."). */
+int dkb_batch_submit_sparse_multi(dkb_ctx *ctx, int n_batches, const uint32_t *const *bases2,
+                                  const uint32_t *const *zoff, const uint8_t *const *zbytes,
+                                  const size_t *zbytes_used, const uint64_t *n_positions, const int *samples);
+/* dkb_batch_submit_reads for up to DKB_MAX_MULTI batches of decoded reads: batch i is
+ * seq[i] / qual[i] / offsets[i] with n_reads[i] reads, into the counters of samples[i], each under
+ * the rules of dkb_batch_submit_reads.  One seq_format and one min_baseq apply to every batch.
+ * qual may be NULL (no batch has qualities), and so may any qual[i].  One launch packs every
+ * batch, then one scan launch counts them.  The call follows the rules of dkb_batch_submit_multi;
+ * a batch of 0 reads is skipped.  A refusal that concerns one batch names it ("batch i: ..."). */
+int dkb_batch_submit_reads_multi(dkb_ctx *ctx, int n_batches, const uint8_t *const *seq, int seq_format,
+                                 const uint8_t *const *qual, const uint64_t *const *offsets,
+                                 const size_t *n_reads, int min_baseq, const int *samples);
 
 /* ---- region-scoped counting (opt-in; DESIGN.md §2) ---------------------------- */
 /* In region mode an occurrence of entry e's key in read r counts iff the read's alignment
@@ -247,8 +266,8 @@ int dkb_table_set_regions(dkb_ctx *ctx, const uint64_t *lo, const uint64_t *hi, 
  * on, a submit returns DKB_ESTATE. */
 int dkb_batch_set_loci(dkb_ctx *ctx, const uint64_t *offsets, const uint64_t *lo,
                        const uint64_t *hi, size_t n_reads);
-/* Region mode: the read loci of the NEXT multi-batch submit (dkb_batch_submit_multi or
- * dkb_batch_submit_device_multi), one set per batch, with the same meaning and validity rules
+/* Region mode: the read loci of the NEXT multi-batch submit (dkb_batch_submit_multi,
+ * _device_multi, _sparse_multi or _reads_multi), one set per batch, with the same meaning and validity rules
  * as dkb_batch_set_loci.  DKB_ESTATE in whole-stream mode; DKB_EINVAL for n_batches outside
  * [0, DKB_MAX_MULTI], descending offsets in any batch, n_reads[i] >= 2^32, or 2^32 or more
  * reads in all.  The submit returns DKB_EINVAL unless its n_batches equals these loci's and

@@ -195,6 +195,50 @@ class Counter {
     }
     check(dkb_batch_submit_multi(ctx_, (int)batches.size(), b.data(), m.data(), n.data(), smp.data()), ctx_);
   }
+  // Up to DKB_MAX_MULTI zero-list streams, (stream, sample), in one expand and ONE scan launch;
+  // the streams must outlive the next sync()
+  void submit_sparse_multi(const std::vector<std::pair<const SparseStream *, int>> &batches) {
+    std::vector<const uint32_t *> b, z;
+    std::vector<const uint8_t *> zb;
+    std::vector<size_t> used;
+    std::vector<uint64_t> n;
+    std::vector<int> smp;
+    for (const auto &x : batches) {
+      b.push_back(x.first->bases2.data());
+      z.push_back(x.first->zoff.data());
+      zb.push_back(x.first->zbytes.data());
+      used.push_back(x.first->zbytes.size());
+      n.push_back(x.first->n_positions);
+      smp.push_back(x.second);
+    }
+    check(dkb_batch_submit_sparse_multi(ctx_, (int)batches.size(), b.data(), z.data(), zb.data(), used.data(),
+                                        n.data(), smp.data()),
+          ctx_);
+  }
+  // One batch of decoded reads for submit_reads_multi (as in submit_reads; qual may be empty)
+  struct ReadsRef {
+    const std::vector<uint8_t> *seq, *qual;
+    const std::vector<uint64_t> *offsets;
+    int sample;
+  };
+  // Up to DKB_MAX_MULTI batches of decoded reads in one pack and ONE scan launch; the vectors
+  // must outlive the next sync()
+  void submit_reads_multi(const std::vector<ReadsRef> &batches, int min_baseq, bool four_bit = false) {
+    std::vector<const uint8_t *> s, q;
+    std::vector<const uint64_t *> o;
+    std::vector<size_t> nr;
+    std::vector<int> smp;
+    for (const ReadsRef &x : batches) {
+      s.push_back(x.seq->data());
+      q.push_back(x.qual->empty() ? nullptr : x.qual->data());
+      o.push_back(x.offsets->data());
+      nr.push_back(x.offsets->empty() ? 0 : x.offsets->size() - 1);
+      smp.push_back(x.sample);
+    }
+    check(dkb_batch_submit_reads_multi(ctx_, (int)batches.size(), s.data(), four_bit ? 1 : 0, q.data(), o.data(),
+                                       nr.data(), min_baseq, smp.data()),
+          ctx_);
+  }
   void sync() { check(dkb_sync(ctx_), ctx_); }
   void reset_counts() { check(dkb_counts_reset(ctx_), ctx_); }
   int n_children() const { return n_children_; }

@@ -13,7 +13,17 @@ Windows are +-500 bases around each candidate.  Arms, each a pair (single, multi
   rg_host       region mode, host memory: the same with loci
   rg_device     region mode, device-resident: three dkb_batch_submit_device vs one
                 dkb_batch_submit_device_multi
-Host streams are in pinned memory.  A step is one batch per sample; its time is a host clock from
+  ws_sparse / rg_sparse    the flags as zero lists: three dkb_batch_submit_sparse vs one
+                dkb_batch_submit_sparse_multi, whole stream / region mode
+  ws_reads / rg_reads      decoded ASCII reads packed on the GPU: three dkb_batch_submit_reads vs
+                one dkb_batch_submit_reads_multi (fetch workload only: the device generator
+                makes packed streams, not reads)
+  ws_reads4 / rg_reads4    the same from BAM 4-bit codes
+  dense_sparse  one dkb_batch_submit_multi ("single") vs one dkb_batch_submit_sparse_multi
+                ("multi"): the dense flags against the zero lists in one launch
+Every arm reports the bytes per base its multi form copies over PCIe.  Counters are compared
+within each pair, and across all arms of one counting mode (whole stream, region).
+Host buffers are in pinned memory.  A step is one batch per sample; its time is a host clock from
 the first submit to dkb_sync, so it includes copies, locus-index builds and launches.  Every
 arm runs --warmup steps, then the arms alternate, --steps steps each, for --passes passes; the
 result is steps per second (median over passes, with min and max), and the scan kernel's own
@@ -55,6 +65,34 @@ def windows(n_var, variants):
     return lo, hi
 
 
+def four_bit(seq, off):
+    """ASCII reads -> BAM 4-bit codes (=ACMGRSVTWYHKDBN), each read on a byte boundary."""
+    lut = np.full(256, 15, dtype=np.uint8)
+    for i, c in enumerate(b"=ACMGRSVTWYHKDBN"):
+        lut[c] = i
+        lut[ord(chr(c).lower())] = i
+    codes = lut[seq]
+    out = []
+    for r in range(len(off) - 1):
+        c = codes[int(off[r]):int(off[r + 1])]
+        if len(c) % 2:
+            c = np.append(c, 0)
+        out.append((c[0::2] << 4) | c[1::2])
+    return np.concatenate(out).astype(np.uint8) if out else np.zeros(0, np.uint8)
+
+
+def extras(host, reads=None):
+    """What the sparse and decoded-read arms submit, in pinned memory: the zero list of the
+    stream's flags, and the decoded reads (ASCII and 4-bit) when the workload has them."""
+    zoff, zbytes = dkb.mask_to_zero_list(host.mask1, host.n_positions)
+    x = {"zl": (pinned(zoff), pinned(zbytes))}
+    if reads is not None:
+        seq, qual, off = reads
+        x["reads"] = (pinned(seq), pinned(qual), pinned(off))
+        x["seq4"] = pinned(four_bit(seq, off))
+    return x
+
+
 def device_workload(argv, dev):
     """bench.py's generator: [(device b2, device m1, host ReadStream, ReadLoci)] per sample."""
     a = bench.parse_args(argv)
@@ -64,7 +102,7 @@ def device_workload(argv, dev):
     for b2, m1, n_pos, n_bases, loci in streams_with_loci(a, genome, variants, dev):
         host = dkb.ReadStream(pinned(b2.cpu().numpy().view(np.uint32)), pinned(m1.cpu().numpy().view(np.uint32)),
                               int(n_pos), int(n_bases))
-        samples.append((b2, m1, host, loci))
+        samples.append((b2, m1, host, loci, extras(host)))
     return a.k, entries, windows(entries.n_variants, variants), samples
 
 
@@ -91,31 +129,69 @@ def fetch_workload(dev):
         host = dkb.ReadStream(pinned(st.bases2), pinned(st.mask1), st.n_positions, st.n_bases)
         b2 = torch.from_numpy(st.bases2.view(np.int32).copy()).to(dev)
         m1 = torch.from_numpy(st.mask1.view(np.int32).copy()).to(dev)
-        samples.append((b2, m1, host, dkb.ReadLoci(boff, lo[idx], hi[idx])))
+        samples.append((b2, m1, host, dkb.ReadLoci(boff, lo[idx], hi[idx]), extras(host, (bseq, bqual, boff))))
     torch.cuda.synchronize()
     return k, entries, (vlo, vhi), samples
 
 
-ARMS = [("ws_host", False, "host"), ("rg_host", True, "host"), ("rg_device", True, "device")]
+ARMS = [("ws_host", False, "host"), ("rg_host", True, "host"), ("rg_device", True, "device"),
+        ("ws_sparse", False, "sparse"), ("rg_sparse", True, "sparse"), ("ws_reads", False, "reads"),
+        ("rg_reads", True, "reads"), ("ws_reads4", False, "reads4"), ("rg_reads4", True, "reads4"),
+        ("dense_sparse", False, "dense_sparse")]
+MIN_BQ = dkb.DEFAULT_MIN_BASEQ
 
 
 def step_fn(kc, samples, regions, form, multi):
     loci = [x[3] for x in samples] if regions else None
+    one = lambda s: loci[s] if regions else None  # noqa: E731
+    smp = list(range(len(samples)))
+    zl = [(x[2].bases2, *x[4]["zl"], x[2].n_positions) for x in samples]
+    if form in ("reads", "reads4"):
+        rd = [(x[4]["seq4"] if form == "reads4" else x[4]["reads"][0], *x[4]["reads"][1:]) for x in samples]
+    if form == "dense_sparse":
+        if multi:
+            return lambda: kc.submit_sparse_multi(zl, smp)
+        return lambda: kc.submit_multi([x[2] for x in samples], smp)
+    if form == "sparse":
+        if multi:
+            return lambda: kc.submit_sparse_multi(zl, smp, loci=loci)
+        return lambda: [kc.submit_sparse(*z[:3], z[3], s, loci=one(s)) for s, z in enumerate(zl)]
+    if form in ("reads", "reads4"):
+        fb = form == "reads4"
+        if multi:
+            return lambda: kc.submit_reads_multi(rd, smp, MIN_BQ, four_bit=fb, loci=loci)
+        return lambda: [kc.submit_reads(*r, s, MIN_BQ, four_bit=fb, loci=one(s)) for s, r in enumerate(rd)]
     if multi and form == "host":
-        return lambda: kc.submit_multi([x[2] for x in samples], [0, 1, 2], loci=loci)
+        return lambda: kc.submit_multi([x[2] for x in samples], smp, loci=loci)
     if multi:
         return lambda: kc.submit_device_multi([(x[0].data_ptr(), x[1].data_ptr(), x[2].n_positions, s)
                                                for s, x in enumerate(samples)], loci=loci)
     if form == "host":
-        return lambda: [kc.submit(x[2], s, loci=loci[s] if regions else None) for s, x in enumerate(samples)]
+        return lambda: [kc.submit(x[2], s, loci=one(s)) for s, x in enumerate(samples)]
     return lambda: [kc.submit_device(x[0].data_ptr(), x[1].data_ptr(), x[2].n_positions, s,
-                                     loci=loci[s] if regions else None) for s, x in enumerate(samples)]
+                                     loci=one(s)) for s, x in enumerate(samples)]
+
+
+def pcie_bytes(samples, form):
+    """Bytes the multi form of an arm copies host -> device per step (device arms: 0)."""
+    n = 0
+    for x in samples:
+        h, e = x[2], x[4]
+        if form in ("host",):
+            n += h.bases2.nbytes + h.mask1.nbytes
+        elif form in ("sparse", "dense_sparse"):
+            n += h.bases2.nbytes + e["zl"][0].nbytes + e["zl"][1].nbytes
+        elif form in ("reads", "reads4"):
+            seq, qual, off = e["reads"]
+            n += (e["seq4"].nbytes + 8 * (len(off) - 1) if form == "reads4" else seq.nbytes) + qual.nbytes + off.nbytes
+    return n
 
 
 def workload(name, k, entries, wins, samples, steps, warmup, passes):
     import torch
     counters = {}
-    for arm, regions, form in ARMS:
+    arms = [a for a in ARMS if a[2] not in ("reads", "reads4") or "reads" in samples[0][4]]
+    for arm, regions, form in arms:
         for multi in (False, True):
             kc = dkb.KmerCounter(k)
             kc.build_table(entries)
@@ -139,7 +215,8 @@ def workload(name, k, entries, wins, samples, steps, warmup, passes):
             scan.append((kc.stats()["scan_ms_total"] - s0) / steps)
     out = {"workload": name, "n_bases": int(sum(x[2].n_bases for x in samples)), "n_entries": len(entries),
            "bases_per_sample": [int(x[2].n_bases) for x in samples]}
-    for arm, _, _ in ARMS:
+    n_bases = sum(x[2].n_bases for x in samples)
+    for arm, _, form in arms:
         res = {}
         for multi in (False, True):
             kc, _, rates, scan = counters[(arm, multi)]
@@ -150,7 +227,12 @@ def workload(name, k, entries, wins, samples, steps, warmup, passes):
         res["counters_equal"] = bool(np.array_equal(a.entry_counts(), b.entry_counts()))
         res["counted"] = int(b.entry_counts().astype(np.uint64).sum())
         res["step_speedup"] = round(res["multi"]["steps_per_s"] / res["single"]["steps_per_s"], 3)
+        res["pcie_bytes_per_base"] = round(pcie_bytes(samples, form) / n_bases, 4)
         out[arm] = res
+    # every arm of one counting mode ran the same steps: its counters equal ws_host's / rg_host's
+    ref = {False: counters[("ws_host", False)][0].entry_counts(), True: counters[("rg_host", False)][0].entry_counts()}
+    out["counters_equal_across_arms"] = all(
+        np.array_equal(counters[(arm, m)][0].entry_counts(), ref[regions]) for arm, regions, _ in arms for m in (False, True))
     for kc, _, _, _ in counters.values():
         kc.close()
     torch.cuda.synchronize()
@@ -177,7 +259,8 @@ def main(argv=None):
     if not args.no_config1:
         out["results"].append(workload("configs[1]", *device_workload([], dev), max(2, args.steps // 10),
                                        1, args.passes))
-    out["all_counters_equal"] = all(r[arm]["counters_equal"] for r in out["results"] for arm, _, _ in ARMS)
+    out["all_counters_equal"] = all(r[arm]["counters_equal"] for r in out["results"] for arm, _, _ in ARMS if arm in r)
+    out["all_counters_equal_across_arms"] = all(r["counters_equal_across_arms"] for r in out["results"])
     print(json.dumps(out))
 
 
