@@ -40,6 +40,19 @@ pub const DKB_MAX_CHILDREN: usize = 6;
 /// Sample index of child `c` in a family (DKB_CHILD_SAMPLE): 0 for c == 0, else 2 + c.
 pub const fn dkb_child_sample(c: usize) -> usize { if c == 0 { 0 } else { c + 2 } }
 pub const DKB_CALL_DENOVO: u8 = 0x01;
+pub const DKB_CALL_CHILD_LOW: u8 = 0x02;
+pub const DKB_CALL_MOTHER_ALT: u8 = 0x04;
+pub const DKB_CALL_FATHER_ALT: u8 = 0x08;
+pub const DKB_CALL_PARENT_UNCOVERED: u8 = 0x10;
+/// The child's sex has no copy of the locus (a daughter at Y).
+pub const DKB_CALL_NO_COPY: u8 = 0x20;
+pub const DKB_LOCUS_AUTOSOMAL: u8 = 0;
+pub const DKB_LOCUS_X: u8 = 1;
+pub const DKB_LOCUS_Y: u8 = 2;
+pub const DKB_LOCUS_MATERNAL: u8 = 3;
+pub const DKB_SEX_UNKNOWN: u8 = 0;
+pub const DKB_SEX_MALE: u8 = 1;
+pub const DKB_SEX_FEMALE: u8 = 2;
 
 extern "C" {
     pub fn dkb_abi_version() -> c_int;
@@ -107,6 +120,8 @@ extern "C" {
     pub fn dkb_finalise_from(ctx: *mut DkbCtx, thr: *const DkbThresholds, d_counts: *const u32) -> c_int;
     pub fn dkb_results_fetch(ctx: *mut DkbCtx, hits: *mut u32, distinct: *mut u32,
                              n_kmers: *mut u32, calls: *mut u8) -> c_int;
+    pub fn dkb_table_set_locus_classes(ctx: *mut DkbCtx, cls: *const u8, n_variants: u32) -> c_int;
+    pub fn dkb_ctx_set_child_sexes(ctx: *mut DkbCtx, sex: *const u8, n_children: c_int) -> c_int;
     pub fn dkb_host_alloc(ctx: *mut DkbCtx, bytes: usize, out: *mut *mut c_void) -> c_int;
     pub fn dkb_host_free(ctx: *mut DkbCtx, p: *mut c_void) -> c_int;
     pub fn dkb_thread_bind_near_gpu(ctx: *mut DkbCtx, numa_node_out: *mut c_int) -> c_int;

@@ -25,6 +25,31 @@ pub const CHILD: i32 = 0;
 pub const MOTHER: i32 = 1;
 pub const FATHER: i32 = 2;
 pub const CALL_DENOVO: u8 = 0x01;
+pub const CALL_NO_COPY: u8 = 0x20;
+
+/// Locus class of a candidate (`include/dkb.h` DKB_LOCUS_*), from the VCF's CHROM and POS and
+/// the assembly's PAR coordinates.
+#[derive(Debug, Clone, Copy, PartialEq, Eq)]
+#[repr(u8)]
+pub enum LocusClass {
+    /// Autosomes, and PAR1 / PAR2 of X and Y.
+    Autosomal = 0,
+    /// X outside the PARs.
+    X = 1,
+    /// Y outside the PARs.
+    Y = 2,
+    /// Mitochondrial.
+    Maternal = 3,
+}
+
+/// Sex of a child (`include/dkb.h` DKB_SEX_*), from the PED file's sex column.
+#[derive(Debug, Clone, Copy, PartialEq, Eq)]
+#[repr(u8)]
+pub enum Sex {
+    Unknown = 0,
+    Male = 1,
+    Female = 2,
+}
 pub use sys::{dkb_child_sample as child_sample, DKB_MAX_CHILDREN as MAX_CHILDREN};
 
 /// Error code of the C ABI plus the library's detail string.
@@ -246,6 +271,26 @@ impl Counter {
 
     pub fn clear_regions(&mut self) -> Result<()> {
         self.ck(unsafe { sys::dkb_table_set_regions(self.ctx, ptr::null(), ptr::null(), 0) })
+    }
+
+    /// Inheritance (`include/dkb.h`): the locus class of every variant of the table.  From now
+    /// on each call applies only the clauses of the parents who can transmit the variant's locus
+    /// to the child.  A new table, or [`Counter::clear_locus_classes`], returns to all autosomal.
+    pub fn set_locus_classes(&mut self, cls: &[LocusClass]) -> Result<()> {
+        let raw: Vec<u8> = cls.iter().map(|&c| c as u8).collect();
+        let n = u32::try_from(raw.len()).unwrap_or(u32::MAX);
+        self.ck(unsafe { sys::dkb_table_set_locus_classes(self.ctx, raw.as_ptr(), n) })
+    }
+
+    pub fn clear_locus_classes(&mut self) -> Result<()> {
+        self.ck(unsafe { sys::dkb_table_set_locus_classes(self.ctx, ptr::null(), 0) })
+    }
+
+    /// Inheritance: the sex of every child, one per child of the context; kept across tables.
+    pub fn set_child_sexes(&mut self, sexes: &[Sex]) -> Result<()> {
+        let raw: Vec<u8> = sexes.iter().map(|&s| s as u8).collect();
+        let n = c_int::try_from(raw.len()).unwrap_or(c_int::MAX);
+        self.ck(unsafe { sys::dkb_ctx_set_child_sexes(self.ctx, raw.as_ptr(), n) })
     }
 
     /// Region mode: the loci of the NEXT submitted batch - the batch's `offsets` (as packed) and

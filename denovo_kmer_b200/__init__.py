@@ -7,7 +7,8 @@ step can import the package), but any call raises ImportError until it is built,
 DKB_ENODEV without a B200.
 """
 from .api import (ALT, CALL_CHILD_LOW, CALL_DENOVO, CALL_FATHER_ALT, CALL_MOTHER_ALT,  # noqa: F401
-                  CALL_PARENT_UNCOVERED, CHILD, DEFAULT_MIN_BASEQ, DEFAULT_THRESHOLDS, FATHER,
+                  CALL_NO_COPY, CALL_PARENT_UNCOVERED, CHILD, DEFAULT_MIN_BASEQ, DEFAULT_THRESHOLDS, FATHER,
+                  LOCUS_AUTOSOMAL, LOCUS_MATERNAL, LOCUS_X, LOCUS_Y, SEX_FEMALE, SEX_MALE, SEX_UNKNOWN,
                   MAX_CHILDREN, MOTHER, REF, KmerCounter, KmerEntries, ReadLoci, ReadStream, child_sample, kmer_canonical,
                   comm_unique_id, kmer_encode, mask_to_zero_list, kmer_revcomp, pack_reads, stream_words, variant_kmers)
 from ._lib import DkbError  # noqa: F401

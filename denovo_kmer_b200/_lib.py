@@ -91,6 +91,8 @@ SYMBOLS = {
     "dkb_finalise": (C.c_int, [C.c_void_p, C.POINTER(Thresholds)]),
     "dkb_finalise_from": (C.c_int, [C.c_void_p, C.POINTER(Thresholds), C.c_void_p]),
     "dkb_results_fetch": (C.c_int, [C.c_void_p, u32p, u32p, u32p, u8p]),
+    "dkb_table_set_locus_classes": (C.c_int, [C.c_void_p, u8p, C.c_uint32]),
+    "dkb_ctx_set_child_sexes": (C.c_int, [C.c_void_p, u8p, C.c_int]),
     "dkb_host_alloc": (C.c_int, [C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p)]),
     "dkb_host_free": (C.c_int, [C.c_void_p, C.c_void_p]),
     "dkb_thread_bind_near_gpu": (C.c_int, [C.c_void_p, C.POINTER(C.c_int)]),

@@ -15,8 +15,11 @@ from ._lib import Stats, Thresholds, Tuning, check, u8p, u16p, u32p, u64p
 
 CHILD, MOTHER, FATHER = 0, 1, 2
 REF, ALT = 0, 1
-CALL_DENOVO, CALL_CHILD_LOW, CALL_MOTHER_ALT, CALL_FATHER_ALT, CALL_PARENT_UNCOVERED = (
-    0x01, 0x02, 0x04, 0x08, 0x10)
+CALL_DENOVO, CALL_CHILD_LOW, CALL_MOTHER_ALT, CALL_FATHER_ALT, CALL_PARENT_UNCOVERED, CALL_NO_COPY = (
+    0x01, 0x02, 0x04, 0x08, 0x10, 0x20)
+# locus class of a variant (set_locus_classes) and sex of a child (set_child_sexes)
+LOCUS_AUTOSOMAL, LOCUS_X, LOCUS_Y, LOCUS_MATERNAL = 0, 1, 2, 3
+SEX_UNKNOWN, SEX_MALE, SEX_FEMALE = 0, 1, 2
 DEFAULT_THRESHOLDS = (3, 2, 0, 1)
 DEFAULT_MIN_BASEQ = 20
 MAX_CHILDREN = _lib.MAX_CHILDREN
@@ -255,6 +258,27 @@ class KmerCounter:
         """Back to whole-stream counting."""
         self._ck(self._L.dkb_table_set_regions(self._h, None, None, 0))
 
+    def set_locus_classes(self, cls):
+        """Locus class of every variant of the table (LOCUS_AUTOSOMAL - PARs included -,
+        LOCUS_X, LOCUS_Y outside the PARs, LOCUS_MATERNAL for MT): from now on a call applies
+        only the clauses of the parents who can transmit the variant's locus to the child
+        (include/dkb.h "inheritance").  A new table returns to all autosomal."""
+        cls = np.ascontiguousarray(cls, dtype=np.uint8)
+        self._ck(self._L.dkb_table_set_locus_classes(self._h, _p(cls, u8p), len(cls)))
+
+    def clear_locus_classes(self):
+        """Back to every variant autosomal."""
+        self._ck(self._L.dkb_table_set_locus_classes(self._h, None, 0))
+
+    def set_child_sexes(self, sexes):
+        """Sex of every child (SEX_UNKNOWN, SEX_MALE, SEX_FEMALE; one per child); None returns
+        every child to unknown.  Kept across table builds."""
+        if sexes is None:
+            self._ck(self._L.dkb_ctx_set_child_sexes(self._h, None, 0))
+            return
+        sx = np.ascontiguousarray(sexes, dtype=np.uint8)
+        self._ck(self._L.dkb_ctx_set_child_sexes(self._h, _p(sx, u8p), len(sx)))
+
     def _set_loci(self, loci):
         if loci is None:
             return
@@ -456,7 +480,8 @@ class KmerCounter:
 
     def reduce_push(self, thresholds=DEFAULT_THRESHOLDS):
         """Snapshot the counters and start their sum over ranks on a side stream; queues
-        kernel 3 for the PREVIOUS snapshot behind the scans submitted since."""
+        kernel 3 for the PREVIOUS snapshot behind the scans submitted since.  The snapshot keeps
+        the locus classes and child sexes in force now; its kernel 3 uses those."""
         t = Thresholds(*[int(x) for x in thresholds])
         self._ck(self._L.dkb_reduce_push(self._h, C.byref(t)))
 

@@ -90,6 +90,11 @@ struct dkb_ctx {
   uint32_t *d_hits = nullptr, *d_distinct = nullptr, *d_nkmers = nullptr;
   uint8_t *d_calls = nullptr;
   bool finalised = false;
+  // inheritance (dkb_table_set_locus_classes, dkb_ctx_set_child_sexes): each variant's locus
+  // class (null: all autosomal) and each child's sex
+  uint8_t *d_cls = nullptr;  // [n_variants], allocated by the first dkb_table_set_locus_classes
+  bool cls_on = false;       // d_cls holds classes in force (else: all autosomal)
+  ChildSexes sexes = 0;
   // profiling counters
   bool prof = false;
   unsigned long long *d_prof = nullptr;
@@ -145,6 +150,11 @@ struct dkb_ctx {
   size_t red_cap = 0;                       // capacity of each, in uint32
   cudaEvent_t ev_snap[2] = {nullptr, nullptr}, ev_red[2] = {nullptr, nullptr};
   int red_next = 0, red_pending = -1, red_last = -1;
+  // the locus classes (copied, on the scan stream; null when all autosomal) and child sexes in
+  // force when each snapshot was pushed: its kernel 3 uses these
+  uint8_t *d_red_cls[2] = {nullptr, nullptr};
+  bool red_has_cls[2] = {false, false};
+  ChildSexes red_sexes[2] = {0, 0};
   // region mode (dkb_table_set_regions): each entry's variant window, and the loci the next
   // submit takes (host buffers, copied by that submit): one batch's (dkb_batch_set_loci) or
   // one set per batch of a multi-batch submit (dkb_batch_set_loci_multi)
@@ -224,6 +234,9 @@ void free_table(dkb_ctx *c) {
   dfree(c->d_calls);
   dfree(c->d_entry_win);
   c->regions = false;  // a new table counts the whole stream until dkb_table_set_regions
+  dfree(c->d_cls);
+  c->cls_on = false;  // ... and is all autosomal until dkb_table_set_locus_classes
+  for (int i = 0; i < 2; i++) dfree(c->d_red_cls[i]);
   drop_loci(c);
   c->n_entries = c->n_live = 0;
   c->occupied_halves = c->direct_halves = 0;
@@ -1019,7 +1032,8 @@ int reduce_setup(dkb_ctx *ctx) {
   return DKB_OK;
 }
 
-int finalise_counts(dkb_ctx *ctx, const dkb_thresholds *thr, const uint32_t *d_counts);
+int finalise_counts(dkb_ctx *ctx, const dkb_thresholds *thr, const uint32_t *d_counts, const uint8_t *cls,
+                    const ChildSexes &sexes);
 
 // Samples a submit may name: [0, n_samples).
 int check_sample(dkb_ctx *ctx, int sample) {
@@ -1128,7 +1142,8 @@ int check_loci(dkb_ctx *ctx, const uint64_t *offsets, const uint64_t *lo, const 
 // Kernel 3 on snapshot b, on the scan stream, once its sum over ranks is complete.
 int finalise_snapshot(dkb_ctx *ctx, const dkb_thresholds *thr, int b) {
   CU(cudaStreamWaitEvent(ctx->s_scan, ctx->ev_red[b], 0));
-  int rc = finalise_counts(ctx, thr, ctx->d_red[b]);
+  int rc = finalise_counts(ctx, thr, ctx->d_red[b], ctx->red_has_cls[b] ? ctx->d_red_cls[b] : nullptr,
+                           ctx->red_sexes[b]);
   ctx->red_last = b;
   return rc;
 }
@@ -1535,6 +1550,42 @@ int dkb_table_set_regions(dkb_ctx *ctx, const uint64_t *lo, const uint64_t *hi, 
   return DKB_OK;
 }
 
+int dkb_table_set_locus_classes(dkb_ctx *ctx, const uint8_t *cls, uint32_t n_variants) {
+  if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
+  if (!ctx->d_tslots) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
+  if (!cls) {
+    if (n_variants) return fail(ctx, DKB_EINVAL, "cls == NULL (all autosomal) takes n_variants 0");
+    ctx->cls_on = false;
+    return DKB_OK;
+  }
+  if (n_variants != ctx->n_variants)
+    return fail(ctx, DKB_EINVAL, "n_variants differs from the table's (" + std::to_string(ctx->n_variants) + ")");
+  for (uint32_t v = 0; v < n_variants; v++)
+    if (cls[v] > DKB_LOCUS_MATERNAL)
+      return fail(ctx, DKB_EINVAL, "locus class of variant " + std::to_string(v) + " is above 3");
+  CU(cudaSetDevice(ctx->device));
+  if (!ctx->d_cls) CU(cudaMalloc(&ctx->d_cls, n_variants ? n_variants : 1));
+  // on the scan stream: a kernel 3 queued before this call still reads the previous classes
+  if (n_variants) CU(cudaMemcpyAsync(ctx->d_cls, cls, n_variants, cudaMemcpyHostToDevice, ctx->s_scan));
+  CU(cudaStreamSynchronize(ctx->s_scan));
+  ctx->cls_on = true;
+  return DKB_OK;
+}
+
+int dkb_ctx_set_child_sexes(dkb_ctx *ctx, const uint8_t *sex, int n_children) {
+  if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
+  if (!sex && n_children == 0) n_children = ctx->n_children;
+  if (n_children != ctx->n_children)
+    return fail(ctx, DKB_EINVAL, "n_children differs from the context's (" + std::to_string(ctx->n_children) + ")");
+  ChildSexes s = 0;
+  for (int c = 0; sex && c < n_children; c++) {
+    if (sex[c] > DKB_SEX_FEMALE) return fail(ctx, DKB_EINVAL, "sex of child " + std::to_string(c) + " is above 2");
+    s |= (ChildSexes)sex[c] << (2 * c);
+  }
+  ctx->sexes = s;
+  return DKB_OK;
+}
+
 int dkb_batch_set_loci(dkb_ctx *ctx, const uint64_t *offsets, const uint64_t *lo, const uint64_t *hi,
                        size_t n_reads) {
   if (!ctx) return fail(nullptr, DKB_EINVAL, "ctx is null");
@@ -1614,7 +1665,7 @@ int dkb_finalise_from(dkb_ctx *ctx, const dkb_thresholds *thr, const uint32_t *d
   if (!ctx || !thr || !d_counts) return fail(ctx, DKB_EINVAL, "null argument");
   if (!ctx->d_counts) return fail(ctx, DKB_ESTATE, "dkb_table_build must come first");
   CU(cudaSetDevice(ctx->device));
-  return finalise_counts(ctx, thr, d_counts);
+  return finalise_counts(ctx, thr, d_counts, ctx->cls_on ? ctx->d_cls : nullptr, ctx->sexes);
 }
 
 }  // extern "C"
@@ -1622,7 +1673,8 @@ int dkb_finalise_from(dkb_ctx *ctx, const dkb_thresholds *thr, const uint32_t *d
 namespace {
 // Kernel 3 for NS samples.
 template <int NS>
-void launch_finalise(dkb_ctx *ctx, const Thresholds &T, const uint32_t *d_counts) {
+void launch_finalise(dkb_ctx *ctx, const Thresholds &T, const uint32_t *d_counts, const uint8_t *cls,
+                     const ChildSexes &sexes) {
   cudaStream_t st = ctx->s_scan;
   const int TB = 256;
   if (ctx->n_entries)
@@ -1631,22 +1683,24 @@ void launch_finalise(dkb_ctx *ctx, const Thresholds &T, const uint32_t *d_counts
         ctx->d_hits, ctx->d_distinct, ctx->d_nkmers);
   const uint32_t n_items = ctx->n_variants * (uint32_t)(NS - 2);  // (variant, child) pairs
   if (n_items)
-    k_calls<NS><<<(n_items + TB - 1) / TB, TB, 0, st>>>(ctx->d_hits, ctx->d_distinct, n_items, T, ctx->d_calls);
+    k_calls<NS><<<(n_items + TB - 1) / TB, TB, 0, st>>>(ctx->d_hits, ctx->d_distinct, n_items, T, cls, sexes,
+                                                        ctx->d_calls);
 }
 
-int finalise_counts(dkb_ctx *ctx, const dkb_thresholds *thr, const uint32_t *d_counts) {
+int finalise_counts(dkb_ctx *ctx, const dkb_thresholds *thr, const uint32_t *d_counts, const uint8_t *cls,
+                    const ChildSexes &sexes) {
   const size_t nv1 = ctx->n_variants ? ctx->n_variants : 1;
   CU(cudaMemsetAsync(ctx->d_hits, 0, nv1 * (4 * (size_t)ctx->n_samples + 2) * 4, ctx->s_scan));
   Thresholds T{thr->min_child_alt_hits, thr->min_child_alt_distinct, thr->max_parent_alt_hits,
                thr->min_parent_ref_hits};
   static_assert(DKB_MAX_CHILDREN == 6, "one kernel-3 instantiation per family size");
   switch (ctx->n_samples) {
-    case 3: launch_finalise<3>(ctx, T, d_counts); break;
-    case 4: launch_finalise<4>(ctx, T, d_counts); break;
-    case 5: launch_finalise<5>(ctx, T, d_counts); break;
-    case 6: launch_finalise<6>(ctx, T, d_counts); break;
-    case 7: launch_finalise<7>(ctx, T, d_counts); break;
-    case 8: launch_finalise<8>(ctx, T, d_counts); break;
+    case 3: launch_finalise<3>(ctx, T, d_counts, cls, sexes); break;
+    case 4: launch_finalise<4>(ctx, T, d_counts, cls, sexes); break;
+    case 5: launch_finalise<5>(ctx, T, d_counts, cls, sexes); break;
+    case 6: launch_finalise<6>(ctx, T, d_counts, cls, sexes); break;
+    case 7: launch_finalise<7>(ctx, T, d_counts, cls, sexes); break;
+    case 8: launch_finalise<8>(ctx, T, d_counts, cls, sexes); break;
     default: return fail(ctx, DKB_EINVAL, "no kernel 3 for this family size");
   }
   CU(cudaGetLastError());
@@ -1739,6 +1793,15 @@ int dkb_reduce_push(dkb_ctx *ctx, const dkb_thresholds *thr) {
   if (ctx->comm && ctx->world > 1 && n)
     NC(nccl()->AllReduce(ctx->d_red[b], ctx->d_red[b], n, NCCL_UINT32, NCCL_SUM, ctx->comm, ctx->s_side));
   CU(cudaEventRecord(ctx->ev_red[b], ctx->s_side));
+  // the classes and sexes in force now go with the snapshot (the copy, on the scan stream, comes
+  // after the kernel 3 that last read this buffer)
+  ctx->red_has_cls[b] = ctx->cls_on;
+  ctx->red_sexes[b] = ctx->sexes;
+  if (ctx->cls_on) {
+    if (!ctx->d_red_cls[b]) CU(cudaMalloc(&ctx->d_red_cls[b], ctx->n_variants ? ctx->n_variants : 1));
+    if (ctx->n_variants)
+      CU(cudaMemcpyAsync(ctx->d_red_cls[b], ctx->d_cls, ctx->n_variants, cudaMemcpyDeviceToDevice, ctx->s_scan));
+  }
   const int prev = ctx->red_pending;
   ctx->red_pending = b;
   if (prev >= 0) return finalise_snapshot(ctx, thr, prev);

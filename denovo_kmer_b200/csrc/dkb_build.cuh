@@ -6,6 +6,7 @@
 // both orientations of the key and every stride class one s-mer of the k-mer
 // is designated as its seed and put in the exact seed table and the filter.
 #pragma once
+#include "../../include/dkb.h"
 #include "dkb_device.cuh"
 
 namespace dkb {
@@ -458,23 +459,43 @@ struct Thresholds {
   uint32_t min_child_alt_hits, min_child_alt_distinct, max_parent_alt_hits, min_parent_ref_hits;
 };
 
-// One thread per (variant, child): the trio rule on child ch's alt support and the parents'
-// hits; calls: [n_variants][NS - 2].  n_items = n_variants * (NS - 2).
+// Child sexes of one kernel 3 (DKB_SEX_*), by value: child c's in bits 2c, 2c + 1 (at most
+// DKB_MAX_CHILDREN of them; a word instead of an array, which indexing would put on the stack).
+typedef uint32_t ChildSexes;
+
+// Which parents' clauses apply to a child of sex `sex` at a locus of class `cls` (DESIGN.md §2
+// "Inheritance"): bit 0 the mother's, bit 1 the father's; bit 2 = the child has no copy of the
+// locus (a daughter at Y), which the call reports as DKB_CALL_NO_COPY.
+__device__ __forceinline__ uint32_t parent_clauses(uint32_t cls, uint32_t sex) {
+  switch (cls) {
+    case DKB_LOCUS_X: return sex == DKB_SEX_MALE ? 1u : 3u;
+    case DKB_LOCUS_Y: return sex == DKB_SEX_MALE ? 2u : sex == DKB_SEX_FEMALE ? 4u : 3u;
+    case DKB_LOCUS_MATERNAL: return 1u;
+    default: return 3u;
+  }
+}
+
+// One thread per (variant, child): the trio rule on child ch's alt support and the hits of the
+// parents whose clauses apply at variant v's locus class (cls[v], all autosomal when cls is
+// null) for child ch's sex; calls: [n_variants][NS - 2].  n_items = n_variants * (NS - 2).
 template <int NS>
 __global__ void k_calls(const uint32_t *hits, const uint32_t *distinct, uint32_t n_items,
-                        const Thresholds T, uint8_t *calls) {
+                        const Thresholds T, const uint8_t *cls, const ChildSexes sex, uint8_t *calls) {
   constexpr uint32_t NC = NS - 2;
   const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= n_items) return;
   const uint32_t v = t / NC, ch = t % NC;
   const uint32_t cs = ch == 0 ? 0 : ch + 2;  // DKB_CHILD_SAMPLE
   const uint32_t *h = hits + (size_t)v * 2 * NS, *d = distinct + (size_t)v * 2 * NS;  // [allele*NS+sample]
+  const uint32_t m = parent_clauses(cls ? cls[v] : (uint32_t)DKB_LOCUS_AUTOSOMAL, (sex >> (2 * ch)) & 3u);
   uint8_t c = 0;
-  if (h[NS + cs] < T.min_child_alt_hits || d[NS + cs] < T.min_child_alt_distinct) c |= 0x02;
-  if (h[NS + 1] > T.max_parent_alt_hits) c |= 0x04;
-  if (h[NS + 2] > T.max_parent_alt_hits) c |= 0x08;
-  if (h[1] < T.min_parent_ref_hits || h[2] < T.min_parent_ref_hits) c |= 0x10;
-  calls[t] = c ? c : 0x01;
+  if (h[NS + cs] < T.min_child_alt_hits || d[NS + cs] < T.min_child_alt_distinct) c |= DKB_CALL_CHILD_LOW;
+  if ((m & 1) && h[NS + 1] > T.max_parent_alt_hits) c |= DKB_CALL_MOTHER_ALT;
+  if ((m & 2) && h[NS + 2] > T.max_parent_alt_hits) c |= DKB_CALL_FATHER_ALT;
+  if (((m & 1) && h[1] < T.min_parent_ref_hits) || ((m & 2) && h[2] < T.min_parent_ref_hits))
+    c |= DKB_CALL_PARENT_UNCOVERED;
+  if (m & 4) c |= DKB_CALL_NO_COPY;
+  calls[t] = c ? c : DKB_CALL_DENOVO;
 }
 
 }  // namespace dkb

@@ -285,6 +285,129 @@ def make_family_host(genome_len: int, depth: float, n_variants: int, k: int, n_c
     return fam
 
 
+# Locus classes and sexes of include/dkb.h (DKB_LOCUS_*, DKB_SEX_*)
+LOCUS_AUTOSOMAL, LOCUS_X, LOCUS_Y, LOCUS_MATERNAL = 0, 1, 2, 3
+SEX_UNKNOWN, SEX_MALE, SEX_FEMALE = 0, 1, 2
+
+# The planted scenarios of make_sexed_family_host: name -> (locus class, the call byte the
+# inheritance rule gives a son, the byte it gives a daughter) at error-free reads and the
+# default thresholds (3, 2, 0, 1).  A parent whose one copy of X or MT carries the alt has no
+# ref hits there, so where that parent's clauses apply the byte has DKB_CALL_PARENT_UNCOVERED.
+SEXED_SCENARIOS = {
+    # the son's X comes from his mother: his alt is de novo although his father carries it
+    "x_denovo_carrier_father": (LOCUS_X, 0x01, 0x18),
+    # the daughter inherits her father's X and its alt; the son does not carry it
+    "x_inherited_paternal": (LOCUS_X, 0x02, 0x18),
+    # a son's de novo on Y; a daughter has no Y
+    "y_denovo": (LOCUS_Y, 0x01, 0x22),
+    # a child's MT de novo at a site where the father's own MT carries the alt
+    "mt_denovo_carrier_father": (LOCUS_MATERNAL, 0x01, 0x01),
+    # every child inherits the mother's MT alt, which the father's own MT carries too
+    "mt_inherited_maternal": (LOCUS_MATERNAL, 0x14, 0x14),
+    # autosomal controls: de novo in every child, and inherited from the mother by every child
+    "autosomal_denovo": (LOCUS_AUTOSOMAL, 0x01, 0x01),
+    "autosomal_inherited": (LOCUS_AUTOSOMAL, 0x04, 0x04),
+}
+
+
+@dataclass
+class SexedFamily(Trio):
+    classes: np.ndarray = None  # uint8 locus class per variant (LOCUS_*)
+    sexes: list = None          # sex of child c (SEX_MALE / SEX_FEMALE)
+    scenarios: list = None      # SEXED_SCENARIOS name of each variant
+    segments: dict = None       # locus class -> [start, end) of its segment in the genome
+
+
+def make_sexed_family_host(sexes, k: int, seed: int = 1, depth: float = 20, per_scenario: int = 3,
+                           seg_len=(60_000, 40_000, 20_000, 16_000), read_len: int = 150,
+                           **read_kw) -> SexedFamily:
+    """A family whose samples hold an autosome, X, Y and mitochondrial (MT) segment at the copy
+    numbers of their sex: mother (sample 1) autosome x2, X x2, her own MT; father (sample 2)
+    autosome x2, X x1, Y x1, his own MT; child c (sample child_sample(c)) of sexes[c] the
+    autosome x2, the mother's first X, and the father's X (daughter) or Y (son), and the
+    mother's MT.  Depth is per copy, so hemizygous segments come out at half the depth.  The
+    segments lie back to back in one genome (fam.segments), and read loci are in its
+    coordinates.  per_scenario SNVs of every SEXED_SCENARIOS scenario are planted, each 3k or
+    more from the next; fam.scenarios names each variant's, fam.classes gives its locus class."""
+    sexes = [int(s) for s in sexes]
+    assert sexes and all(s in (SEX_MALE, SEX_FEMALE) for s in sexes)
+    rng = np.random.default_rng(seed)
+    order = (LOCUS_AUTOSOMAL, LOCUS_X, LOCUS_Y, LOCUS_MATERNAL)
+    genome = make_genome(sum(seg_len), seed)
+    segments, s0 = {}, 0
+    for cls, n in zip(order, seg_len):
+        segments[cls] = (s0, s0 + n)
+        s0 += n
+    # SNVs on an even grid inside their segment, away from its ends
+    by_cls = {c: [name for name, sc in SEXED_SCENARIOS.items() if sc[0] == c] for c in order}
+    variants, scen = [], []
+    for cls in order:
+        names = [nm for nm in by_cls[cls] for _ in range(per_scenario)]
+        lo, hi = segments[cls]
+        step = (hi - lo - 8 * k) // max(len(names), 1)
+        assert step >= 3 * k, "segment too short for its scenarios"
+        for i, nm in enumerate(names):
+            pos = lo + 4 * k + i * step + int(rng.integers(0, step - 2 * k))
+            ref = chr(genome[pos])
+            alt = "ACGT"[("ACGT".index(ref) + int(rng.integers(1, 4))) % 4]
+            variants.append(Variant(pos, ref, alt))
+            scen.append(nm)
+
+    def alts(*names):
+        """{pos: alt base} of every variant of the named scenarios"""
+        return {v.pos: v.alt for v, nm in zip(variants, scen) if nm in names}
+
+    # copies: (locus class, {pos: base})
+    mat_a = (LOCUS_AUTOSOMAL, alts("autosomal_inherited"))
+    mat_x = (LOCUS_X, {})
+    mat_mt = (LOCUS_MATERNAL, alts("mt_inherited_maternal"))
+    pat_x = (LOCUS_X, alts("x_denovo_carrier_father", "x_inherited_paternal"))
+    pat_y = (LOCUS_Y, {})
+    copies = {
+        1: [mat_a, (LOCUS_AUTOSOMAL, {}), mat_x, (LOCUS_X, {}), mat_mt],
+        2: [(LOCUS_AUTOSOMAL, {}), (LOCUS_AUTOSOMAL, {}), pat_x, pat_y,
+            (LOCUS_MATERNAL, alts("mt_denovo_carrier_father", "mt_inherited_maternal"))],
+    }
+    for c, sex in enumerate(sexes):
+        child = [mat_a, (LOCUS_AUTOSOMAL, alts("autosomal_denovo")),
+                 (LOCUS_MATERNAL, {**mat_mt[1], **alts("mt_denovo_carrier_father")})]
+        if sex == SEX_MALE:
+            child += [(LOCUS_X, alts("x_denovo_carrier_father")), (LOCUS_Y, alts("y_denovo"))]
+        else:
+            child += [mat_x, pat_x]
+        copies[child_sample(c)] = child
+    fam = SexedFamily(k, genome, variants, n_children=len(sexes), classes=np.array(
+        [SEXED_SCENARIOS[nm][0] for nm in scen], dtype=np.uint8), sexes=sexes, scenarios=scen, segments=segments)
+    for smp in sorted(copies):
+        seqs, quals, lens, los = [], [], [], []
+        for j, cls in enumerate(order):
+            lo, hi = segments[cls]
+            haps = []
+            for ccls, edits in copies[smp]:
+                if ccls != cls:
+                    continue
+                h = genome[lo:hi].copy()
+                for p, b in edits.items():
+                    h[p - lo] = ord(b)
+                haps.append(h)
+            if not haps:
+                continue
+            n_reads = int(round((hi - lo) * depth * len(haps) / read_len))
+            seq, qual, off, (hap_of, starts) = sample_reads(haps, n_reads, read_len, seed + 10 + 4 * smp + j,
+                                                            return_meta=True, **read_kw)
+            seqs.append(seq)
+            quals.append(qual)
+            lens.append(np.diff(off).astype(np.int64))
+            los.append(starts + lo)
+        lens = np.concatenate(lens)
+        off = np.zeros(len(lens) + 1, dtype=np.uint64)
+        off[1:] = np.cumsum(lens)
+        fam.reads[smp] = (np.concatenate(seqs), np.concatenate(quals), off)
+        lo = np.concatenate(los)
+        fam.loci[smp] = (lo.astype(np.uint64), (lo + lens).astype(np.uint64))
+    return fam
+
+
 # ---------------------------------------------------------------------------------------
 # GPU generator: packed streams built in HBM (bench workload; no host copy of the reads)
 # ---------------------------------------------------------------------------------------

@@ -75,7 +75,9 @@ typedef struct dkb_ctx dkb_ctx;
  *   father alt hits     <= max_parent_alt_hits     and
  *   mother ref hits     >= min_parent_ref_hits     and
  *   father ref hits     >= min_parent_ref_hits.
- * Failing clauses set bits 1..4 (see DKB_CALL_*). */
+ * Failing clauses set bits 1..4 (see DKB_CALL_*).  With locus classes and child sexes set
+ * (dkb_table_set_locus_classes, dkb_ctx_set_child_sexes) only the clauses of the parents who can
+ * transmit the locus to that child apply; see "inheritance" below. */
 typedef struct dkb_thresholds {
   uint32_t min_child_alt_hits;
   uint32_t min_child_alt_distinct;
@@ -88,6 +90,17 @@ typedef struct dkb_thresholds {
 #define DKB_CALL_MOTHER_ALT 0x04u     /* mother carries alt k-mers */
 #define DKB_CALL_FATHER_ALT 0x08u     /* father carries alt k-mers */
 #define DKB_CALL_PARENT_UNCOVERED 0x10u /* a parent lacks ref k-mer coverage */
+#define DKB_CALL_NO_COPY 0x20u        /* the child's sex has no copy of the locus (a daughter at Y) */
+
+/* Locus class of a variant (dkb_table_set_locus_classes) */
+#define DKB_LOCUS_AUTOSOMAL 0 /* autosomes, and PAR1 / PAR2 of X and Y */
+#define DKB_LOCUS_X 1         /* X outside the PARs */
+#define DKB_LOCUS_Y 2         /* Y outside the PARs */
+#define DKB_LOCUS_MATERNAL 3  /* mitochondrial */
+/* Sex of a child (dkb_ctx_set_child_sexes) */
+#define DKB_SEX_UNKNOWN 0
+#define DKB_SEX_MALE 1
+#define DKB_SEX_FEMALE 2
 
 /* Scan tuning, normally left to the library (dkb_ctx_set_tuning(ctx, NULL)). */
 typedef struct dkb_tuning {
@@ -302,6 +315,33 @@ int dkb_finalise_from(dkb_ctx *ctx, const dkb_thresholds *thr, const uint32_t *d
  * byte at calls[v * n_children + c] (a trio: [n_variants]).  Any pointer may be NULL. */
 int dkb_results_fetch(dkb_ctx *ctx, uint32_t *hits, uint32_t *distinct, uint32_t *n_kmers,
                       uint8_t *calls);
+
+/* ---- inheritance: which parents can transmit a locus (opt-in; DESIGN.md §2) ----------- */
+/* With nothing set every variant is autosomal and every child's sex unknown: the rule above
+ * applies both parents' clauses to every call.  Otherwise, for variant v of class cls[v] and
+ * child c of sex sex[c], only these parents' clauses apply ("M": DKB_CALL_MOTHER_ALT and the
+ * mother's half of DKB_CALL_PARENT_UNCOVERED; "F": the father's):
+ *   class \ sex   unknown  male  female
+ *   autosomal     M F      M F   M F
+ *   X             M F      M     M F
+ *   Y             M F      F     none, and DKB_CALL_NO_COPY is set
+ *   maternal      M        M     M
+ * DKB_CALL_CHILD_LOW is unchanged, and bit 0 (DKB_CALL_DENOVO) is set iff no other bit is, so a
+ * DKB_CALL_NO_COPY byte is never a call.  Thresholds and counting are unchanged.
+ * dkb_finalise / dkb_finalise_from use the classes and sexes in force when called;
+ * dkb_reduce_push records them with its snapshot, and that snapshot's kernel 3 (queued by the
+ * next push or the flush) uses what was recorded.  A kernel 3 already queued never sees a later
+ * change.  Multi-GPU: every rank computes the calls from the same summed counters, so every
+ * rank must set the same classes and sexes; no collective is involved. */
+/* After dkb_table_build: cls[v] in 0..3 (DKB_LOCUS_*) for each of the table's n_variants.
+ * cls == NULL (n_variants 0) returns to all-autosomal; so does a new dkb_table_build.
+ * DKB_ESTATE before dkb_table_build; DKB_EINVAL if n_variants differs from the table's or a
+ * class is above 3. */
+int dkb_table_set_locus_classes(dkb_ctx *ctx, const uint8_t *cls, uint32_t n_variants);
+/* sex[c] in 0..2 (DKB_SEX_*) for each of the context's n_children children; sex == NULL
+ * (n_children 0 or the context's) returns every child to unknown.  Any time; kept across table
+ * builds.  DKB_EINVAL if n_children differs from the context's or a sex is above 2. */
+int dkb_ctx_set_child_sexes(dkb_ctx *ctx, const uint8_t *sex, int n_children);
 
 /* ---- pinned staging next to the GPU ------------------------------------------ */
 /* Page-locked host memory for the packed batches, allocated on the NUMA node the GPU's PCIe

@@ -156,6 +156,15 @@ class Counter {
     check(dkb_table_set_regions(ctx_, lo.data(), hi.data(), (uint32_t)lo.size()), ctx_);
   }
   void clear_regions() { check(dkb_table_set_regions(ctx_, nullptr, nullptr, 0), ctx_); }
+  // Inheritance (dkb.h): the locus class of every variant (DKB_LOCUS_*) and the sex of every
+  // child (DKB_SEX_*) decide which parents' clauses each call applies.
+  void set_locus_classes(const std::vector<uint8_t> &cls) {
+    check(dkb_table_set_locus_classes(ctx_, cls.data(), (uint32_t)cls.size()), ctx_);
+  }
+  void clear_locus_classes() { check(dkb_table_set_locus_classes(ctx_, nullptr, 0), ctx_); }
+  void set_child_sexes(const std::vector<uint8_t> &sex) {
+    check(dkb_ctx_set_child_sexes(ctx_, sex.data(), (int)sex.size()), ctx_);
+  }
   // The loci of the next submit: the batch's offsets and its reads' [lo, hi).  The vectors
   // must stay alive and unchanged until sync().
   void set_loci(const std::vector<uint64_t> &offsets, const std::vector<uint64_t> &lo,
